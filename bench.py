@@ -17,6 +17,7 @@ single-env drop-in of config 1; and a per-rank parity spot check against the CPU
 
   python bench.py [--gpus N] [--steps K] [--warmup W]           our arm (one rank per GPU under torchrun)
   python bench.py --impl reference ...                          the CPU arm: the oracle port on the host cores
+  python bench.py ... --dump-outputs DIR                        also write what the last timed step computed (rank 0)
 
 Prints ONE JSON line (rank 0).
 """
@@ -63,7 +64,29 @@ def parse():
     ap.add_argument("--no-multi", action="store_true", help="one launch per actor step + a separate greedy-controller "
                     "kernel every `spacing` steps (round-1 scheme) instead of te_step_multi")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last of them computed "
+                    "(rank 0: obs, reward, done and the actions in force, one row per env) as DIR/<name>.npy, so that two "
+                    "builds can be compared on the same inputs; a seeded sample of the env rows when all exceed 64 MB")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return a
+
+
+DUMP_MAX_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(path, arrays, max_bytes=DUMP_MAX_BYTES, seed=0):
+    """Writes every [E, ...] host array of `arrays` as path/<name>.npy in float32, plus path/env_index.npy (float64): the
+    env rows written.  All E rows when they fit `max_bytes`, else the same seeded sample of rows from every array."""
+    E = len(next(iter(arrays.values())))
+    row_bytes = 8 + sum(4 * int(np.prod(a.shape[1:])) for a in arrays.values())
+    n = min(E, (max_bytes - 256 * (len(arrays) + 1)) // row_bytes)       # 256: room for each file's .npy header
+    idx = np.arange(E) if n == E else np.sort(np.random.RandomState(seed).choice(E, n, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "env_index.npy"), idx.astype(np.float64))
+    for name, arr in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(arr[idx], dtype=np.float32))
 
 
 # --------------------------------------------------------------------------- clocks
@@ -483,6 +506,14 @@ class Runner(object):
         return dict(ms=ms_max, local=d, vu=tot[0], ticks=tot[1], asteps=tot[2], gen=tot[3], ovf=tot[4], episodes=tot[5],
                     launches=self.launches)
 
+    def last_step_outputs(self, steps):
+        """On the host: what the last actor step of device_steps(steps) returned to its caller - obs, reward and done of
+        every env, and the actions in force during that step.  Valid until the next device_steps call."""
+        j = launch_plan(0, steps, self.spl)[-1][0] - 1 if self.multi else 0      # its slot in the last launch's outputs
+        self.c.torch.cuda.synchronize()
+        return {"obs": self.d_obs[j].cpu().numpy(), "reward": self.d_rew[j].cpu().numpy(),
+                "done": self.d_done[j].cpu().numpy(), "actions": self.d_act.cpu().numpy()}
+
     def timed_host(self, steps, warmup, wire=False, agent=False):
         """agent=True: actions come from the host every decision (host_steps_agent); else the controller runs in the kernel."""
         c, env = self.c, self.env
@@ -738,6 +769,8 @@ def b200_arm(a):
     occ = run.occupancy()
     d = run.timed_device(a.steps, a.warmup)
     mark = sampler.mark()
+    if a.dump_outputs and c.rank == 0:
+        dump_outputs(a.dump_outputs, run.last_step_outputs(a.steps))
     ms_max, n_launch = d["ms"], d["launches"]
     vu_all, ticks_all, asteps_all, gen_all, ovf_all = d["vu"], d["ticks"], d["asteps"], d["gen"], d["ovf"]
     loc = d["local"]

@@ -5,6 +5,8 @@ import json
 import os
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import bench  # noqa: E402
@@ -73,3 +75,28 @@ def test_launch_plan_keeps_decisions_on_the_same_steps():
                 assert decisions == [t for t in range(s0, s0 + n) if t % sp == 0]
     assert bench.launch_plan(0, 21, 6) == [(6, "greedy"), (6, "greedy"), (6, "greedy"), (3, "greedy")]
     assert bench.launch_plan(4, 10, 6) == [(2, "given"), (6, "greedy"), (2, "greedy")]
+
+
+def test_dump_outputs_rows_and_budget(tmp_path):
+    """bench.dump_outputs: every array as float32 .npy holding the same env rows (listed in env_index.npy, float64) -
+    all of them when they fit the byte budget, else a seeded sample that is the same every time - within the budget."""
+    rng = np.random.RandomState(1)
+    E = 1000
+    arrays = {"obs": rng.rand(E, 81).astype(np.float32), "reward": rng.rand(E, 9).astype(np.float32),
+              "done": rng.randint(2, size=E).astype(np.uint8), "actions": rng.randint(2, size=(E, 9)).astype(np.uint8)}
+    for budget in (10 ** 6, 10 ** 5):
+        dumps = []
+        for rep in range(2):
+            out = tmp_path / ("%d_%d" % (budget, rep))
+            bench.dump_outputs(str(out), arrays, max_bytes=budget)
+            assert sorted(os.listdir(out)) == sorted(n + ".npy" for n in list(arrays) + ["env_index"])
+            assert sum(os.path.getsize(out / f) for f in os.listdir(out)) <= budget
+            idx = np.load(out / "env_index.npy")
+            assert idx.dtype == np.float64 and (np.diff(idx) > 0).all() and 0 <= idx[0] and idx[-1] < E
+            rows = idx.astype(np.int64)
+            for name, arr in arrays.items():
+                got = np.load(out / (name + ".npy"))
+                assert got.dtype == np.float32 and (got == arr[rows]).all()
+            dumps.append(rows)
+        assert (dumps[0] == dumps[1]).all()
+        assert (len(dumps[0]) == E) == (budget == 10 ** 6) and len(dumps[0]) > E // 10
