@@ -185,6 +185,8 @@ const char *te_pool_last_error(te_pool *p);
 typedef struct te_wire_layout_t {
   int32_t stride, passed, detected, light, reward, done; /* byte offsets inside one record */
   int32_t max_k_ticks;
+  int32_t host_float_dma; /* 1: te_step(TE_HOST) has the copy engine write the float arrays instead of expanding
+                             wire records on the host (few host cores per GPU, or TE_HOST_FLOAT_DMA=1 at te_create) */
 } te_wire_layout_t;
 int te_wire_layout(const te_handle *h, te_wire_layout_t *out);
 int te_step_wire(te_handle *h, const uint8_t *actions, int32_t k_ticks, void *records, int memspace, void *stream);

@@ -52,7 +52,8 @@ class TeStats(C.Structure):
 
 
 class TeWireLayout(C.Structure):
-    _fields_ = [(k, C.c_int32) for k in ("stride", "passed", "detected", "light", "reward", "done", "max_k_ticks")]
+    _fields_ = [(k, C.c_int32) for k in ("stride", "passed", "detected", "light", "reward", "done", "max_k_ticks",
+                                            "host_float_dma")]
 
 
 class TrafficB200Error(RuntimeError):

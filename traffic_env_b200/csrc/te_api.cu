@@ -12,6 +12,7 @@
 #include <cstring>
 #include <atomic>
 #include <condition_variable>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -41,23 +42,66 @@ static int fail(const char *fmt, ...) {
     if (e_ != cudaSuccess) return fail("%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
   } while (0)
 
-// ---- host side of the wire format (te_kernels.cuh: wire_stride_bytes): expand compact env records into the caller's
+// Owners of CUDA resources (handle members, test hooks): each frees its resource when it goes.
+struct DeviceMem {
+  static cudaError_t alloc(void **p, size_t bytes) { return cudaMalloc(p, bytes); }
+  void operator()(void *p) const { cudaFree(p); }
+};
+struct PinnedMem {
+  static cudaError_t alloc(void **p, size_t bytes) { return cudaHostAlloc(p, bytes, cudaHostAllocDefault); }
+  void operator()(void *p) const { cudaFreeHost(p); }
+};
+struct StreamDestroy { void operator()(cudaStream_t s) const { cudaStreamDestroy(s); } };
+struct EventDestroy { void operator()(cudaEvent_t e) const { cudaEventDestroy(e); } };
+template <typename T> using dev_buf = std::unique_ptr<T[], DeviceMem>;       // device memory
+template <typename T> using pinned_buf = std::unique_ptr<T[], PinnedMem>;    // page-locked host memory
+using stream_ptr = std::unique_ptr<CUstream_st, StreamDestroy>;
+using event_ptr = std::unique_ptr<CUevent_st, EventDestroy>;
+
+// (Re)allocation of n elements (16 bytes at least); the old buffer is freed first.
+template <typename T, typename Mem> static cudaError_t alloc(std::unique_ptr<T[], Mem> &b, size_t n) {
+  b.reset();
+  void *p = nullptr;
+  const cudaError_t e = Mem::alloc(&p, n * sizeof(T) > 0 ? n * sizeof(T) : 16);
+  b.reset(e == cudaSuccess ? static_cast<T *>(p) : nullptr);
+  return e;
+}
+static cudaError_t create(stream_ptr &s) {
+  cudaStream_t raw = nullptr;
+  const cudaError_t e = cudaStreamCreateWithFlags(&raw, cudaStreamNonBlocking);
+  s.reset(e == cudaSuccess ? raw : nullptr);
+  return e;
+}
+static cudaError_t create(event_ptr &ev, unsigned flags = cudaEventDisableTiming) {
+  cudaEvent_t raw = nullptr;
+  const cudaError_t e = cudaEventCreateWithFlags(&raw, flags);
+  ev.reset(e == cudaSuccess ? raw : nullptr);
+  return e;
+}
+
+// A staging buffer replaced by one of n elements (zeroed when asked) once the device is idle: steps queued on other
+// streams may still use the old one.
+template <typename Buf> static int grow(Buf &b, size_t n, bool zero = false) {
+  CU(cudaDeviceSynchronize());
+  CU(alloc(b, n));
+  if (zero) CU(cudaMemset(b.get(), 0, n * sizeof(*b.get())));
+  return 0;
+}
+
+// ---- host side of the wire format (te_kernels.cuh: wire_layout): expand compact env records into the caller's
 // float observation / reward / done arrays (te_host.cpp).  The work is memory-bound and overlapped with the simulation
 // of the following slices (ExpandPool).
-void te_expand_records_host(const unsigned char *recs, int r, int I, int stride, long long n, float *obs, float *reward,
-                            uint8_t *done);   // te_host.cpp
-static void expand_records(const unsigned char *recs, int r, int I, int stride, long long n, float *obs, float *reward,
-                           uint8_t *done) {
-  te_expand_records_host(recs, r, I, stride, n, obs, reward, done);
-}
+void te_expand_records_host(const unsigned char *recs, const te_wire_layout_t &wl, int r, int I, long long n, float *obs,
+                            float *reward, uint8_t *done);   // te_host.cpp
 
 // A few helper threads per handle that wait for a slice's device-to-host copy (CUDA event) and expand it while the
 // GPU simulates the next slices.  Slices are dealt round-robin; the calling thread takes its share too.
 struct ExpandJob {
   const unsigned char *recs; float *obs, *reward; uint8_t *done;
   const uint8_t *mask;           // nullable (host pointer): only envs with a non-zero byte were stepped
-  int r, I, stride, nslice, per, E, nsteps;
-  cudaEvent_t *copied;
+  te_wire_layout_t wl;
+  int r, I, nslice, per, E, nsteps;
+  const event_ptr *copied;
 };
 struct ExpandPool {
   std::vector<std::thread> workers;
@@ -71,18 +115,18 @@ struct ExpandPool {
 
   void run_share(const ExpandJob &j, int tid) {
     for (int k = tid; k < j.nslice; k += nthreads) {
-      if (cudaEventSynchronize(j.copied[k]) != cudaSuccess) { failed.store(1); continue; }
+      if (cudaEventSynchronize(j.copied[k].get()) != cudaSuccess) { failed.store(1); continue; }
       const int e0 = k * j.per, ne = std::min(j.per, j.E - e0);
       if (ne <= 0) continue;
       const int ol = 2 * j.r + j.I;
       for (int st = 0; st < j.nsteps; st++) {
         const size_t eo = (size_t)st * j.E + e0;       // [nsteps][E] env slots
         if (!j.mask) {
-          expand_records(j.recs + eo * j.stride, j.r, j.I, j.stride, ne, j.obs + eo * ol, j.reward + eo * j.I, j.done + eo);
+          te_expand_records_host(j.recs + eo * j.wl.stride, j.wl, j.r, j.I, ne, j.obs + eo * ol, j.reward + eo * j.I, j.done + eo);
         } else {
           for (int e = 0; e < ne; e++)
             if (j.mask[e0 + e])
-              expand_records(j.recs + (eo + e) * j.stride, j.r, j.I, j.stride, 1, j.obs + (eo + e) * ol, j.reward + (eo + e) * j.I, j.done + eo + e);
+              te_expand_records_host(j.recs + (eo + e) * j.wl.stride, j.wl, j.r, j.I, 1, j.obs + (eo + e) * ol, j.reward + (eo + e) * j.I, j.done + eo + e);
         }
       }
     }
@@ -115,53 +159,55 @@ struct ExpandPool {
     { std::unique_lock<std::mutex> lk(mu); cv_done.wait(lk, [&] { return pending == 0; }); }
     return failed.load() == 0;
   }
-  void shutdown() {
+  ~ExpandPool() {
     { std::lock_guard<std::mutex> lk(mu); stop = true; }
     cv_go.notify_all();
     for (std::thread &t : workers) t.join();
-    workers.clear();
   }
 };
 
+// Members go in reverse order of declaration: the helper threads stop before the page-locked records they read are
+// freed, and every event and buffer goes before the streams.
 struct te_handle {
-  te_config cfg;
-  int V, r, R, Rp, I, n_entry;
-  int device;
-  cudaStream_t stream, stream2, stream_copy;
-  cudaEvent_t ev0, ev1, ev_fork, ev_join, ev_copied, ev_slice[64];
-  bool timed;
-  StepParams base;  // everything except per-call pointers
+  te_config cfg = {};
+  int V = 0, r = 0, R = 0, Rp = 0, I = 0, n_entry = 0;
+  int device = 0;
+  stream_ptr stream, stream2, stream_copy;
+  event_ptr ev0, ev1, ev_fork, ev_join, ev_copied, ev_slice[64], ev_copy[64];
+  bool timed = false;
+  StepParams base = {};  // everything except per-call pointers
   std::vector<int> dest, nexts, phases, entry;
   // device buffers
-  float *x, *v;
-  int *elapsed;
-  uint8_t *phase, *passed_dst;
-  EnvScalars *env;
-  DeviceStats *stats;
-  short *d_nexts, *d_up;
-  signed char *d_entry_idx;
-  long long *d_sched_off;
-  short *d_sched_roads;
-  uint32_t *d_gap_cdf;
-  IdmConst *d_idm;
+  dev_buf<float> x, v;
+  dev_buf<int> elapsed;
+  dev_buf<uint8_t> phase, passed_dst;
+  dev_buf<EnvScalars> env;
+  dev_buf<DeviceStats> stats;
+  dev_buf<short> d_nexts, d_up;
+  dev_buf<signed char> d_entry_idx;
+  dev_buf<long long> d_sched_off;
+  dev_buf<short> d_sched_roads;
+  dev_buf<uint32_t> d_gap_cdf;
+  dev_buf<IdmConst> d_idm;
   // staging for TE_HOST calls
-  uint8_t *d_actions, *d_done, *d_mask, *d_init_phase;
-  float *d_obs_f, *d_reward;
-  int *d_obs_i, *d_cars;
-  float *w; TripRecord *d_trips; unsigned long long *d_trip_count; long long trip_cap;
-  int warps;
-  int G, threads;        // env instances per CTA, threads per CTA (G * R rounded up to whole warps)
-  int smem_optin;
+  dev_buf<uint8_t> d_actions, d_done, d_mask, d_init_phase;
+  dev_buf<float> d_reward;
+  dev_buf<int> d_obs_i, d_cars;   // d_obs_i: raw observations, or (read as float) fused ones: never live together
+  dev_buf<float> w; dev_buf<TripRecord> d_trips; dev_buf<unsigned long long> d_trip_count; long long trip_cap = 0;
+  int warps = 0;
+  int G = 1, threads = 0;        // env instances per CTA, threads per CTA (G * R rounded up to whole warps)
+  int smem_optin = 0;
   // wire path of the host API
-  unsigned char *d_wire, *h_wire;   // [E][wire_stride] device / page-locked host
-  int wire_stride, host_slices, wire_steps, float_steps;
-  bool tame;             // every car the device has seen is tame (te_math.cuh: CHECKED = false may run)
-  float v_cap;           // speed bound of the tame domain for this archetype (tame_archetype)
-  int ctrl_spacing;      // TE_CTRL_GREEDY: a new decision every so many actor steps inside a te_step_multi launch (0: one per launch)
-  int actions_cap;       // decisions d_actions has room for
-  bool float_dma;        // te_step(TE_HOST) with float outputs: let the copy engine write the float arrays (no host expansion)
-  cudaEvent_t ev_copy[64];
-  ExpandPool *pool;
+  dev_buf<unsigned char> d_wire; pinned_buf<unsigned char> h_wire;   // [steps][E][wire_stride] device / page-locked host
+  int wire_stride = 0, host_slices = 1;
+  int wire_steps = 1, float_steps = 1;   // actor steps the wire records / float staging have room for
+  bool tame = false;     // every car the device has seen is tame (te_math.cuh: CHECKED = false may run)
+  float v_cap = 0.f;     // speed bound of the tame domain for this archetype (tame_archetype)
+  int ctrl_spacing = 0;  // TE_CTRL_GREEDY: a new decision every so many actor steps inside a te_step_multi launch (0: one per launch)
+  int actions_cap = 1;   // decisions d_actions has room for
+  bool float_dma = false;  // te_step(TE_HOST) with float outputs: let the copy engine write the float arrays (no host expansion)
+  std::unique_ptr<ExpandPool> pool;
+  ~te_handle() { cudaSetDevice(device); }
 };
 
 // One thread per (padded) road.  A kernel variant is compiled per row capacity MAXT >= Rp (its shared-memory layout
@@ -319,41 +365,13 @@ static std::vector<uint32_t> build_gap_cdf(double cars_per_tick) {
   return t;
 }
 
-static void free_handle(te_handle *h) {
-  if (!h) return;
-  cudaSetDevice(h->device);
-  if (h->pool) { h->pool->shutdown(); delete h->pool; h->pool = nullptr; }
-  if (h->d_wire) cudaFree(h->d_wire);
-  if (h->h_wire) cudaFreeHost(h->h_wire);
-  for (cudaEvent_t e : h->ev_copy) if (e) cudaEventDestroy(e);
-  void *ptrs[] = {h->w, h->x, h->v, h->elapsed, h->phase, h->passed_dst, h->env, h->stats, h->d_nexts, h->d_up,
-                  h->d_entry_idx, h->d_sched_off, h->d_sched_roads, h->d_gap_cdf, h->d_idm, h->d_actions,
-                  h->d_done, h->d_mask, h->d_init_phase, h->d_reward, h->d_obs_i /* d_obs_f aliases it */, h->d_cars,
-                  h->d_trips, h->d_trip_count};
-  for (void *p : ptrs) if (p) cudaFree(p);
-  if (h->ev0) cudaEventDestroy(h->ev0);
-  if (h->ev1) cudaEventDestroy(h->ev1);
-  if (h->ev_fork) cudaEventDestroy(h->ev_fork);
-  if (h->ev_join) cudaEventDestroy(h->ev_join);
-  if (h->ev_copied) cudaEventDestroy(h->ev_copied);
-  for (cudaEvent_t e : h->ev_slice) if (e) cudaEventDestroy(e);
-  if (h->stream) cudaStreamDestroy(h->stream);
-  if (h->stream2) cudaStreamDestroy(h->stream2);
-  if (h->stream_copy) cudaStreamDestroy(h->stream_copy);
-  delete h;
-}
-
-extern "C" int te_destroy(te_handle *h) { free_handle(h); return 0; }
-
-template <typename T>
-static cudaError_t dalloc(T **p, size_t n) { return cudaMalloc((void **)p, n * sizeof(T) > 0 ? n * sizeof(T) : 16); }
+extern "C" int te_destroy(te_handle *h) { delete h; return 0; }
 
 // Threads per CTA, env instances per CTA and the kernel variant of a handle; called by te_create and again when a
 // handle stops being tame (te_set_state with a wild car: the checked, one-env-per-CTA kernels take over).
 static int select_layout(te_handle *h) {
   const te_config *cfg = &h->cfg;
   StepParams &p = h->base;
-#define CUH(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return fail("%s failed: %s", #call, cudaGetErrorString(e_)); } while (0)
   // One thread per road.  Small grids put G env instances on one CTA (its rows are the G * R roads of those envs) so
   // that no lane is a padding lane and a warp's car list is long: G in 1..4 with at most 256 rows, chosen for the
   // fewest padding lanes (ties: the smaller G).  Default 3x3 grid: R = 48 -> G = 2, 96 threads, three warps.
@@ -369,20 +387,14 @@ static int select_layout(te_handle *h) {
       if (waste < best - 1e-9) { best = waste; h->G = g; h->threads = th; }
     }
   }
-  if (const char *ev = getenv("TE_ENVS_PER_CTA")) {   // study knob
-    const int g = atoi(ev);
-    if (g >= 1 && g <= 8 && g * h->R <= 256 && !validate && fast_arch(h)) { h->G = g; h->threads = g == 1 ? h->Rp : (g * h->R + 31) / 32 * 32; }
-  }
   h->warps = h->threads / GROUP_ROADS;
   p.G = h->G;
-  CUH(cudaDeviceGetAttribute(&h->smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
+  CU(cudaDeviceGetAttribute(&h->smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
   const StepVariant sv = step_variant_for(h->threads, validate, fast_arch(h), h->G > 1);
   if (h->threads > sv.maxt) { return fail("te_create: %d roads exceed the largest%s kernel variant (%d)", h->threads, validate ? " validate-mode" : "", sv.maxt); }
   const int smem_max = smem_bytes(sv.maxt, validate, MAX_K, h->n_entry, h->G);
   if (smem_max > h->smem_optin) { return fail("te_create: env needs %d B of shared memory, device allows %d", smem_max, h->smem_optin); }
-  CUH(cudaFuncSetAttribute(sv.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
-
-#undef CUH
+  CU(cudaFuncSetAttribute(sv.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
   return 0;
 }
 
@@ -412,21 +424,11 @@ extern "C" int te_create(const te_config *cfg, te_handle **out) {
   if (e != cudaSuccess || ndev == 0)
     return fail("te_create: no CUDA device (%s); this library has no CPU path", cudaGetErrorString(e));
   if (cfg->device < 0 || cfg->device >= ndev) return fail("te_create: device %d out of range", cfg->device);
-  te_handle *h = new te_handle();
-  memset((void *)&h->base, 0, sizeof(h->base));
+  std::unique_ptr<te_handle> owner(new te_handle());   // frees whatever was set up when te_create fails
+  te_handle *h = owner.get();
   h->cfg = *cfg; h->device = cfg->device;
-  h->x = h->v = h->w = nullptr; h->elapsed = nullptr; h->phase = h->passed_dst = nullptr; h->env = nullptr; h->stats = nullptr;
-  h->d_nexts = h->d_up = nullptr; h->d_entry_idx = nullptr; h->d_sched_off = nullptr;
-  h->d_sched_roads = nullptr; h->d_gap_cdf = nullptr; h->d_idm = nullptr; h->d_actions = h->d_done = h->d_mask = h->d_init_phase = nullptr;
-  h->d_obs_f = h->d_reward = nullptr; h->d_obs_i = h->d_cars = nullptr; h->d_trips = nullptr; h->d_trip_count = nullptr;
-  h->stream = h->stream2 = h->stream_copy = nullptr; h->ev0 = h->ev1 = h->ev_fork = h->ev_join = h->ev_copied = nullptr;
-  for (cudaEvent_t &e : h->ev_slice) e = nullptr;
-  for (cudaEvent_t &e : h->ev_copy) e = nullptr;
-  h->d_wire = h->h_wire = nullptr; h->pool = nullptr; h->wire_stride = 0; h->host_slices = 1; h->wire_steps = 0; h->float_steps = 1;
-  h->timed = false; h->trip_cap = 0;
-#define CUH(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { free_handle(h); return fail("%s failed: %s", #call, cudaGetErrorString(e_)); } } while (0)
-  CUH(cudaSetDevice(h->device));
-  CUH(upload_math_consts());
+  CU(cudaSetDevice(h->device));
+  CU(upload_math_consts());
   const int m = cfg->m, n = cfg->n;
   h->V = m * n; h->I = h->V; h->r = 4 * h->V; h->R = h->r + 2 * n + 2 * m;
   h->Rp = (h->R + GROUP_ROADS - 1) / GROUP_ROADS * GROUP_ROADS;
@@ -436,10 +438,6 @@ extern "C" int te_create(const te_config *cfg, te_handle **out) {
     // 10x10 grid: 440 roads -> 512 threads, 16 warps, 64 registers: +1.7 % (measured A/B, 3 runs each).
     const int rp128 = (h->R + 127) / 128 * 128;
     if (rp128 * 5 <= h->R * 6) h->Rp = rp128;
-  }
-  if (const char *ev = getenv("TE_RP_ALIGN")) {   // study knob: pad the CTA to a multiple of this many threads
-    const int al = atoi(ev);
-    if (al >= 32 && al % 32 == 0 && al <= 1024) h->Rp = (h->R + al - 1) / al * al;
   }
   // topology (roadgraph.py:35-39, 42-51)
   h->dest.resize(h->R); h->nexts.resize(h->R); h->phases.resize(h->R);
@@ -452,7 +450,7 @@ extern "C" int te_create(const te_config *cfg, te_handle **out) {
     nx[i] = (short)h->nexts[i];
   }
   for (int i = 0; i < h->R; i++) if (h->nexts[i] >= 0) {
-    if (up[h->nexts[i]] != -1) { free_handle(h); return fail("te_create: successor table is not injective"); }
+    if (up[h->nexts[i]] != -1) return fail("te_create: successor table is not injective");
     up[h->nexts[i]] = (short)i;
   }
   const uint32_t spec = cfg->entry_spec;
@@ -462,41 +460,35 @@ extern "C" int te_create(const te_config *cfg, te_handle **out) {
   if (((spec >> 2) & 1) == 0) for (int i = 0; i < n; i++) h->entry.push_back(2 * v + i);
   if (((spec >> 3) & 1) == 0) for (int i = 0; i < n; i++) h->entry.push_back(3 * v + n * (m - 1) + i);
   h->n_entry = (int)h->entry.size();
-  if (h->n_entry > 127) { free_handle(h); return fail("te_create: more than 127 entry roads"); }
+  if (h->n_entry > 127) return fail("te_create: more than 127 entry roads");
   for (int k = 0; k < h->n_entry; k++) eidx[h->entry[k]] = (signed char)k;
 
   const size_t E = (size_t)cfg->num_envs;
-  CUH(cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
-  CUH(cudaStreamCreateWithFlags(&h->stream2, cudaStreamNonBlocking));
-  CUH(cudaStreamCreateWithFlags(&h->stream_copy, cudaStreamNonBlocking));
-  CUH(cudaEventCreateWithFlags(&h->ev_copied, cudaEventDisableTiming));
-  for (cudaEvent_t &e : h->ev_slice) CUH(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-  for (cudaEvent_t &e : h->ev_copy) CUH(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-  CUH(cudaEventCreate(&h->ev0)); CUH(cudaEventCreate(&h->ev1));
-  CUH(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
-  CUH(cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
-  CUH(dalloc(&h->x, E * h->Rp * CAP)); CUH(dalloc(&h->v, E * h->Rp * CAP));
+  CU(create(h->stream)); CU(create(h->stream2)); CU(create(h->stream_copy));
+  CU(create(h->ev_copied));
+  for (event_ptr &e : h->ev_slice) CU(create(e));
+  for (event_ptr &e : h->ev_copy) CU(create(e));
+  CU(create(h->ev0, cudaEventDefault)); CU(create(h->ev1, cudaEventDefault));
+  CU(create(h->ev_fork)); CU(create(h->ev_join));
+  CU(alloc(h->x, E * h->Rp * CAP)); CU(alloc(h->v, E * h->Rp * CAP));
   if (cfg->flags & TE_VALIDATE) {
-    CUH(dalloc(&h->w, E * h->Rp * CAP));
-    CUH(cudaMemset(h->w, 0, E * h->Rp * CAP * sizeof(float)));
+    CU(alloc(h->w, E * h->Rp * CAP));
+    CU(cudaMemset(h->w.get(), 0, E * h->Rp * CAP * sizeof(float)));
     h->trip_cap = std::max<long long>(1ll << 20, 64ll * (long long)E);
-    CUH(dalloc(&h->d_trips, (size_t)h->trip_cap)); CUH(dalloc(&h->d_trip_count, 1));
-    CUH(cudaMemset(h->d_trip_count, 0, sizeof(unsigned long long)));
+    CU(alloc(h->d_trips, (size_t)h->trip_cap)); CU(alloc(h->d_trip_count, 1));
+    CU(cudaMemset(h->d_trip_count.get(), 0, sizeof(unsigned long long)));
   }
-  CUH(dalloc(&h->elapsed, E * h->I)); CUH(dalloc(&h->phase, E * h->I)); CUH(dalloc(&h->passed_dst, E * h->I));
-  CUH(dalloc(&h->env, E)); CUH(dalloc(&h->stats, 1));
-  CUH(dalloc(&h->d_nexts, (size_t)h->Rp)); CUH(dalloc(&h->d_up, (size_t)h->Rp));
-  CUH(dalloc(&h->d_entry_idx, (size_t)h->Rp));
-  CUH(dalloc(&h->d_actions, E * h->I)); CUH(dalloc(&h->d_done, E)); CUH(dalloc(&h->d_mask, E));
-  h->actions_cap = 1; h->ctrl_spacing = 0;
-  CUH(dalloc(&h->d_init_phase, E * h->I));
-  CUH(dalloc(&h->d_obs_i, E * (2 * h->r + 2 * h->I)));
-  CUH(dalloc(&h->d_reward, E * h->I));
-  h->d_obs_f = reinterpret_cast<float *>(h->d_obs_i);  // raw and fused observations are never live together
-  h->wire_stride = wire_stride_bytes(h->r, h->I);
-  CUH(dalloc(&h->d_wire, E * (size_t)h->wire_stride));
-  CUH(cudaHostAlloc((void **)&h->h_wire, E * (size_t)h->wire_stride, cudaHostAllocDefault));
-  h->wire_steps = 1;
+  CU(alloc(h->elapsed, E * h->I)); CU(alloc(h->phase, E * h->I)); CU(alloc(h->passed_dst, E * h->I));
+  CU(alloc(h->env, E)); CU(alloc(h->stats, 1));
+  CU(alloc(h->d_nexts, (size_t)h->Rp)); CU(alloc(h->d_up, (size_t)h->Rp));
+  CU(alloc(h->d_entry_idx, (size_t)h->Rp));
+  CU(alloc(h->d_actions, E * h->I)); CU(alloc(h->d_done, E)); CU(alloc(h->d_mask, E));
+  CU(alloc(h->d_init_phase, E * h->I));
+  CU(alloc(h->d_obs_i, E * (2 * h->r + 2 * h->I)));
+  CU(alloc(h->d_reward, E * h->I));
+  h->wire_stride = wire_layout(h->r, h->I).stride;
+  CU(alloc(h->d_wire, E * (size_t)h->wire_stride));
+  CU(alloc(h->h_wire, E * (size_t)h->wire_stride));
   {
     // Host path: the batch is launched in slices (te_step, TE_HOST) and a few helper threads expand the compact
     // records of finished slices into the caller's float arrays meanwhile.  TE_HOST_SLICES / TE_HOST_THREADS tune it.
@@ -510,7 +502,7 @@ extern "C" int te_create(const te_config *cfg, te_handle **out) {
     if ((size_t)cfg->num_envs * (size_t)(2 * h->r) < (1u << 20)) nthr = 1;   // small batches: not worth waking anybody
     if (const char *ev = getenv("TE_HOST_THREADS")) { const int v = atoi(ev); if (v >= 1 && v <= 64) nthr = v; }
     if (nthr > nslice) nthr = nslice;
-    h->pool = new ExpandPool();
+    h->pool.reset(new ExpandPool());
     h->pool->start(h->device, nthr);
     // Float outputs in host memory can travel two ways: as wire records expanded by the helper threads (fewer PCIe
     // bytes; needs ~4 spare cores per GPU: measured 0.91 of the device rate on a 16-core / 1-GPU box, 0.51 with 8 ranks
@@ -520,26 +512,26 @@ extern "C" int te_create(const te_config *cfg, te_handle **out) {
     h->float_dma = hw && ndev > 0 && hw / (unsigned)ndev < 8;
     if (const char *ev = getenv("TE_HOST_FLOAT_DMA")) h->float_dma = atoi(ev) != 0;
   }
-  CUH(cudaMemcpy(h->d_nexts, nx.data(), nx.size() * sizeof(short), cudaMemcpyHostToDevice));
-  CUH(cudaMemcpy(h->d_up, up.data(), up.size() * sizeof(short), cudaMemcpyHostToDevice));
-  CUH(cudaMemcpy(h->d_entry_idx, eidx.data(), eidx.size(), cudaMemcpyHostToDevice));
-  CUH(cudaMemset(h->stats, 0, sizeof(DeviceStats)));
-  CUH(cudaMemset(h->x, 0, E * h->Rp * CAP * sizeof(float)));
-  CUH(cudaMemset(h->v, 0, E * h->Rp * CAP * sizeof(float)));
-  CUH(cudaMemset(h->elapsed, 0, E * h->I * sizeof(int)));
-  CUH(cudaMemset(h->phase, 0, E * h->I)); CUH(cudaMemset(h->passed_dst, 0, E * h->I));
-  CUH(cudaMemset(h->d_done, 0, E));
+  CU(cudaMemcpy(h->d_nexts.get(), nx.data(), nx.size() * sizeof(short), cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(h->d_up.get(), up.data(), up.size() * sizeof(short), cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(h->d_entry_idx.get(), eidx.data(), eidx.size(), cudaMemcpyHostToDevice));
+  CU(cudaMemset(h->stats.get(), 0, sizeof(DeviceStats)));
+  CU(cudaMemset(h->x.get(), 0, E * h->Rp * CAP * sizeof(float)));
+  CU(cudaMemset(h->v.get(), 0, E * h->Rp * CAP * sizeof(float)));
+  CU(cudaMemset(h->elapsed.get(), 0, E * h->I * sizeof(int)));
+  CU(cudaMemset(h->phase.get(), 0, E * h->I)); CU(cudaMemset(h->passed_dst.get(), 0, E * h->I));
+  CU(cudaMemset(h->d_done.get(), 0, E));
 
   std::vector<uint32_t> cdf = build_gap_cdf(cfg->cars_per_tick);
   if (cfg->arrival_mode == TE_ARRIVALS_PHILOX && (cdf.empty() || h->n_entry == 0)) {
-    free_handle(h); return fail("te_create: Philox arrivals need cars_per_tick > 0 and at least one entry road");
+    return fail("te_create: Philox arrivals need cars_per_tick > 0 and at least one entry road");
   }
   if (cfg->arrival_mode == TE_ARRIVALS_PHILOX && cfg->cars_per_tick > 16.0 * h->n_entry) {
     // per-tick per-road arrival counts are 8-bit; a ring holds 18 cars anyway
-    free_handle(h); return fail("te_create: cars_per_tick %.1f is beyond what %d entry roads can take", cfg->cars_per_tick, h->n_entry);
+    return fail("te_create: cars_per_tick %.1f is beyond what %d entry roads can take", cfg->cars_per_tick, h->n_entry);
   }
-  CUH(dalloc(&h->d_gap_cdf, cdf.size()));
-  if (!cdf.empty()) CUH(cudaMemcpy(h->d_gap_cdf, cdf.data(), cdf.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
+  CU(alloc(h->d_gap_cdf, cdf.size()));
+  if (!cdf.empty()) CU(cudaMemcpy(h->d_gap_cdf.get(), cdf.data(), cdf.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
 
   // per-env scalars; the Philox stream draws its first gap at seeding time, like poisson() does on first next()
   std::vector<EnvScalars> es(E);
@@ -547,7 +539,7 @@ extern "C" int te_create(const te_config *cfg, te_handle **out) {
     memset(&es[i], 0, sizeof(EnvScalars));
     es[i].ep_mult = 1.0;
   }
-  CUH(cudaMemcpy(h->env, es.data(), E * sizeof(EnvScalars), cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(h->env.get(), es.data(), E * sizeof(EnvScalars), cudaMemcpyHostToDevice));
 
   StepParams &p = h->base;
   p.V = h->V; p.r = h->r; p.R = h->R; p.Rp = h->Rp; p.I = h->I; p.n_entry = h->n_entry;
@@ -562,23 +554,24 @@ extern "C" int te_create(const te_config *cfg, te_handle **out) {
   p.gamma = cfg->gamma;
   fill_idm(p.idm, cfg->archetype, cfg->rate);
   h->tame = tame_archetype(cfg, &h->v_cap);
-  CUH(dalloc(&h->d_idm, 1));
-  CUH(cudaMemcpy(h->d_idm, &p.idm, sizeof(IdmConst), cudaMemcpyHostToDevice));
-  p.idm_g = h->d_idm;
-  p.x = h->x; p.v = h->v; p.w = h->w; p.trips = h->d_trips; p.trip_count = h->d_trip_count; p.trip_cap = h->trip_cap;
-  p.elapsed = h->elapsed; p.phase = h->phase; p.passed_dst = h->passed_dst;
-  p.env = h->env; p.stats = h->stats; p.nexts = h->d_nexts; p.up = h->d_up; p.entry_idx = h->d_entry_idx;
-  p.gap_cdf = h->d_gap_cdf; p.n_gap = (int)cdf.size();
+  CU(alloc(h->d_idm, 1));
+  CU(cudaMemcpy(h->d_idm.get(), &p.idm, sizeof(IdmConst), cudaMemcpyHostToDevice));
+  p.idm_g = h->d_idm.get();
+  p.x = h->x.get(); p.v = h->v.get(); p.w = h->w.get(); p.trips = h->d_trips.get(); p.trip_count = h->d_trip_count.get(); p.trip_cap = h->trip_cap;
+  p.elapsed = h->elapsed.get(); p.phase = h->phase.get(); p.passed_dst = h->passed_dst.get();
+  p.env = h->env.get(); p.stats = h->stats.get(); p.nexts = h->d_nexts.get(); p.up = h->d_up.get(); p.entry_idx = h->d_entry_idx.get();
+  p.gap_cdf = h->d_gap_cdf.get(); p.n_gap = (int)cdf.size();
   p.seed = (uint32_t)(cfg->seed ^ (cfg->seed >> 32)); p.env_id_base = cfg->env_id_base;
   p.sched_off = nullptr; p.sched_roads = nullptr; p.horizon = 0; p.sched_first = 0;
   p.nsteps = 1; p.controller = CTRL_GIVEN; p.actions_out = nullptr; p.env_mask = nullptr; p.decide_every = 0;
 
-  if (int rc = select_layout(h)) { free_handle(h); return rc; }
+  if (int rc = select_layout(h)) return rc;
 
   // as-if-reset initial state with all-zero phases (the reference leaves state undefined before reset())
-  te_reset_kernel<<<(cfg->num_envs + RESET_ENVS_PER_CTA - 1) / RESET_ENVS_PER_CTA, 128, 0, h->stream>>>(p, nullptr, nullptr, 0);
-  CUH(cudaGetLastError());
-  CUH(cudaMemsetAsync(h->phase, 0, E * h->I, h->stream));
+  cudaStream_t st = h->stream.get();
+  te_reset_kernel<<<(cfg->num_envs + RESET_ENVS_PER_CTA - 1) / RESET_ENVS_PER_CTA, 128, 0, st>>>(p, nullptr, nullptr, 0);
+  CU(cudaGetLastError());
+  CU(cudaMemsetAsync(h->phase.get(), 0, E * h->I, st));
   // seed the arrival stream (draw 0 is the initial gap)
   if (cfg->arrival_mode == TE_ARRIVALS_PHILOX) {
     // done on the host: one Philox block per env, identical integer arithmetic
@@ -595,13 +588,12 @@ extern "C" int te_create(const te_config *cfg, te_handle **out) {
       while (lo < hi) { const size_t mid = (lo + hi) / 2; if (cdf[mid] <= c[0]) lo = mid + 1; else hi = mid; }
       es[i].ph_skip = (uint32_t)lo; es[i].ph_draw = 1; es[i].reset_count = 1;
     }
-    CUH(cudaStreamSynchronize(h->stream));
-    CUH(cudaMemcpy(h->env, es.data(), E * sizeof(EnvScalars), cudaMemcpyHostToDevice));
+    CU(cudaStreamSynchronize(st));
+    CU(cudaMemcpy(h->env.get(), es.data(), E * sizeof(EnvScalars), cudaMemcpyHostToDevice));
   }
-  CUH(cudaStreamSynchronize(h->stream));
-  CUH(cudaDeviceSynchronize());   // the blocking table / scalar uploads above are complete before any stream steps
-#undef CUH
-  *out = h;
+  CU(cudaStreamSynchronize(st));
+  CU(cudaDeviceSynchronize());   // the blocking table / scalar uploads above are complete before any stream steps
+  *out = owner.release();
   return 0;
 }
 
@@ -622,7 +614,7 @@ extern "C" int te_get_topology(const te_handle *h, int32_t *dest, int32_t *nexts
   return 0;
 }
 
-static cudaStream_t pick_stream(te_handle *h, void *stream) { return stream ? (cudaStream_t)stream : h->stream; }
+static cudaStream_t pick_stream(te_handle *h, void *stream) { return stream ? (cudaStream_t)stream : h->stream.get(); }
 
 extern "C" int te_reset(te_handle *h, const uint8_t *env_mask, const uint8_t *init_phase, int memspace, void *stream) {
   if (!h) return fail("te_reset: null handle");
@@ -631,8 +623,8 @@ extern "C" int te_reset(te_handle *h, const uint8_t *env_mask, const uint8_t *in
   const size_t E = (size_t)h->cfg.num_envs;
   const uint8_t *dm = env_mask, *dp = init_phase;
   if (memspace == TE_HOST) {
-    if (env_mask) { CU(cudaMemcpyAsync(h->d_mask, env_mask, E, cudaMemcpyHostToDevice, st)); dm = h->d_mask; }
-    if (init_phase) { CU(cudaMemcpyAsync(h->d_init_phase, init_phase, E * h->I, cudaMemcpyHostToDevice, st)); dp = h->d_init_phase; }
+    if (env_mask) { CU(cudaMemcpyAsync(h->d_mask.get(), env_mask, E, cudaMemcpyHostToDevice, st)); dm = h->d_mask.get(); }
+    if (init_phase) { CU(cudaMemcpyAsync(h->d_init_phase.get(), init_phase, E * h->I, cudaMemcpyHostToDevice, st)); dp = h->d_init_phase.get(); }
   }
   te_reset_kernel<<<(h->cfg.num_envs + RESET_ENVS_PER_CTA - 1) / RESET_ENVS_PER_CTA, 128, 0, st>>>(h->base, dm, dp, 0);
   CU(cudaGetLastError());
@@ -663,16 +655,15 @@ extern "C" int te_set_arrivals(te_handle *h, const int64_t *offsets, const int16
     if (roads[k] < 0 || roads[k] >= h->R || !is_entry[roads[k]]) return fail("te_set_arrivals: road %d is not an entry road", (int)roads[k]);
   // steps may still be queued on caller-provided streams (TE_DEVICE) and read the old schedule
   CU(cudaDeviceSynchronize());
-  if (h->d_sched_off) { cudaFree(h->d_sched_off); h->d_sched_off = nullptr; }
-  if (h->d_sched_roads) { cudaFree(h->d_sched_roads); h->d_sched_roads = nullptr; }
   h->base.sched_off = nullptr; h->base.sched_roads = nullptr; h->base.horizon = 0;
-  CU(dalloc(&h->d_sched_off, no)); CU(dalloc(&h->d_sched_roads, (size_t)(num_roads > 0 ? num_roads : 1)));
+  CU(alloc(h->d_sched_off, no)); CU(alloc(h->d_sched_roads, (size_t)(num_roads > 0 ? num_roads : 1)));
   static_assert(sizeof(long long) == sizeof(int64_t), "int64");
-  CU(cudaMemcpyAsync(h->d_sched_off, offsets, no * sizeof(int64_t), cudaMemcpyHostToDevice, h->stream));
-  if (num_roads > 0) CU(cudaMemcpyAsync(h->d_sched_roads, roads, (size_t)num_roads * sizeof(int16_t), cudaMemcpyHostToDevice, h->stream));
-  CU(cudaStreamSynchronize(h->stream));
+  cudaStream_t st = h->stream.get();
+  CU(cudaMemcpyAsync(h->d_sched_off.get(), offsets, no * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+  if (num_roads > 0) CU(cudaMemcpyAsync(h->d_sched_roads.get(), roads, (size_t)num_roads * sizeof(int16_t), cudaMemcpyHostToDevice, st));
+  CU(cudaStreamSynchronize(st));
   CU(cudaDeviceSynchronize());   // order the upload against every stream a later step may be launched on
-  h->base.sched_off = h->d_sched_off; h->base.sched_roads = h->d_sched_roads; h->base.horizon = horizon;
+  h->base.sched_off = h->d_sched_off.get(); h->base.sched_roads = h->d_sched_roads.get(); h->base.horizon = horizon;
   h->base.sched_first = first_tick;
   return 0;
 }
@@ -689,49 +680,143 @@ struct StepReq {
   const char *who = "te_step";
 };
 
-static int ensure_wire_steps(te_handle *h, int nsteps) {
-  if (nsteps <= h->wire_steps) return 0;
-  CU(cudaDeviceSynchronize());
-  const size_t bytes = (size_t)nsteps * h->cfg.num_envs * h->wire_stride;
-  if (h->d_wire) { cudaFree(h->d_wire); h->d_wire = nullptr; }
-  if (h->h_wire) { cudaFreeHost(h->h_wire); h->h_wire = nullptr; }
-  h->wire_steps = 0;
-  CU(dalloc(&h->d_wire, bytes));
-  CU(cudaHostAlloc((void **)&h->h_wire, bytes, cudaHostAllocDefault));
-  h->wire_steps = nsteps;
-  return 0;
+// Where a step's results go.  DEVICE: the caller's device buffers (te_step_wire: records).  WIRE: compact records
+// copied to host memory (te_step_wire's buffer, or the handle's, which its helper threads expand into the caller's
+// float arrays).  FLOATS: float (te_step_raw: int) arrays staged on the device and copied into the caller's arrays.
+enum class Route { DEVICE, WIRE, FLOATS };
+
+// Host float outputs travel as wire records unless the handle lets the copy engine write them (float_dma); a masked
+// step takes records whenever they fit, so that only the stepped envs are expanded.  Raw ticks and steps of more than
+// WIRE_MAX_K ticks do not fit a record.
+static Route pick_route(const te_handle *h, const StepReq &q) {
+  if (q.memspace != TE_HOST) return Route::DEVICE;
+  const bool wire = !q.raw && q.K <= WIRE_MAX_K && (q.wire_only || !h->float_dma || q.env_mask);
+  return wire ? Route::WIRE : Route::FLOATS;
 }
 
-// device staging of the float outputs of an n-step launch (host path without wire records)
-static int ensure_float_steps(te_handle *h, int nsteps) {
-  if (nsteps <= h->float_steps) return 0;
-  CU(cudaDeviceSynchronize());
+// controller decisions of a launch
+static int decisions(const StepParams &p) { return p.decide_every > 0 ? (p.nsteps + p.decide_every - 1) / p.decide_every : 1; }
+
+// The kernel parameters of a request on its route.  The host routes stage the inputs (actions, env mask) on `st` and
+// first grow the handle's staging buffers to the launch; a buffer's capacity reads 0 while it is being replaced.
+static int step_params(te_handle *h, const StepReq &q, Route route, cudaStream_t st, StepParams &p) {
+  const bool greedy = q.controller == CTRL_GREEDY;
+  p = h->base;
+  p.K = q.K; p.raw = q.raw; p.nsteps = q.nsteps; p.controller = q.controller;
+  p.decide_every = greedy ? h->ctrl_spacing : 0;
+  if (route == Route::DEVICE) {
+    p.actions = q.actions; p.actions_out = greedy ? const_cast<uint8_t *>(q.actions) : nullptr; p.env_mask = q.env_mask;
+    p.obs_f = (float *)q.obs; p.obs_i = (int *)q.obs; p.reward = q.reward; p.done = q.done;
+    if (q.wire_only) { p.wire = (unsigned char *)q.obs; p.wire_stride = h->wire_stride; }
+    return 0;
+  }
   const size_t E = (size_t)h->cfg.num_envs;
-  if (h->d_obs_i) { cudaFree(h->d_obs_i); h->d_obs_i = nullptr; h->d_obs_f = nullptr; }
-  if (h->d_reward) { cudaFree(h->d_reward); h->d_reward = nullptr; }
-  if (h->d_done) { cudaFree(h->d_done); h->d_done = nullptr; }
-  h->float_steps = 0;
-  CU(dalloc(&h->d_obs_i, (size_t)nsteps * E * (2 * h->r + 2 * h->I)));
-  CU(dalloc(&h->d_reward, (size_t)nsteps * E * h->I));
-  CU(dalloc(&h->d_done, (size_t)nsteps * E));
-  CU(cudaMemset(h->d_done, 0, (size_t)nsteps * E));
-  h->d_obs_f = reinterpret_cast<float *>(h->d_obs_i);
-  h->float_steps = nsteps;
+  const int ndec = decisions(p);
+  if (ndec > h->actions_cap) {
+    h->actions_cap = 0;
+    if (int rc = grow(h->d_actions, (size_t)ndec * E * h->I)) return rc;
+    h->actions_cap = ndec;
+  }
+  if (!greedy) CU(cudaMemcpyAsync(h->d_actions.get(), q.actions, E * h->I, cudaMemcpyHostToDevice, st));
+  if (q.env_mask) CU(cudaMemcpyAsync(h->d_mask.get(), q.env_mask, E, cudaMemcpyHostToDevice, st));
+  if (route == Route::WIRE && q.nsteps > h->wire_steps) {
+    const size_t n = (size_t)q.nsteps * E * h->wire_stride;
+    h->wire_steps = 0;
+    if (int rc = grow(h->d_wire, n)) return rc;
+    if (int rc = grow(h->h_wire, n)) return rc;
+    h->wire_steps = q.nsteps;
+  }
+  if (route == Route::FLOATS && q.nsteps > h->float_steps) {
+    const size_t n = (size_t)q.nsteps * E;
+    h->float_steps = 0;
+    if (int rc = grow(h->d_obs_i, n * (2 * h->r + 2 * h->I))) return rc;
+    if (int rc = grow(h->d_reward, n * h->I)) return rc;
+    if (int rc = grow(h->d_done, n, true)) return rc;
+    h->float_steps = q.nsteps;
+  }
+  p.actions = h->d_actions.get(); p.actions_out = greedy ? h->d_actions.get() : nullptr;
+  p.env_mask = q.env_mask ? h->d_mask.get() : nullptr;
+  p.obs_f = reinterpret_cast<float *>(h->d_obs_i.get()); p.obs_i = h->d_obs_i.get();
+  p.reward = h->d_reward.get(); p.done = h->d_done.get();
+  if (route == Route::WIRE) { p.wire = h->d_wire.get(); p.wire_stride = h->wire_stride; }
   return 0;
 }
 
-// room for the decisions of one launch in the device-side action buffer (host path)
-static int ensure_actions(te_handle *h, int ndec) {
-  if (ndec <= h->actions_cap) return 0;
-  CU(cudaDeviceSynchronize());
-  cudaFree(h->d_actions); h->d_actions = nullptr; h->actions_cap = 0;
-  CU(dalloc(&h->d_actions, (size_t)ndec * h->cfg.num_envs * h->I));
-  h->actions_cap = ndec;
+// The record layout of a handle (te_kernels.cuh: wire_layout) and the host path te_create chose for it.
+static te_wire_layout_t wire_layout_of(const te_handle *h) {
+  const WireLayout w = wire_layout(h->r, h->I);
+  return {w.stride, w.passed, w.detected, w.light, w.reward, w.done, WIRE_MAX_K, h->float_dma ? 1 : 0};
+}
+
+// Host buffers: the batch is launched in slices on two alternating streams (the tail of one slice overlaps the
+// head of the next), and a third stream copies each finished slice's results to the host while the following slices
+// are simulated (envs are independent: any slicing gives the same results).  Fused steps of up to WIRE_MAX_K ticks
+// travel as compact wire records (one copy per slice and actor step, 2.5 x fewer bytes than the float observation)
+// that the handle's helper threads expand into the caller's arrays while the GPU works on the next slices.
+static int launch_sliced(te_handle *h, const StepReq &q, Route route, StepParams &p, StepVariant sv, int smem,
+                         cudaStream_t st) {
+  const int nsteps = q.nsteps, G = h->G;
+  const size_t E = (size_t)h->cfg.num_envs;
+  const size_t obs_len = q.raw ? (size_t)(2 * h->r + 2 * h->I) : (size_t)(2 * h->r + h->I);
+  const int E_i = h->cfg.num_envs;
+  const int nslice = h->host_slices;
+  const int per = ((E_i + nslice - 1) / nslice + G - 1) / G * G;   // whole CTAs (G envs each) per slice
+  CU(cudaEventRecord(h->ev_fork.get(), st));         // actions (and the auto-reset) are complete on `st`
+  CU(cudaStreamWaitEvent(h->stream2.get(), h->ev_fork.get(), 0));
+  cudaStream_t lanes[2] = {st, h->stream2.get()}, cs_copy = h->stream_copy.get();
+  const char *src_obs = (const char *)h->d_obs_i.get();   // int (raw) or float observations
+  unsigned char *host_wire = q.wire_only ? (unsigned char *)q.obs : h->h_wire.get();
+  const unsigned char *dev_wire = h->d_wire.get();
+  const size_t wstep = E * (size_t)h->wire_stride;   // records of one actor step
+  int nk = 0;
+  for (int k = 0, e0 = 0; e0 < E_i; k++, e0 += per) {
+    const int ne = (E_i - e0) < per ? (E_i - e0) : per;
+    cudaStream_t cs = lanes[k & 1];
+    p.env0 = e0; p.env_end = e0 + ne;
+    sv.fn<<<(ne + G - 1) / G, h->threads, smem, cs>>>(p);
+    CU(cudaGetLastError());
+    CU(cudaEventRecord(h->ev_slice[k].get(), cs));
+    CU(cudaStreamWaitEvent(cs_copy, h->ev_slice[k].get(), 0));
+    if (route == Route::WIRE) {
+      for (int j = 0; j < nsteps; j++)
+        CU(cudaMemcpyAsync(host_wire + j * wstep + (size_t)e0 * h->wire_stride, dev_wire + j * wstep + (size_t)e0 * h->wire_stride,
+                           (size_t)ne * h->wire_stride, cudaMemcpyDeviceToHost, cs_copy));
+      CU(cudaEventRecord(h->ev_copy[k].get(), cs_copy));
+    } else {
+      for (int j = 0; j < nsteps; j++) {      // float arrays written by the copy engine, [nsteps][E][...]
+        const size_t eo = (size_t)j * E + e0;
+        CU(cudaMemcpyAsync((char *)q.obs + eo * obs_len * 4, src_obs + eo * obs_len * 4, (size_t)ne * obs_len * 4,
+                           cudaMemcpyDeviceToHost, cs_copy));
+        CU(cudaMemcpyAsync(q.reward + eo * h->I, h->d_reward.get() + eo * h->I, (size_t)ne * h->I * sizeof(float),
+                           cudaMemcpyDeviceToHost, cs_copy));
+        CU(cudaMemcpyAsync(q.done + eo, h->d_done.get() + eo, (size_t)ne, cudaMemcpyDeviceToHost, cs_copy));
+      }
+    }
+    nk = k + 1;
+  }
+  if (q.controller == CTRL_GREEDY && q.actions)   // the controller's choices, for the caller
+    CU(cudaMemcpyAsync(const_cast<uint8_t *>(q.actions), h->d_actions.get(), (size_t)decisions(p) * E * h->I,
+                       cudaMemcpyDeviceToHost, cs_copy));
+  CU(cudaEventRecord(h->ev_join.get(), h->stream2.get()));
+  CU(cudaEventRecord(h->ev_copied.get(), cs_copy));
+  CU(cudaStreamWaitEvent(st, h->ev_join.get(), 0));
+  CU(cudaStreamWaitEvent(st, h->ev_copied.get(), 0));
+  CU(cudaEventRecord(h->ev1.get(), st));
+  h->timed = true;
+  if (route == Route::WIRE && !q.wire_only) {
+    const ExpandJob j = {h->h_wire.get(), (float *)q.obs, q.reward, q.done, q.env_mask, wire_layout_of(h), h->r, h->I, nk,
+                         per, E_i, nsteps, h->ev_copy};
+    const bool ok = h->pool->run(j);
+    CU(cudaStreamSynchronize(st));
+    if (!ok) return fail("%s: a device-to-host copy failed: %s", q.who, cudaGetErrorString(cudaGetLastError()));
+    return 0;
+  }
+  CU(cudaStreamSynchronize(st));
   return 0;
 }
 
 static int launch_step(te_handle *h, const StepReq &q) {
-  const int K = q.K, raw = q.raw, nsteps = q.nsteps;
+  const int K = q.K, nsteps = q.nsteps;
   const bool greedy = q.controller == CTRL_GREEDY;
   if (!h || !q.obs || (!greedy && !q.actions) || (!q.wire_only && (!q.reward || !q.done))) return fail("%s: null argument", q.who);
   if (K < 1 || K > MAX_K) return fail("%s: k_ticks must be in [1, %d]", q.who, MAX_K);
@@ -741,106 +826,23 @@ static int launch_step(te_handle *h, const StepReq &q) {
   if (h->cfg.arrival_mode == TE_ARRIVALS_INJECTED && !h->base.sched_off) return fail("%s: no arrival schedule set", q.who);
   CU(cudaSetDevice(h->device));
   cudaStream_t st = pick_stream(h, q.stream);
-  const size_t E = (size_t)h->cfg.num_envs;
-  const size_t obs_len = raw ? (size_t)(2 * h->r + 2 * h->I) : (size_t)(2 * h->r + h->I);
-  const bool host = q.memspace == TE_HOST;
-  const bool use_wire = !raw && K <= WIRE_MAX_K && (q.wire_only || (host && (!h->float_dma || q.env_mask)));
-  StepParams p = h->base;
-  p.K = K; p.raw = raw; p.nsteps = nsteps; p.controller = q.controller; p.actions_out = nullptr; p.env_mask = q.env_mask;
-  p.decide_every = greedy ? h->ctrl_spacing : 0;
-  const int ndec = p.decide_every > 0 ? (nsteps + p.decide_every - 1) / p.decide_every : 1;   // controller decisions of this launch
-  if (host) {
-    if (int rc = ensure_actions(h, ndec)) return rc;
-    if (!greedy) CU(cudaMemcpyAsync(h->d_actions, q.actions, E * h->I, cudaMemcpyHostToDevice, st));
-    if (q.env_mask) { CU(cudaMemcpyAsync(h->d_mask, q.env_mask, E, cudaMemcpyHostToDevice, st)); p.env_mask = h->d_mask; }
-    p.actions = h->d_actions; p.actions_out = greedy ? h->d_actions : nullptr;
-    p.obs_f = h->d_obs_f; p.obs_i = h->d_obs_i; p.reward = h->d_reward; p.done = h->d_done;
-    if (use_wire) {
-      if (int rc = ensure_wire_steps(h, nsteps)) return rc;
-      p.wire = h->d_wire; p.wire_stride = h->wire_stride;
-    } else {
-      if (int rc = ensure_float_steps(h, nsteps)) return rc;
-      p.obs_f = h->d_obs_f; p.obs_i = h->d_obs_i; p.reward = h->d_reward; p.done = h->d_done;
-    }
-  } else {
-    p.actions = q.actions; p.actions_out = greedy ? const_cast<uint8_t *>(q.actions) : nullptr;
-    p.obs_f = (float *)q.obs; p.obs_i = (int *)q.obs; p.reward = q.reward; p.done = q.done;
-    if (q.wire_only) { p.wire = (unsigned char *)q.obs; p.wire_stride = h->wire_stride; }
-  }
-  if (!raw && (h->cfg.flags & TE_AUTO_RESET)) {
+  const Route route = pick_route(h, q);
+  StepParams p;
+  if (int rc = step_params(h, q, route, st, p)) return rc;
+  if (!q.raw && (h->cfg.flags & TE_AUTO_RESET)) {
     te_reset_kernel<<<(h->cfg.num_envs + RESET_ENVS_PER_CTA - 1) / RESET_ENVS_PER_CTA, 128, 0, st>>>(p, p.env_mask, nullptr, 1);
     CU(cudaGetLastError());
   }
   const bool validate = (h->cfg.flags & TE_VALIDATE) != 0;
   const StepVariant sv = step_variant_for(h->threads, validate, fast_arch(h), h->G > 1);
   const int smem = smem_bytes(sv.maxt, validate, K * nsteps, h->n_entry, h->G);
-  const int G = h->G;
-  p.G = G;
-  CU(cudaEventRecord(h->ev0, st));
-  if (!host) {
-    p.env0 = 0; p.env_end = h->cfg.num_envs;
-    sv.fn<<<(h->cfg.num_envs + G - 1) / G, h->threads, smem, st>>>(p);
-    CU(cudaGetLastError());
-    CU(cudaEventRecord(h->ev1, st));
-    h->timed = true;
-    return 0;
-  }
-  // Host buffers: the batch is launched in slices on two alternating streams (the tail of one slice overlaps the
-  // head of the next), and a third stream copies each finished slice's results to the host while the following slices
-  // are simulated (envs are independent: any slicing gives the same results).  Fused steps of up to WIRE_MAX_K ticks
-  // travel as compact wire records (one copy per slice and actor step, 2.5 x fewer bytes than the float observation)
-  // that the handle's helper threads expand into the caller's arrays while the GPU works on the next slices.
-  const int E_i = h->cfg.num_envs;
-  const int nslice = h->host_slices;
-  const int per = ((E_i + nslice - 1) / nslice + G - 1) / G * G;   // whole CTAs (G envs each) per slice
-  CU(cudaEventRecord(h->ev_fork, st));               // actions (and the auto-reset) are complete on `st`
-  CU(cudaStreamWaitEvent(h->stream2, h->ev_fork, 0));
-  cudaStream_t lanes[2] = {st, h->stream2};
-  const char *src_obs = raw ? (const char *)h->d_obs_i : (const char *)h->d_obs_f;   // (after ensure_float_steps)
-  unsigned char *host_wire = q.wire_only ? (unsigned char *)q.obs : h->h_wire;
-  const size_t wstep = E * (size_t)h->wire_stride;   // records of one actor step
-  int nk = 0;
-  for (int k = 0, e0 = 0; e0 < E_i; k++, e0 += per) {
-    const int ne = (E_i - e0) < per ? (E_i - e0) : per;
-    cudaStream_t cs = lanes[k & 1];
-    p.env0 = e0; p.env_end = e0 + ne;
-    sv.fn<<<(ne + G - 1) / G, h->threads, smem, cs>>>(p);
-    CU(cudaGetLastError());
-    CU(cudaEventRecord(h->ev_slice[k], cs));
-    CU(cudaStreamWaitEvent(h->stream_copy, h->ev_slice[k], 0));
-    if (use_wire) {
-      for (int j = 0; j < nsteps; j++)
-        CU(cudaMemcpyAsync(host_wire + j * wstep + (size_t)e0 * h->wire_stride, h->d_wire + j * wstep + (size_t)e0 * h->wire_stride,
-                           (size_t)ne * h->wire_stride, cudaMemcpyDeviceToHost, h->stream_copy));
-      CU(cudaEventRecord(h->ev_copy[k], h->stream_copy));
-    } else {
-      for (int j = 0; j < nsteps; j++) {      // float arrays written by the copy engine, [nsteps][E][...]
-        const size_t eo = (size_t)j * E + e0;
-        CU(cudaMemcpyAsync((char *)q.obs + eo * obs_len * 4, src_obs + eo * obs_len * 4, (size_t)ne * obs_len * 4,
-                           cudaMemcpyDeviceToHost, h->stream_copy));
-        CU(cudaMemcpyAsync(q.reward + eo * h->I, h->d_reward + eo * h->I, (size_t)ne * h->I * sizeof(float),
-                           cudaMemcpyDeviceToHost, h->stream_copy));
-        CU(cudaMemcpyAsync(q.done + eo, h->d_done + eo, (size_t)ne, cudaMemcpyDeviceToHost, h->stream_copy));
-      }
-    }
-    nk = k + 1;
-  }
-  if (greedy && q.actions)   // the controller's choices, for the caller
-    CU(cudaMemcpyAsync(const_cast<uint8_t *>(q.actions), h->d_actions, (size_t)ndec * E * h->I, cudaMemcpyDeviceToHost, h->stream_copy));
-  CU(cudaEventRecord(h->ev_join, h->stream2));
-  CU(cudaEventRecord(h->ev_copied, h->stream_copy));
-  CU(cudaStreamWaitEvent(st, h->ev_join, 0));
-  CU(cudaStreamWaitEvent(st, h->ev_copied, 0));
-  CU(cudaEventRecord(h->ev1, st));
+  CU(cudaEventRecord(h->ev0.get(), st));
+  if (route != Route::DEVICE) return launch_sliced(h, q, route, p, sv, smem, st);
+  p.env0 = 0; p.env_end = h->cfg.num_envs;
+  sv.fn<<<(h->cfg.num_envs + h->G - 1) / h->G, h->threads, smem, st>>>(p);
+  CU(cudaGetLastError());
+  CU(cudaEventRecord(h->ev1.get(), st));
   h->timed = true;
-  if (use_wire && !q.wire_only) {
-    ExpandJob j = {h->h_wire, (float *)q.obs, q.reward, q.done, q.env_mask, h->r, h->I, h->wire_stride, nk, per, E_i, nsteps, h->ev_copy};
-    const bool ok = h->pool->run(j);
-    CU(cudaStreamSynchronize(st));
-    if (!ok) return fail("%s: a device-to-host copy failed: %s", q.who, cudaGetErrorString(cudaGetLastError()));
-    return 0;
-  }
-  CU(cudaStreamSynchronize(st));
   return 0;
 }
 
@@ -889,14 +891,13 @@ extern "C" int te_step_wire(te_handle *h, const uint8_t *actions, int32_t k_tick
 
 extern "C" int te_wire_layout(const te_handle *h, te_wire_layout_t *out) {
   if (!h || !out) return fail("te_wire_layout: null argument");
-  out->stride = h->wire_stride; out->passed = 0; out->detected = h->r; out->light = 2 * h->r;
-  out->reward = 2 * h->r + 4 * h->I; out->done = 2 * h->r + 8 * h->I; out->max_k_ticks = WIRE_MAX_K;
+  *out = wire_layout_of(h);
   return 0;
 }
 
 extern "C" int te_expand_wire(const te_handle *h, const void *records, int32_t count, float *obs, float *reward, uint8_t *done) {
   if (!h || !records || !obs || !reward || !done || count < 0) return fail("te_expand_wire: bad argument");
-  expand_records((const unsigned char *)records, h->r, h->I, h->wire_stride, count, obs, reward, done);
+  te_expand_records_host((const unsigned char *)records, wire_layout_of(h), h->r, h->I, count, obs, reward, done);
   return 0;
 }
 
@@ -911,7 +912,7 @@ extern "C" int te_remi_reward(te_handle *h, float *reward, int memspace, void *s
   if (!h || !reward) return fail("te_remi_reward: null argument");
   CU(cudaSetDevice(h->device));
   cudaStream_t st = pick_stream(h, stream);
-  float *dr = memspace == TE_HOST ? h->d_reward : reward;
+  float *dr = memspace == TE_HOST ? h->d_reward.get() : reward;
   te_remi_kernel<<<h->cfg.num_envs, 128, 0, st>>>(h->base, dr);
   CU(cudaGetLastError());
   if (memspace == TE_HOST) {
@@ -928,8 +929,8 @@ extern "C" int te_cars_on_roads(te_handle *h, int32_t *out, int memspace, void *
   const size_t n = (size_t)h->cfg.num_envs * h->R;
   int *d = out;
   if (memspace == TE_HOST) {
-    if (!h->d_cars) CU(dalloc(&h->d_cars, n));
-    d = h->d_cars;
+    if (!h->d_cars) CU(alloc(h->d_cars, n));
+    d = h->d_cars.get();
   }
   te_cars_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(h->base, d);
   CU(cudaGetLastError());
@@ -945,7 +946,7 @@ extern "C" int te_greedy_actions(te_handle *h, uint8_t *actions, int memspace, v
   CU(cudaSetDevice(h->device));
   cudaStream_t st = pick_stream(h, stream);
   const size_t n = (size_t)h->cfg.num_envs * h->I;
-  uint8_t *d = memspace == TE_HOST ? h->d_actions : actions;
+  uint8_t *d = memspace == TE_HOST ? h->d_actions.get() : actions;
   te_greedy_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(h->base, d);
   CU(cudaGetLastError());
   if (memspace == TE_HOST) {
@@ -966,12 +967,12 @@ extern "C" int te_get_state(te_handle *h, int32_t env_begin, int32_t count, int3
   std::vector<int> hel((size_t)h->I * count);
   std::vector<uint8_t> hph((size_t)h->I * count), hpd((size_t)h->I * count);
   std::vector<EnvScalars> hes(count);
-  CU(cudaMemcpy(hx.data(), h->x + env_begin * row, hx.size() * 4, cudaMemcpyDeviceToHost));
-  CU(cudaMemcpy(hv.data(), h->v + env_begin * row, hv.size() * 4, cudaMemcpyDeviceToHost));
-  CU(cudaMemcpy(hel.data(), h->elapsed + (size_t)env_begin * h->I, hel.size() * 4, cudaMemcpyDeviceToHost));
-  CU(cudaMemcpy(hph.data(), h->phase + (size_t)env_begin * h->I, hph.size(), cudaMemcpyDeviceToHost));
-  CU(cudaMemcpy(hpd.data(), h->passed_dst + (size_t)env_begin * h->I, hpd.size(), cudaMemcpyDeviceToHost));
-  CU(cudaMemcpy(hes.data(), h->env + env_begin, hes.size() * sizeof(EnvScalars), cudaMemcpyDeviceToHost));
+  CU(cudaMemcpy(hx.data(), h->x.get() + env_begin * row, hx.size() * 4, cudaMemcpyDeviceToHost));
+  CU(cudaMemcpy(hv.data(), h->v.get() + env_begin * row, hv.size() * 4, cudaMemcpyDeviceToHost));
+  CU(cudaMemcpy(hel.data(), h->elapsed.get() + (size_t)env_begin * h->I, hel.size() * 4, cudaMemcpyDeviceToHost));
+  CU(cudaMemcpy(hph.data(), h->phase.get() + (size_t)env_begin * h->I, hph.size(), cudaMemcpyDeviceToHost));
+  CU(cudaMemcpy(hpd.data(), h->passed_dst.get() + (size_t)env_begin * h->I, hpd.size(), cudaMemcpyDeviceToHost));
+  CU(cudaMemcpy(hes.data(), h->env.get() + env_begin, hes.size() * sizeof(EnvScalars), cudaMemcpyDeviceToHost));
   const int R = h->R, r = h->r, I = h->I, ol = 2 * r + 2 * I;
   for (int e = 0; e < count; e++) {
     for (int rd = 0; rd < R; rd++) {
@@ -1007,7 +1008,7 @@ extern "C" int te_set_state(te_handle *h, int32_t env_begin, int32_t count, cons
   std::vector<int> hel((size_t)I * count);
   std::vector<uint8_t> hph((size_t)I * count), hpd((size_t)I * count);
   std::vector<EnvScalars> hes(count);
-  CU(cudaMemcpy(hes.data(), h->env + env_begin, hes.size() * sizeof(EnvScalars), cudaMemcpyDeviceToHost));
+  CU(cudaMemcpy(hes.data(), h->env.get() + env_begin, hes.size() * sizeof(EnvScalars), cudaMemcpyDeviceToHost));
   bool wild = false;
   for (int e = 0; e < count; e++) {
     for (int rd = 0; rd < h->Rp; rd++) {
@@ -1045,13 +1046,14 @@ extern "C" int te_set_state(te_handle *h, int32_t env_begin, int32_t count, cons
   }
   // uploads go through the handle's stream and the device is synchronised afterwards, so they are ordered against
   // steps on ANY stream (the step streams are non-blocking: the legacy default stream does not order against them)
-  CU(cudaMemcpyAsync(h->x + env_begin * row, hx.data(), hx.size() * 4, cudaMemcpyHostToDevice, h->stream));
-  CU(cudaMemcpyAsync(h->v + env_begin * row, hv.data(), hv.size() * 4, cudaMemcpyHostToDevice, h->stream));
-  CU(cudaMemcpyAsync(h->elapsed + (size_t)env_begin * I, hel.data(), hel.size() * 4, cudaMemcpyHostToDevice, h->stream));
-  CU(cudaMemcpyAsync(h->phase + (size_t)env_begin * I, hph.data(), hph.size(), cudaMemcpyHostToDevice, h->stream));
-  CU(cudaMemcpyAsync(h->passed_dst + (size_t)env_begin * I, hpd.data(), hpd.size(), cudaMemcpyHostToDevice, h->stream));
-  CU(cudaMemcpyAsync(h->env + env_begin, hes.data(), hes.size() * sizeof(EnvScalars), cudaMemcpyHostToDevice, h->stream));
-  CU(cudaStreamSynchronize(h->stream));
+  cudaStream_t st = h->stream.get();
+  CU(cudaMemcpyAsync(h->x.get() + env_begin * row, hx.data(), hx.size() * 4, cudaMemcpyHostToDevice, st));
+  CU(cudaMemcpyAsync(h->v.get() + env_begin * row, hv.data(), hv.size() * 4, cudaMemcpyHostToDevice, st));
+  CU(cudaMemcpyAsync(h->elapsed.get() + (size_t)env_begin * I, hel.data(), hel.size() * 4, cudaMemcpyHostToDevice, st));
+  CU(cudaMemcpyAsync(h->phase.get() + (size_t)env_begin * I, hph.data(), hph.size(), cudaMemcpyHostToDevice, st));
+  CU(cudaMemcpyAsync(h->passed_dst.get() + (size_t)env_begin * I, hpd.data(), hpd.size(), cudaMemcpyHostToDevice, st));
+  CU(cudaMemcpyAsync(h->env.get() + env_begin, hes.data(), hes.size() * sizeof(EnvScalars), cudaMemcpyHostToDevice, st));
+  CU(cudaStreamSynchronize(st));
   CU(cudaDeviceSynchronize());
   if (wild && h->tame) {      // from now on: the kernels with the per-car validity predicate, one env per CTA
     h->tame = false;
@@ -1080,7 +1082,7 @@ extern "C" int te_get_stats(te_handle *h, te_stats *out) {
   CU(cudaSetDevice(h->device));
   CU(cudaDeviceSynchronize());  // steps may have been queued on caller-provided streams
   DeviceStats s;
-  CU(cudaMemcpy(&s, h->stats, sizeof(s), cudaMemcpyDeviceToHost));
+  CU(cudaMemcpy(&s, h->stats.get(), sizeof(s), cudaMemcpyDeviceToHost));
   out->ticks = s.ticks; out->actor_steps = s.actor_steps; out->vehicle_updates = s.vehicle_updates;
   out->overflows = s.overflows; out->cars_generated = s.cars_generated; out->episodes = s.episodes;
   out->return_sum = s.return_sum; out->disc_return_sum = s.disc_return_sum; out->seq_fallback_ticks = s.seq_fallback_ticks; out->cars_exited = s.cars_exited;
@@ -1094,7 +1096,7 @@ extern "C" int te_get_trip_times(te_handle *h, int32_t *env_out, float *trip_out
   CU(cudaSetDevice(h->device));
   CU(cudaDeviceSynchronize());
   unsigned long long n = 0;
-  CU(cudaMemcpy(&n, h->d_trip_count, sizeof(n), cudaMemcpyDeviceToHost));
+  CU(cudaMemcpy(&n, h->d_trip_count.get(), sizeof(n), cudaMemcpyDeviceToHost));
   // The device counts every trip but records only the first trip_cap of them: on overflow the recorded ones are still
   // returned (and cleared when asked), and the call reports the truncation with return code 1.
   const bool truncated = (long long)n > h->trip_cap;
@@ -1102,14 +1104,14 @@ extern "C" int te_get_trip_times(te_handle *h, int32_t *env_out, float *trip_out
   *count = (int64_t)have;
   if (have && (env_out || trip_out)) {
     std::vector<TripRecord> recs(have);
-    CU(cudaMemcpy(recs.data(), h->d_trips, have * sizeof(TripRecord), cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(recs.data(), h->d_trips.get(), have * sizeof(TripRecord), cudaMemcpyDeviceToHost));
     // the reference appends in (env-local) tick order, road-index order, pop order
     std::sort(recs.begin(), recs.end(), [](const TripRecord &a, const TripRecord &b) {
       return a.env != b.env ? a.env < b.env : a.order < b.order; });
     const int64_t m = (int64_t)have < cap ? (int64_t)have : cap;
     for (int64_t i = 0; i < m; i++) { if (env_out) env_out[i] = recs[i].env; if (trip_out) trip_out[i] = recs[i].trip; }
   }
-  if (clear) CU(cudaMemset(h->d_trip_count, 0, sizeof(unsigned long long)));
+  if (clear) CU(cudaMemset(h->d_trip_count.get(), 0, sizeof(unsigned long long)));
   if (truncated) {
     g_err = "te_get_trip_times: " + std::to_string(n) + " trips since the last clear but the buffer holds " +
             std::to_string(h->trip_cap) + "; the first ones were returned, read more often";
@@ -1121,7 +1123,7 @@ extern "C" int te_get_trip_times(te_handle *h, int32_t *env_out, float *trip_out
 extern "C" int te_synchronize(te_handle *h) {
   if (!h) return fail("te_synchronize: null handle");
   CU(cudaSetDevice(h->device));
-  CU(cudaStreamSynchronize(h->stream));
+  CU(cudaStreamSynchronize(h->stream.get()));
   return 0;
 }
 
@@ -1135,14 +1137,15 @@ extern "C" int te_stage_bandwidth(te_handle *h, int32_t repeats, double *gbytes_
   CU(cudaFuncSetAttribute(te_stage_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, stage_smem));
   StepParams p = h->base;
   p.K = 10;
-  te_stage_kernel<<<h->cfg.num_envs, h->Rp, stage_smem, h->stream>>>(p, validate);  // warm-up (state is rewritten unchanged)
-  CU(cudaEventRecord(h->ev0, h->stream));
-  for (int i = 0; i < repeats; i++) te_stage_kernel<<<h->cfg.num_envs, h->Rp, stage_smem, h->stream>>>(p, validate);
-  CU(cudaEventRecord(h->ev1, h->stream));
-  CU(cudaEventSynchronize(h->ev1));
+  cudaStream_t st = h->stream.get();
+  te_stage_kernel<<<h->cfg.num_envs, h->Rp, stage_smem, st>>>(p, validate);  // warm-up (state is rewritten unchanged)
+  CU(cudaEventRecord(h->ev0.get(), st));
+  for (int i = 0; i < repeats; i++) te_stage_kernel<<<h->cfg.num_envs, h->Rp, stage_smem, st>>>(p, validate);
+  CU(cudaEventRecord(h->ev1.get(), st));
+  CU(cudaEventSynchronize(h->ev1.get()));
   CU(cudaGetLastError());
   float ms = 0.f;
-  CU(cudaEventElapsedTime(&ms, h->ev0, h->ev1));
+  CU(cudaEventElapsedTime(&ms, h->ev0.get(), h->ev1.get()));
   const double bytes = 2.0 /* planes */ * 2.0 /* in + out */ * (double)h->cfg.num_envs * h->R * CAP * 4.0 * repeats;
   *gbytes_per_sec = bytes / (ms * 1e-3) / 1e9;
   return 0;
@@ -1162,21 +1165,20 @@ extern "C" int te_host_free(void *ptr) {
 extern "C" int te_last_kernel_ms(te_handle *h, float *ms) {
   if (!h || !ms) return fail("te_last_kernel_ms: null argument");
   if (!h->timed) return fail("te_last_kernel_ms: no step has been launched");
-  CU(cudaEventSynchronize(h->ev1));
-  CU(cudaEventElapsedTime(ms, h->ev0, h->ev1));
+  CU(cudaEventSynchronize(h->ev1.get()));
+  CU(cudaEventElapsedTime(ms, h->ev0.get(), h->ev1.get()));
   return 0;
 }
 
 // ------------------------------------------------------------------ test hooks
 extern "C" int te_test_powf(int device, const float *x, float y, float *out, int64_t n) {
   CU(cudaSetDevice(device));
-  float *dx = nullptr, *dout = nullptr;
-  CU(cudaMalloc(&dx, n * 4)); CU(cudaMalloc(&dout, n * 4));
-  CU(cudaMemcpy(dx, x, n * 4, cudaMemcpyHostToDevice));
-  te_test_powf_kernel<<<(unsigned)((n + 255) / 256), 256>>>(dx, y, dout, n);
+  dev_buf<float> dx, dout;
+  CU(alloc(dx, n)); CU(alloc(dout, n));
+  CU(cudaMemcpy(dx.get(), x, n * 4, cudaMemcpyHostToDevice));
+  te_test_powf_kernel<<<(unsigned)((n + 255) / 256), 256>>>(dx.get(), y, dout.get(), n);
   CU(cudaGetLastError());
-  CU(cudaMemcpy(out, dout, n * 4, cudaMemcpyDeviceToHost));
-  cudaFree(dx); cudaFree(dout);
+  CU(cudaMemcpy(out, dout.get(), n * 4, cudaMemcpyDeviceToHost));
   return 0;
 }
 
@@ -1196,19 +1198,18 @@ static int test_idm(int device, float rate, const float *a, const float *xl, con
   CU(upload_math_consts());
   IdmConst c;
   fill_idm(c, a, rate);
-  float *d[7];
+  dev_buf<float> d[7];
   const float *src[5] = {xl, vl, ll, x, v};
-  IdmConst *dc = nullptr;
-  CU(cudaMalloc(&dc, sizeof(IdmConst)));
-  CU(cudaMemcpy(dc, &c, sizeof(IdmConst), cudaMemcpyHostToDevice));
-  for (int i = 0; i < 7; i++) CU(cudaMalloc(&d[i], n * 4));
-  for (int i = 0; i < 5; i++) CU(cudaMemcpy(d[i], src[i], n * 4, cudaMemcpyHostToDevice));
-  te_test_idm_kernel<<<(unsigned)((n + 255) / 256), 256>>>(c, dc, d[0], d[1], d[2], d[3], d[4], d[5], d[6], n, unchecked);
+  dev_buf<IdmConst> dc;
+  CU(alloc(dc, 1));
+  CU(cudaMemcpy(dc.get(), &c, sizeof(IdmConst), cudaMemcpyHostToDevice));
+  for (int i = 0; i < 7; i++) CU(alloc(d[i], n));
+  for (int i = 0; i < 5; i++) CU(cudaMemcpy(d[i].get(), src[i], n * 4, cudaMemcpyHostToDevice));
+  te_test_idm_kernel<<<(unsigned)((n + 255) / 256), 256>>>(c, dc.get(), d[0].get(), d[1].get(), d[2].get(), d[3].get(),
+                                                           d[4].get(), d[5].get(), d[6].get(), n, unchecked);
   CU(cudaGetLastError());
-  CU(cudaMemcpy(x_out, d[5], n * 4, cudaMemcpyDeviceToHost));
-  CU(cudaMemcpy(v_out, d[6], n * 4, cudaMemcpyDeviceToHost));
-  for (int i = 0; i < 7; i++) cudaFree(d[i]);
-  cudaFree(dc);
+  CU(cudaMemcpy(x_out, d[5].get(), n * 4, cudaMemcpyDeviceToHost));
+  CU(cudaMemcpy(v_out, d[6].get(), n * 4, cudaMemcpyDeviceToHost));
   return 0;
 }
 
@@ -1232,23 +1233,22 @@ extern "C" int te_idm_peak_form(int device, const float *a, float rate, int32_t 
   CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
   int threads = 256, blocks = sms * 8;  // warps_per_sm == 0: 2048 resident threads per SM
   if (warps_per_sm) { threads = 32 * warps_per_sm; blocks = sms; }   // one CTA of w warps per SM
-  float *sink = nullptr;
-  CU(cudaMalloc(&sink, (size_t)threads * blocks * 4));
-  IdmConst *dc = nullptr;
-  CU(cudaMalloc(&dc, sizeof(IdmConst)));
-  CU(cudaMemcpy(dc, &c, sizeof(IdmConst), cudaMemcpyHostToDevice));
-  cudaEvent_t e0, e1;
-  CU(cudaEventCreate(&e0)); CU(cudaEventCreate(&e1));
-  te_idm_peak_kernel<<<blocks, threads>>>(c, dc, iters / 4 + 1, sink, form);  // warm-up
-  CU(cudaEventRecord(e0));
-  te_idm_peak_kernel<<<blocks, threads>>>(c, dc, iters, sink, form);
-  CU(cudaEventRecord(e1));
-  CU(cudaEventSynchronize(e1));
+  dev_buf<float> sink;
+  CU(alloc(sink, (size_t)threads * blocks));
+  dev_buf<IdmConst> dc;
+  CU(alloc(dc, 1));
+  CU(cudaMemcpy(dc.get(), &c, sizeof(IdmConst), cudaMemcpyHostToDevice));
+  event_ptr e0, e1;
+  CU(create(e0, cudaEventDefault)); CU(create(e1, cudaEventDefault));
+  te_idm_peak_kernel<<<blocks, threads>>>(c, dc.get(), iters / 4 + 1, sink.get(), form);  // warm-up
+  CU(cudaEventRecord(e0.get()));
+  te_idm_peak_kernel<<<blocks, threads>>>(c, dc.get(), iters, sink.get(), form);
+  CU(cudaEventRecord(e1.get()));
+  CU(cudaEventSynchronize(e1.get()));
   CU(cudaGetLastError());
   float ms = 0.f;
-  CU(cudaEventElapsedTime(&ms, e0, e1));
+  CU(cudaEventElapsedTime(&ms, e0.get(), e1.get()));
   *updates_per_sec = (double)threads * blocks * iters * ((form == 1 || form == 3) ? 2 : 1) / (ms * 1e-3);
-  cudaEventDestroy(e0); cudaEventDestroy(e1); cudaFree(sink); cudaFree(dc);
   return 0;
 }
 
@@ -1259,39 +1259,36 @@ extern "C" int te_idm_peak(int device, const float *a, float rate, int32_t iters
 extern "C" int te_test_powf4_exhaustive(int device, uint64_t tau, uint64_t out[4]) {
   if (!out) return fail("te_test_powf4_exhaustive: null argument");
   CU(cudaSetDevice(device));
-  unsigned long long *d = nullptr;
-  CU(cudaMalloc(&d, 4 * sizeof(unsigned long long)));
-  CU(cudaMemset(d, 0, 4 * sizeof(unsigned long long)));
-  te_powf4_exhaustive_kernel<<<148 * 16, 256>>>((unsigned long long)tau, d);
+  dev_buf<unsigned long long> d;
+  CU(alloc(d, 4));
+  CU(cudaMemset(d.get(), 0, 4 * sizeof(unsigned long long)));
+  te_powf4_exhaustive_kernel<<<148 * 16, 256>>>((unsigned long long)tau, d.get());
   CU(cudaGetLastError());
-  CU(cudaMemcpy(out, d, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-  cudaFree(d);
+  CU(cudaMemcpy(out, d.get(), 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
   return 0;
 }
 
 extern "C" int te_test_fdiv_const_exhaustive(int device, float cst, uint64_t out[3]) {
   if (!out) return fail("te_test_fdiv_const_exhaustive: null argument");
   CU(cudaSetDevice(device));
-  unsigned long long *d = nullptr;
-  CU(cudaMalloc(&d, 3 * sizeof(unsigned long long)));
-  CU(cudaMemset(d, 0, 3 * sizeof(unsigned long long)));
+  dev_buf<unsigned long long> d;
+  CU(alloc(d, 3));
+  CU(cudaMemset(d.get(), 0, 3 * sizeof(unsigned long long)));
   volatile float y = 1.0f / cst;
-  te_fdiv_const_exhaustive_kernel<<<148 * 16, 256>>>(cst, y, d);
+  te_fdiv_const_exhaustive_kernel<<<148 * 16, 256>>>(cst, y, d.get());
   CU(cudaGetLastError());
-  CU(cudaMemcpy(out, d, 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-  cudaFree(d);
+  CU(cudaMemcpy(out, d.get(), 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
   return 0;
 }
 
 extern "C" int te_test_philox(int device, const uint32_t *ctr, const uint32_t *key, uint32_t *out) {
   CU(cudaSetDevice(device));
-  uint32_t *d = nullptr;
-  CU(cudaMalloc(&d, 10 * 4));
-  CU(cudaMemcpy(d, ctr, 16, cudaMemcpyHostToDevice));
-  CU(cudaMemcpy(d + 4, key, 8, cudaMemcpyHostToDevice));
-  te_test_philox_kernel<<<1, 1>>>(d, d + 4, d + 6);
+  dev_buf<uint32_t> d;
+  CU(alloc(d, 10));
+  CU(cudaMemcpy(d.get(), ctr, 16, cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(d.get() + 4, key, 8, cudaMemcpyHostToDevice));
+  te_test_philox_kernel<<<1, 1>>>(d.get(), d.get() + 4, d.get() + 6);
   CU(cudaGetLastError());
-  CU(cudaMemcpy(out, d + 6, 16, cudaMemcpyDeviceToHost));
-  cudaFree(d);
+  CU(cudaMemcpy(out, d.get() + 6, 16, cudaMemcpyDeviceToHost));
   return 0;
 }

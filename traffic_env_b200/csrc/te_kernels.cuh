@@ -126,9 +126,13 @@ struct StepParams {
 };
 
 // Wire record of one env actor step: everything te_step returns, in 1/2.5 of the bytes of the float observation
-// (passed <= 19 K and detected <= 18 fit a byte for K <= 13 ticks).  Offsets: passed 0, detected r, light 2r
-// (4-byte aligned: r = 4 V), reward 2r + 4I, done 2r + 8I; stride rounded up to 16 bytes.
-__host__ __device__ constexpr int wire_stride_bytes(int r, int I) { return (2 * r + 8 * I + 1 + 15) / 16 * 16; }
+// (passed <= 19 K and detected <= 18 fit a byte for K <= 13 ticks).  Byte offsets of the fields of a record and the
+// stride between records: u8 passed[r] | u8 detected[r] | f32 light[I] (4-byte aligned: r = 4 V) | f32 reward[I] |
+// u8 done, rounded up to 16 bytes.  The kernel epilogue, te_wire_layout and the host expansion read it from here.
+struct WireLayout { int passed, detected, light, reward, done, stride; };
+__host__ __device__ constexpr WireLayout wire_layout(int r, int I) {
+  return {0, r, 2 * r, 2 * r + 4 * I, 2 * r + 8 * I, (2 * r + 8 * I + 1 + 15) / 16 * 16};
+}
 constexpr int WIRE_MAX_K = 13;     // 13 * 19 = 247 <= 255
 
 // HBM row header: x[road][0] bits = leading | lastcar << 8 | detected << 16, v[road][0] bits = waiting.
@@ -862,8 +866,8 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
       // Repeater: obs[-I:] / 100 * (2 * phase - 1): int32 / int -> float64, cast to float32 on store
       const float light = __double2float_rn(__dmul_rn(__ddiv_rn((double)el_f, 100.0), (double)(2 * ph_f - 1)));
       if (wire_rec) {
-        reinterpret_cast<float *>(wire_rec + 2 * p.r)[ii] = light;
-        reinterpret_cast<float *>(wire_rec + 2 * p.r + 4 * p.I)[ii] = rew;
+        reinterpret_cast<float *>(wire_rec + wire_layout(p.r, p.I).light)[ii] = light;
+        reinterpret_cast<float *>(wire_rec + wire_layout(p.r, p.I).reward)[ii] = rew;
       } else {
         p.reward[step_env0 * p.I + ibase + i] = rew;
         p.obs_f[(step_env0 + env) * obs_f_len + 2 * p.r + ii] = light;
@@ -879,8 +883,8 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
       p.obs_i[(size_t)env * obs_i_len + p.r + my_road] = det;
     } else if (use_wire) {
       unsigned char *wire_rec = p.wire + (step_env0 + env) * p.wire_stride;
-      wire_rec[my_road] = (unsigned char)passed;
-      wire_rec[p.r + my_road] = (unsigned char)det;
+      wire_rec[wire_layout(p.r, p.I).passed + my_road] = (unsigned char)passed;
+      wire_rec[wire_layout(p.r, p.I).detected + my_road] = (unsigned char)det;
     } else {
       p.obs_f[(step_env0 + env) * obs_f_len + my_road] = (float)passed;
       p.obs_f[(step_env0 + env) * obs_f_len + p.r + my_road] = (float)det;
@@ -911,6 +915,7 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
     const int ticks_run = overflowed ? ov + 1 : p.K;   // >= 1
     const int ticks_total = envm[ENVM_WORDS * g + ENVM_TB] + ticks_run;   // ticks env g has run in this launch
     EnvScalars *esg = p.env + env;
+    // (wire_layout(p.r, p.I).done, spelled out: through the function the compiler schedules this kernel differently)
     if (use_wire) p.wire[(step_env0 + env) * p.wire_stride + 2 * p.r + 8 * p.I] = overflowed ? 1 : 0;
     else p.done[step_env0 + env] = overflowed ? 1 : 0;
     if (!p.raw) {

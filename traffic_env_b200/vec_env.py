@@ -326,14 +326,8 @@ class VecTrafficEnv(object):
 
     def host_float_dma(self):
         """True when te_step(TE_HOST) delivers float outputs through the copy engine instead of expanding wire records
-        on the host (te_api.cu: float_dma; few host cores per GPU, or TE_HOST_FLOAT_DMA=1)."""
-        import os
-        ev = os.environ.get("TE_HOST_FLOAT_DMA")
-        if ev is not None:
-            return ev not in ("0", "")
-        n = C.c_int32(0)
-        self._L.te_device_count(C.byref(n))
-        return bool(n.value) and (os.cpu_count() or 1) // n.value < 8
+        on the host, as the library decided at te_create (few host cores per GPU, or TE_HOST_FLOAT_DMA=1)."""
+        return bool(self.wire.host_float_dma)
 
     def host_path_note(self):
         return ("compact wire records of %d B per env (u8 passed / detected, f32 light / reward, u8 done) expanded on the "
