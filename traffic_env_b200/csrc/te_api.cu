@@ -188,7 +188,6 @@ struct te_handle {
   dev_buf<long long> d_sched_off;
   dev_buf<short> d_sched_roads;
   dev_buf<uint32_t> d_gap_cdf;
-  dev_buf<IdmConst> d_idm;
   // staging for TE_HOST calls
   dev_buf<uint8_t> d_actions, d_done, d_mask, d_init_phase;
   dev_buf<float> d_reward;
@@ -216,44 +215,38 @@ struct te_handle {
 // x 2 CTAs, 101.7 KB each; 3x3 grid: 64 threads x 16 CTAs).
 typedef void (*step_kernel_t)(const StepParams);
 struct StepVariant { step_kernel_t fn; int maxt; };
-#ifndef TE_MINB512
-#define TE_MINB512 2
-#endif
-#ifndef TE_MINB96
-#define TE_MINB96 10   // CTAs per SM the 96-thread variant is compiled for (10: 64 registers; 9: 72)
-#endif
-#ifndef TE_FAST_ARCH
-#define TE_FAST_ARCH 1   // compile the car loop a second time for the reference's archetype (IdmConst.pow2 && delta_is_four)
-#endif
-template <int MAXT, int MINB, bool VALIDATE, bool GROUPED>
-static StepVariant pick_fa(bool fa) {
-#if TE_FAST_ARCH
-  if (fa) return {te_step_kernel<MAXT, MINB, VALIDATE, true, GROUPED>, MAXT};
-#endif
-  (void)fa;
-  return {te_step_kernel<MAXT, MINB, VALIDATE, false, GROUPED>, MAXT};
-}
-// threads = rows of the CTA; grouped = several env instances per CTA (small grids with the reference's archetype,
-// te_create).  20 instantiations of the step kernel: the set is kept small for the sake of build time.
+// threads = rows of the CTA; fa = the car loop compiled for the reference's archetype (IdmConst.pow2 && delta_is_four,
+// tame handles); grouped = several env instances per CTA (small grids with the reference's archetype, te_create).
+// 20 instantiations of the step kernel: the set is kept small for the sake of build time.
 static StepVariant step_variant_for(int threads, bool validate, bool fa, bool grouped) {
   if (validate) {  // + the birth-tick plane in shared memory: one CTA fewer per SM
-    if (threads <= 256) return pick_fa<256, 2, true, false>(false);
-    if (threads <= 512) return pick_fa<512, 1, true, false>(false);
-    return pick_fa<768, 1, true, false>(false);
+    if (threads <= 256) return {te_step_kernel<256, 2, true, false, false>, 256};
+    if (threads <= 512) return {te_step_kernel<512, 1, true, false, false>, 512};
+    return {te_step_kernel<768, 1, true, false, false>, 768};
   }
   if (grouped) {   // (only built for the fast archetype: te_create keeps G = 1 otherwise)
     if (threads <= 64) return {te_step_kernel<64, 16, false, true, true>, 64};
-    if (threads <= 96) return {te_step_kernel<96, TE_MINB96, false, true, true>, 96};   // default 3x3 grid: two envs (2 x 48 roads) on three warps, 20 envs per SM
+    // default 3x3 grid: two envs (2 x 48 roads) on three warps, 20 envs per SM at 64 registers (72 registers and 9 CTAs
+    // per SM measured 2.4 % slower)
+    if (threads <= 96) return {te_step_kernel<96, 10, false, true, true>, 96};
     if (threads <= 128) return {te_step_kernel<128, 8, false, true, true>, 128};
     if (threads <= 160) return {te_step_kernel<160, 6, false, true, true>, 160};
     return {te_step_kernel<256, 4, false, true, true>, 256};
   }
-  if (threads <= 64) return pick_fa<64, 16, false, false>(fa);
-  if (threads <= 128) return pick_fa<128, 8, false, false>(fa);
-  if (threads <= 256) return pick_fa<256, 4, false, false>(fa);
-  if (threads <= 512) return pick_fa<512, TE_MINB512, false, false>(fa);
-  if (threads <= 768) return pick_fa<768, 1, false, false>(fa);
-  return pick_fa<1024, 1, false, false>(fa);
+  if (fa) {
+    if (threads <= 64) return {te_step_kernel<64, 16, false, true, false>, 64};
+    if (threads <= 128) return {te_step_kernel<128, 8, false, true, false>, 128};
+    if (threads <= 256) return {te_step_kernel<256, 4, false, true, false>, 256};
+    if (threads <= 512) return {te_step_kernel<512, 2, false, true, false>, 512};
+    if (threads <= 768) return {te_step_kernel<768, 1, false, true, false>, 768};
+    return {te_step_kernel<1024, 1, false, true, false>, 1024};
+  }
+  if (threads <= 64) return {te_step_kernel<64, 16, false, false, false>, 64};
+  if (threads <= 128) return {te_step_kernel<128, 8, false, false, false>, 128};
+  if (threads <= 256) return {te_step_kernel<256, 4, false, false, false>, 256};
+  if (threads <= 512) return {te_step_kernel<512, 2, false, false, false>, 512};
+  if (threads <= 768) return {te_step_kernel<768, 1, false, false, false>, 768};
+  return {te_step_kernel<1024, 1, false, false, false>, 1024};
 }
 static bool fast_arch(const te_handle *h);
 
@@ -280,7 +273,7 @@ static void fill_idm(IdmConst &c, const float *a, float rate) {
   c.pow2 = is_pow2_f(a[7]) && is_pow2_f(rate) && !getenv("TE_NO_POW2_SHORTCUT");
 }
 
-// The FA kernels are compiled for the reference's archetype AND (TE_TAME_FAST) without the per-car validity predicate:
+// The FA kernels are compiled for the reference's archetype AND without the per-car validity predicate:
 // they may only run while the handle is tame.
 static bool fast_arch(const te_handle *h) { return h->base.idm.pow2 && h->base.idm.delta_is_four && h->tame; }
 
@@ -554,9 +547,6 @@ extern "C" int te_create(const te_config *cfg, te_handle **out) {
   p.gamma = cfg->gamma;
   fill_idm(p.idm, cfg->archetype, cfg->rate);
   h->tame = tame_archetype(cfg, &h->v_cap);
-  CU(alloc(h->d_idm, 1));
-  CU(cudaMemcpy(h->d_idm.get(), &p.idm, sizeof(IdmConst), cudaMemcpyHostToDevice));
-  p.idm_g = h->d_idm.get();
   p.x = h->x.get(); p.v = h->v.get(); p.w = h->w.get(); p.trips = h->d_trips.get(); p.trip_count = h->d_trip_count.get(); p.trip_cap = h->trip_cap;
   p.elapsed = h->elapsed.get(); p.phase = h->phase.get(); p.passed_dst = h->passed_dst.get();
   p.env = h->env.get(); p.stats = h->stats.get(); p.nexts = h->d_nexts.get(); p.up = h->d_up.get(); p.entry_idx = h->d_entry_idx.get();
@@ -978,9 +968,10 @@ extern "C" int te_get_state(te_handle *h, int32_t env_begin, int32_t count, int3
     for (int rd = 0; rd < R; rd++) {
       uint32_t w0; memcpy(&w0, &hx[e * row + (size_t)rd * CAP], 4);
       int wt; memcpy(&wt, &hv[e * row + (size_t)rd * CAP], 4);
-      if (leading) leading[(size_t)e * R + rd] = w0 & 0xff;
-      if (lastcar) lastcar[(size_t)e * R + rd] = (w0 >> 8) & 0xff;
-      if (obs && rd < r) { obs[(size_t)e * ol + rd] = 0; obs[(size_t)e * ol + r + rd] = (w0 >> 16) & 0xff; }
+      const RowHeader m = unpack_meta(w0);
+      if (leading) leading[(size_t)e * R + rd] = m.leading;
+      if (lastcar) lastcar[(size_t)e * R + rd] = m.lastcar;
+      if (obs && rd < r) { obs[(size_t)e * ol + rd] = 0; obs[(size_t)e * ol + r + rd] = m.detected; }
       if (waiting && rd < r) waiting[(size_t)e * r + rd] = wt;
       if (x) { memcpy(&x[((size_t)e * R + rd) * CAP], &hx[e * row + (size_t)rd * CAP], CAP * 4); x[((size_t)e * R + rd) * CAP] = NAN; }
       if (v) { memcpy(&v[((size_t)e * R + rd) * CAP], &hv[e * row + (size_t)rd * CAP], CAP * 4); v[((size_t)e * R + rd) * CAP] = NAN; }
@@ -1200,12 +1191,9 @@ static int test_idm(int device, float rate, const float *a, const float *xl, con
   fill_idm(c, a, rate);
   dev_buf<float> d[7];
   const float *src[5] = {xl, vl, ll, x, v};
-  dev_buf<IdmConst> dc;
-  CU(alloc(dc, 1));
-  CU(cudaMemcpy(dc.get(), &c, sizeof(IdmConst), cudaMemcpyHostToDevice));
   for (int i = 0; i < 7; i++) CU(alloc(d[i], n));
   for (int i = 0; i < 5; i++) CU(cudaMemcpy(d[i].get(), src[i], n * 4, cudaMemcpyHostToDevice));
-  te_test_idm_kernel<<<(unsigned)((n + 255) / 256), 256>>>(c, dc.get(), d[0].get(), d[1].get(), d[2].get(), d[3].get(),
+  te_test_idm_kernel<<<(unsigned)((n + 255) / 256), 256>>>(c, d[0].get(), d[1].get(), d[2].get(), d[3].get(),
                                                            d[4].get(), d[5].get(), d[6].get(), n, unchecked);
   CU(cudaGetLastError());
   CU(cudaMemcpy(x_out, d[5].get(), n * 4, cudaMemcpyDeviceToHost));
@@ -1235,14 +1223,11 @@ extern "C" int te_idm_peak_form(int device, const float *a, float rate, int32_t 
   if (warps_per_sm) { threads = 32 * warps_per_sm; blocks = sms; }   // one CTA of w warps per SM
   dev_buf<float> sink;
   CU(alloc(sink, (size_t)threads * blocks));
-  dev_buf<IdmConst> dc;
-  CU(alloc(dc, 1));
-  CU(cudaMemcpy(dc.get(), &c, sizeof(IdmConst), cudaMemcpyHostToDevice));
   event_ptr e0, e1;
   CU(create(e0, cudaEventDefault)); CU(create(e1, cudaEventDefault));
-  te_idm_peak_kernel<<<blocks, threads>>>(c, dc.get(), iters / 4 + 1, sink.get(), form);  // warm-up
+  te_idm_peak_kernel<<<blocks, threads>>>(c, iters / 4 + 1, sink.get(), form);  // warm-up
   CU(cudaEventRecord(e0.get()));
-  te_idm_peak_kernel<<<blocks, threads>>>(c, dc.get(), iters, sink.get(), form);
+  te_idm_peak_kernel<<<blocks, threads>>>(c, iters, sink.get(), form);
   CU(cudaEventRecord(e1.get()));
   CU(cudaEventSynchronize(e1.get()));
   CU(cudaGetLastError());

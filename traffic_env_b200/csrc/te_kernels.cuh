@@ -82,7 +82,8 @@ struct StepParams {
   int flags, arrival_mode, K, raw, episode_len;
   float gamma;
   IdmConst idm;
-  const IdmConst *idm_g;   // the same constants in global memory (for the out-of-line generic IDM routine)
+  long long env_id_base;        // Philox key of env e: (seed, env_id_base + e).  (Here rather than next to `seed`: at the
+                                // end of the struct, ptxas gives the 768-thread validate kernel two more registers.)
   // state (HBM)
   float *x, *v;           // [E][Rp][20]; slot 0 of a row carries packed ring indices (see pack_meta)
   float *w;               // [E][Rp][20] birth tick of each car (validate mode only, traffic_env.py:34,279)
@@ -122,7 +123,6 @@ struct StepParams {
   const uint32_t *gap_cdf;
   int n_gap;
   uint32_t seed;
-  long long env_id_base;
 };
 
 // Wire record of one env actor step: everything te_step returns, in 1/2.5 of the bytes of the float observation
@@ -136,8 +136,12 @@ __host__ __device__ constexpr WireLayout wire_layout(int r, int I) {
 constexpr int WIRE_MAX_K = 13;     // 13 * 19 = 247 <= 255
 
 // HBM row header: x[road][0] bits = leading | lastcar << 8 | detected << 16, v[road][0] bits = waiting.
+struct RowHeader { int leading, lastcar, detected; };
 __host__ __device__ inline uint32_t pack_meta(int leading, int lastcar, int detected) {
   return (uint32_t)leading | ((uint32_t)lastcar << 8) | ((uint32_t)detected << 16);
+}
+__host__ __device__ inline RowHeader unpack_meta(uint32_t w) {
+  return {(int)(w & 0xff), (int)((w >> 8) & 0xff), (int)((w >> 16) & 0xff)};
 }
 
 // Shared-memory layout of one CTA.  A CTA simulates G env instances (G = 1 for large grids; small grids share a CTA so
@@ -152,6 +156,14 @@ enum : int { ENVM_OVF = 0,    // first overflowing tick of the current actor ste
              ENVM_SKIP = 3,   // env not stepped (env_mask)
              ENVM_SEG = 4,    // tick of the launch (for this env) at which the current controller decision was applied
              ENVM_WORDS = 5 };
+// CTA-level counters (Smem::misc)
+enum : int { CTA_RUNNING = 0,         // envs still running (an env stops after its first overflowing tick)
+             CTA_ORD_TICK = 1,        // last tick of the launch in which some env needed ordered transfers (-1: none)
+             CTA_VEH_UPDATES = 2,     // vehicle updates
+             CTA_OVERFLOWS = 3,       // cars dropped on full rings
+             CTA_GENERATED = 4,       // cars generated
+             CTA_ORD_ENV_TICKS = 5,   // env-ticks that ran ordered transfers
+             CTA_EXITED = 6 };        // cars that left the map
 constexpr int MAX_G = 8;           // most env instances one CTA can hold (te_api.cu: select_layout)
 
 struct SmemLayout {
@@ -284,6 +296,50 @@ __device__ __forceinline__ void red_add_shared(uint32_t a, uint32_t v) {
 
 __device__ __forceinline__ int ring_wrap(int a) { return a >= CAP ? 1 : a; }
 __device__ __forceinline__ int ring_count(int ld, int lc) { return lc - ld + (ld > lc ? RING : 0); }
+// cars on a road from its row header (or from any word with the header's leading and lastcar bytes)
+__device__ __forceinline__ int ring_count(uint32_t header) {
+  const RowHeader m = unpack_meta(header);
+  return ring_count(m.leading, m.lastcar);
+}
+
+// greedy controller (algorithms/greedy.py:14-16): cars_on_roads()[row, col, :] . [1, 1, -1, -1] < 0, where
+// cars(dd) is the number of cars on approach dd (road dd * V + intersection) of the intersection
+template <class Cars>
+__device__ __forceinline__ int greedy_action(Cars cars) {
+  int bal = 0;
+  for (int dd = 0; dd < 4; dd++) {
+    const int n = cars(dd);
+    bal += dd < 2 ? n : -n;
+  }
+  return bal < 0;
+}
+
+// phase / elapsed after the first tick of action `act` (traffic_env.py:225-232)
+__device__ __forceinline__ void apply_action(int &ph, int &el, int act, bool learn_switch) {
+  int change;
+  if (learn_switch) { change = act; ph ^= act; } else { change = ph ^ act; ph = act; }
+  el = (el + 1) * (change ? 0 : 1);
+}
+
+// phase / elapsed n ticks later while the action stays the same: learn_switch with a set action (ls_act) toggles the
+// phase every tick, which keeps elapsed at 0; otherwise the phase is constant and elapsed grows by one per tick
+__device__ __forceinline__ void light_after(int &ph, int &el, bool ls_act, int n) {
+  if (ls_act) { ph ^= n & 1; el = 0; } else el += n;
+}
+
+// remi (traffic_env.py:64-78) of one intersection in phase ph, over its 4 approaches in road order; waiting(dd): cars
+// wait on approach dd
+template <class Waiting>
+__device__ __forceinline__ float remi_reward(int ph, bool passed_dst, Waiting waiting) {
+  float rew = 0.f;
+  for (int dd = 0; dd < 4; dd++) {
+    const bool green = ((dd < 2) ? 1 : 0) != ph;
+    const bool w = waiting(dd);
+    if (w && !green && !passed_dst) rew = __fsub_rn(rew, 0.5f);
+    else if (passed_dst && green && !w) rew = __fadd_rn(rew, 0.5f);
+  }
+  return rew;
+}
 
 // add_car (traffic_env.py:97-114) for one identical-archetype car at (xin, vin); `chk` is the value
 // of leading[road] the reference would see at that moment.  Returns false when the ring is full.
@@ -307,9 +363,11 @@ struct Smem {
   float *rew;            // reward of the finished actor step per intersection (for the return statistic)
   unsigned long long *mbar;
   int *envm;             // per env of the CTA: ENVM_WORDS words (tick stamps, ticks run, skip flag)
-  int *misc;             // CTA level: [0] envs still running, [1] last tick in which some env needed ordered transfers, [2] vehicle updates, [3] overflows, [4] generated, [5] ordered-transfer env-ticks, [6] cars that left the map
+  int *misc;             // CTA level: the CTA_* counters
   uint8_t *warp, *phase, *act, *pdst, *cnt;
   const PowfTables *tabs;  // glibc powf tables (global memory, L1-resident: read by ~0.4 % of the cars)
+  // word w (ENVM_*) of env g of the CTA
+  __device__ __forceinline__ int &env_word(int g, int w) const { return envm[g * ENVM_WORDS + w]; }
 };
 
 __device__ __forceinline__ Smem carve(unsigned char *base, const SmemLayout &L) {
@@ -344,12 +402,23 @@ __device__ __forceinline__ int transfer(const StepParams &p, const Smem &s, int 
 }
 
 constexpr int NO_OVERFLOW = 0x7fffffff;
-#ifndef TE_TAME_FAST
-#define TE_TAME_FAST 1   // the FA kernels run the unchecked arithmetic (te_math.cuh: CHECKED = false); te_api.cu only launches them on tame handles
-#endif
-#ifndef TE_UNIFORM_CAR_LOOP
-#define TE_UNIFORM_CAR_LOOP 1   // measured: the per-lane trip count (0) is 4.5 % / 8 % slower (10x10 / 3x3): lanes drifting apart cost more than the re-convergence
-#endif
+
+// `dropped` cars of env g were lost on full rings in tick t; the env's first overflow stops it after this tick
+__device__ __forceinline__ void note_overflow(const Smem &s, int g, int t, int dropped) {
+  atomicAdd(&s.misc[CTA_OVERFLOWS], dropped);
+  if (atomicMin(&s.env_word(g, ENVM_OVF), t) == NO_OVERFLOW) atomicSub(&s.misc[CTA_RUNNING], 1);
+}
+
+// update_lights (traffic_env.py:81-94) in closed form: while an action holds, the approach of train road `road` of
+// intersection i is blocked (red or yellow) at tick tt of the launch  <=>  tt < light_ylim(...).  learn_switch with a set
+// action toggles every tick, which keeps elapsed at 0 (always yellow); otherwise phase is constant and elapsed grows by
+// one per tick from the state s.phase / s.elapsed that the action's first tick, tick `origin` of the launch, left.
+// (A new actor step with the same action changes nothing: its first tick finds phase == action.)
+__device__ __forceinline__ int light_ylim(const Smem &s, int i, int road, int V, bool learn_switch, int origin) {
+  const bool ls_act = learn_switch && s.act[i];
+  const int road_phase = (road / V) < 2;
+  return (ls_act || road_phase == (int)s.phase[i]) ? 0x7fffffff : origin + YELLOW_TICKS - s.elapsed[i];
+}
 
 // GROUPED = false: one env per CTA (p.G == 1), everything about env groups folds away at compile time.
 template <int MAXT, int MINB, bool VALIDATE, bool FA, bool GROUPED>
@@ -376,7 +445,6 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
   // run-time tail of the shared-memory layout (per env: arrival counts, Philox snapshots)
   const int cnt_stride = cnt_stride_bytes(KT, p.n_entry);
   uint32_t *const snap_base = reinterpret_cast<uint32_t *>(s.cnt + tail_snap_offset(KT, p.n_entry, G));
-  int *const envm = s.envm;
   const int nrows = ng * p.R;                                // live rows (super-roads) of this CTA
   const int nI = ng * p.I;
   const size_t ibase = (size_t)env_first * p.I;              // the per-intersection arrays of consecutive envs are contiguous
@@ -395,11 +463,14 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
       if (VALIDATE) bulk_load(s.ws + g * p.R * CAP, p.w + off, plane_bytes, s.mbar);
     }
   }
-  if (tid == 0) { s.misc[0] = nactive; s.misc[1] = -1; s.misc[2] = 0; s.misc[3] = 0; s.misc[4] = 0; s.misc[5] = 0; s.misc[6] = 0; }
+  if (tid == 0) {
+    s.misc[CTA_RUNNING] = nactive; s.misc[CTA_ORD_TICK] = -1; s.misc[CTA_VEH_UPDATES] = 0; s.misc[CTA_OVERFLOWS] = 0;
+    s.misc[CTA_GENERATED] = 0; s.misc[CTA_ORD_ENV_TICKS] = 0; s.misc[CTA_EXITED] = 0;
+  }
   if (tid < G) {
-    envm[ENVM_WORDS * tid + ENVM_OVF] = NO_OVERFLOW; envm[ENVM_WORDS * tid + ENVM_ORD] = -1; envm[ENVM_WORDS * tid + ENVM_TB] = 0;
-    envm[ENVM_WORDS * tid + ENVM_SEG] = 0;
-    envm[ENVM_WORDS * tid + ENVM_SKIP] = (tid >= ng) || (p.env_mask && p.env_mask[env_first + tid] == 0);
+    s.env_word(tid, ENVM_OVF) = NO_OVERFLOW; s.env_word(tid, ENVM_ORD) = -1; s.env_word(tid, ENVM_TB) = 0;
+    s.env_word(tid, ENVM_SEG) = 0;
+    s.env_word(tid, ENVM_SKIP) = (tid >= ng) || (p.env_mask && p.env_mask[env_first + tid] == 0);
   }
   for (int g = warp; g < ng; g += nwarps) {
     // arrivals of the KT ticks of env g as per-tick, per-entry-road counts (cars are identical, so the
@@ -481,21 +552,12 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
   mbar_wait(s.mbar, 0);  // the ring planes have landed
   if (tid < nI) {
     const int i = tid;
-    if (p.controller == CTRL_GREEDY) {
-      // algorithms/greedy.py:14-16: cars_on_roads()[row, col, :] . [1, 1, -1, -1] < 0 from the ring indices as staged
+    if (p.controller == CTRL_GREEDY) {   // from the row headers as staged
       const int g = i / p.I, ii = i - g * p.I;
-      int bal = 0;
-      for (int dd = 0; dd < 4; dd++) {
-        const uint32_t w0 = __float_as_uint(s.xs[(g * p.R + dd * p.V + ii) * CAP]);
-        const int cn = ring_count(w0 & 0xff, (w0 >> 8) & 0xff);
-        bal += dd < 2 ? cn : -cn;
-      }
-      li_act = bal < 0;
+      li_act = greedy_action([&](int dd) { return ring_count(__float_as_uint(s.xs[(g * p.R + dd * p.V + ii) * CAP])); });
       if (p.actions_out) p.actions_out[ibase + i] = (uint8_t)li_act;
     }
-    int change;
-    if (learn_switch) { change = li_act; li_ph ^= li_act; } else { change = li_ph ^ li_act; li_ph = li_act; }
-    li_el = (li_el + 1) * (change ? 0 : 1);
+    apply_action(li_ph, li_el, li_act, learn_switch);
     s.phase[i] = (uint8_t)li_ph; s.act[i] = (uint8_t)li_act; s.elapsed[i] = li_el;
     s.pdst[i] = (uint8_t)li_pd; s.ovf[i] = 0;
   }
@@ -514,8 +576,7 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
     short *owner = reinterpret_cast<short *>(s.meta);        // idle until the tick loop
     for (int i = tid; i < 40; i += blockDim.x) hist[i] = 0;
     __syncthreads();
-    const uint32_t w0 = __float_as_uint(s.xs[tid * CAP]);
-    const int n0 = ring_count(w0 & 0xff, (w0 >> 8) & 0xff);
+    const int n0 = ring_count(__float_as_uint(s.xs[tid * CAP]));
     atomicAdd(&hist[n0], 1);
     __syncthreads();
     int base = 0;
@@ -536,12 +597,11 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
   float *xr = s.xs + my_sr * CAP, *vr = s.vs + my_sr * CAP;
   float *wr = VALIDATE ? s.ws + my_sr * CAP : nullptr;
   const float steps0 = p.env[env_first + my_g].steps;  // np.float32 tick counter at the start of this launch (small integer: exact)
-  const int emi = ENVM_WORDS * my_g;                         // my env's words inside envm
   int ld, lc, wait, det, passed = 0;
   float leadx;
   {
-    const uint32_t w0 = __float_as_uint(xr[0]);
-    ld = w0 & 0xff; lc = (w0 >> 8) & 0xff; det = (w0 >> 16) & 0xff;
+    const RowHeader m = unpack_meta(__float_as_uint(xr[0]));
+    ld = m.leading; lc = m.lastcar; det = m.detected;
     wait = __float_as_int(vr[0]);
     leadx = xr[ld];
     s.tailx[my_sr] = (lc != ld) ? xr[lc] : INF;
@@ -557,17 +617,7 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
     }
   }
   const int dst = is_train ? my_g * p.I + my_road % p.V : 0;
-  // update_lights (traffic_env.py:81-94) in closed form: within one launch the action is constant, so the approach
-  // is blocked (red or yellow) at tick tt of the launch  <=>  tt < ylim.  learn_switch with a set action toggles every
-  // tick, which keeps elapsed at 0 (always yellow); otherwise phase is constant and elapsed = elapsed_0 + tt.  (A new
-  // actor step with the same action changes nothing: its first tick finds phase == action.)
-  int ylim = 0;
-  if (is_train) {
-    const bool ls_act = learn_switch && s.act[dst];
-    const int road_phase = (my_road / p.V) < 2;
-    const int el0 = s.elapsed[dst];
-    ylim = (ls_act || road_phase == (int)s.phase[dst]) ? 0x7fffffff : YELLOW_TICKS - el0;
-  }
+  int ylim = is_train ? light_ylim(s, dst, my_road, p.V, learn_switch, 0) : 0;   // the approach is blocked while tt < ylim
   // per-warp tables of the car loop (rebuilt every tick)
   // (all three are reached from ONE 32-bit shared address, rt_a, with immediates: no generic pointers kept per table)
   const uint32_t rt_a = smem_u32(s.warp + warp * WARP_AREA);             // rt: non-empty roads of the warp, in lane order:
@@ -585,7 +635,7 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
   const bool clear_remi = !p.raw && (p.flags & F_REMI);
   const bool use_wire = !p.raw && p.wire;
   // a row that never takes part: padding, or a road of an env that is not stepped (env_mask)
-  const bool out_of_play = GROUPED ? (!is_road || envm[emi + ENVM_SKIP] != 0) : false;
+  const bool out_of_play = GROUPED ? (!is_road || s.env_word(my_g, ENVM_SKIP) != 0) : false;
   int veh_local = 0, gen_local = 0, exit_local = 0;
   int tb = 0;            // ticks my env ran in the earlier actor steps of this launch (te_step_multi)
 
@@ -603,32 +653,19 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
     __syncthreads();
     if (tid < nI) {
       const int i = tid, g = i / p.I, ii = i - g * p.I;
-      if (!(GROUPED && envm[ENVM_WORDS * g + ENVM_SKIP])) {
-        const int rel = envm[ENVM_WORDS * g + ENVM_TB] - 1 - envm[ENVM_WORDS * g + ENVM_SEG];   // last tick run, from the segment origin
-        const bool ls_prev = learn_switch && s.act[i];
-        int ph = s.phase[i] ^ (ls_prev ? (rel & 1) : 0);
-        int el = ls_prev ? 0 : s.elapsed[i] + rel;
-        int bal = 0;
-        for (int dd = 0; dd < 4; dd++) {
-          const uint32_t m = s.meta[g * p.R + dd * p.V + ii];
-          const int cn = ring_count(m & 0xff, (m >> 8) & 0xff);
-          bal += dd < 2 ? cn : -cn;
-        }
-        const int act = bal < 0;
+      if (!(GROUPED && s.env_word(g, ENVM_SKIP))) {
+        int ph = s.phase[i], el = s.elapsed[i];
+        light_after(ph, el, learn_switch && s.act[i],   // to the last tick run, from the segment origin
+                    s.env_word(g, ENVM_TB) - 1 - s.env_word(g, ENVM_SEG));
+        const int act = greedy_action([&](int dd) { return ring_count(s.meta[g * p.R + dd * p.V + ii]); });
         if (p.actions_out) p.actions_out[(size_t)(step / p.decide_every) * p.num_envs * p.I + ibase + i] = (uint8_t)act;
-        int change;
-        if (learn_switch) { change = act; ph ^= act; } else { change = ph ^ act; ph = act; }
-        el = (el + 1) * (change ? 0 : 1);
+        apply_action(ph, el, act, learn_switch);
         s.phase[i] = (uint8_t)ph; s.act[i] = (uint8_t)act; s.elapsed[i] = el;
       }
     }
     __syncthreads();
-    if (tid < ng) envm[ENVM_WORDS * tid + ENVM_SEG] = envm[ENVM_WORDS * tid + ENVM_TB];
-    if (is_train) {
-      const bool ls_act = learn_switch && s.act[dst];
-      const int road_phase = (my_road / p.V) < 2;
-      ylim = (ls_act || road_phase == (int)s.phase[dst]) ? 0x7fffffff : tb + YELLOW_TICKS - s.elapsed[dst];
-    }
+    if (tid < ng) s.env_word(tid, ENVM_SEG) = s.env_word(tid, ENVM_TB);
+    if (is_train) ylim = light_ylim(s, dst, my_road, p.V, learn_switch, tb);
   }
   bool frozen = out_of_play;
   for (int t = 0; t < p.K; t++) {
@@ -693,19 +730,15 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
       }
       __syncwarp();  // every run has read the leader of its first car before any lane overwrites a slot
       unsigned int acc = 0u;
-#if TE_UNIFORM_CAR_LOOP
+      // a uniform trip count: a per-lane one (the lanes of the shorter runs leaving early) measured 4.5 % / 8 % slower
+      // (10x10 / 3x3): lanes drifting apart cost more than the re-convergence
       for (int i = 0; i < q; i++) {
         if (i < cnt) {
-#else
-      // per-lane trip count: the lanes of the last, shorter runs simply leave the loop early (nothing inside is a
-      // warp-level operation), which spares the loop a uniform counter and a warp re-convergence per iteration
-      for (int i = cnt; i > 0; i--) {
-        {
-#endif
           float xn = lds_f32(addr), vn = lds_f32_off<VOFF>(addr);
           const float xl = px, vl = pv, ll = pl;
           px = xn; pv = vn; pl = c.len;
-          idm_update<FA, !(FA && TE_TAME_FAST)>(c, p.idm_g, s.tabs, xl, vl, ll, xn, vn);
+          // the FA kernels run the unchecked arithmetic; te_api.cu only launches them on tame handles
+          idm_update<FA, !FA>(c, s.tabs, xl, vl, ll, xn, vn);
           sts_f32(addr, xn); sts_f32_off<VOFF>(addr, vn);
           // wrapped ring, low segment (slot < leading): the reference tests x, not v (traffic_env.py:210).
           // THRESH = 0.2 is compared in double by the reference; 0.2f is the smallest float above 0.2, so for every
@@ -766,7 +799,7 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
           // Two or more pops while the upstream road has a higher index: its insert (which in the
           // reference runs after these pops were consumed) could reuse the slots the popped cars
           // still occupy.  Run this tick's transfers of this env in strict road order instead.
-          if (npop >= 2 && upr > my_sr) { envm[emi + ENVM_ORD] = gt; s.misc[1] = gt; }
+          if (npop >= 2 && upr > my_sr) { s.env_word(my_g, ENVM_ORD) = gt; s.misc[CTA_ORD_TICK] = gt; }
         }
       }
     }
@@ -774,48 +807,45 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
     __syncthreads();
     // ---------------------------------------------------------------- phase C
     const bool want_parallel = !frozen && upr >= 0 && (s.meta[upr] >> 24) != 0;
-    if (s.misc[1] == gt || (p.flags & F_ORDERED)) {      // (CTA-uniform) some env of the CTA needs ordered transfers
-      const bool ord_env = !frozen && (GROUPED ? is_road : true) && (envm[emi + ENVM_ORD] == gt || (p.flags & F_ORDERED));
-      if (ord_env) {
-        if (my_road == 0) {                              // one lane per env walks its roads in the reference's order
-          const int row0 = my_g * p.R;
-          int dr_total = 0;
-          for (int e = 0; e < p.R; e++) {
-            const int d = p.nexts[e];
-            if (d < 0 || (s.meta[row0 + e] >> 24) == 0) continue;
-            const uint32_t md = s.meta[row0 + d];
-            int dlc = (md >> 8) & 0xff;
-            const int chk = (e < d) ? (md >> 16) & 0xff : md & 0xff;
-            const int dr = transfer(p, s, row0 + e, row0 + d, chk, dlc, VALIDATE);
-            s.meta[row0 + d] = (md & 0xffff00ffu) | ((uint32_t)dlc << 8);
-            if (dr) { if (d < p.r) atomicAdd(&s.ovf[my_g * p.I + d % p.V], dr); dr_total += dr; }
-          }
-          if (dr_total) {
-            atomicAdd(&s.misc[3], dr_total);
-            if (atomicMin(&envm[emi + ENVM_OVF], t) == NO_OVERFLOW) atomicSub(&s.misc[0], 1);
-          }
-          atomicAdd(&s.misc[5], 1);
+    // (CTA-uniform) some env of the CTA needs ordered transfers in this tick
+    const bool ordered_tick = s.misc[CTA_ORD_TICK] == gt || (p.flags & F_ORDERED);
+    const bool ord_env = ordered_tick && !frozen && (GROUPED ? is_road : true) &&
+                         (s.env_word(my_g, ENVM_ORD) == gt || (p.flags & F_ORDERED));
+    if (ord_env) {
+      if (my_road == 0) {                                // one lane per env walks its roads in the reference's order
+        const int row0 = my_g * p.R;
+        int dr_total = 0;
+        for (int e = 0; e < p.R; e++) {
+          const int d = p.nexts[e];
+          if (d < 0 || (s.meta[row0 + e] >> 24) == 0) continue;
+          const uint32_t md = s.meta[row0 + d];
+          int dlc = (md >> 8) & 0xff;
+          const int chk = (e < d) ? (md >> 16) & 0xff : md & 0xff;
+          const int dr = transfer(p, s, row0 + e, row0 + d, chk, dlc, VALIDATE);
+          s.meta[row0 + d] = (md & 0xffff00ffu) | ((uint32_t)dlc << 8);
+          if (dr) { if (d < p.r) atomicAdd(&s.ovf[my_g * p.I + d % p.V], dr); dr_total += dr; }
         }
-      } else if (want_parallel) {
-        dropped += transfer(p, s, upr, my_sr, (upr < my_sr) ? ld_pre : ld, lc, VALIDATE);
+        if (dr_total) note_overflow(s, my_g, t, dr_total);
+        atomicAdd(&s.misc[CTA_ORD_ENV_TICKS], 1);
       }
-      __syncthreads();
-      if (ord_env) lc = (s.meta[my_sr] >> 8) & 0xff;
     } else if (want_parallel) {
       dropped += transfer(p, s, upr, my_sr, (upr < my_sr) ? ld_pre : ld, lc, VALIDATE);
     }
+    if (ordered_tick) {
+      __syncthreads();
+      if (ord_env) lc = (s.meta[my_sr] >> 8) & 0xff;
+    }
     if (dropped) {  // OVERFLOW_PENALTY on the road's intersection, traffic_env.py:109-111; done
       if (is_train) atomicAdd(&s.ovf[dst], dropped);
-      atomicAdd(&s.misc[3], dropped);
-      if (atomicMin(&envm[emi + ENVM_OVF], t) == NO_OVERFLOW) atomicSub(&s.misc[0], 1);   // the first overflow of this env: it stops after this tick
+      note_overflow(s, my_g, t, dropped);
     }
     s.tailx[my_sr] = (lc != ld) ? xr[lc] : INF;
     __syncthreads();
     // tick-stamped (a fast warp that has already flagged tick t + 1 cannot be mistaken for tick t)
     if (GROUPED) {
-      frozen = frozen || envm[emi + ENVM_OVF] <= t;
-      if (s.misc[0] <= 0) break;  // every env of the CTA has stopped
-    } else if (envm[ENVM_OVF] <= t) break;
+      frozen = frozen || s.env_word(my_g, ENVM_OVF) <= t;
+      if (s.misc[CTA_RUNNING] <= 0) break;  // every env of the CTA has stopped
+    } else if (s.env_word(0, ENVM_OVF) <= t) break;
   }
 
   // ------------------------------------------------------------ end of the actor step: observation, reward, done
@@ -823,38 +853,28 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
   s.wait[my_sr] = wait;
   __syncthreads();
   {
-    const int ov = envm[emi + ENVM_OVF];
+    const int ov = s.env_word(my_g, ENVM_OVF);
     tb += (ov != NO_OVERFLOW) ? ov + 1 : p.K;     // ticks my env has run so far in this launch
   }
   const size_t step_env0 = (size_t)step * p.num_envs;      // outputs of actor step j: j * num_envs env slots further on
   // final light state after the ticks each env ran, reward
   for (int i = tid; i < nI; i += blockDim.x) {
     const int g = i / p.I, ii = i - g * p.I;
-    if (GROUPED && envm[ENVM_WORDS * g + ENVM_SKIP]) continue;
+    if (GROUPED && s.env_word(g, ENVM_SKIP)) continue;
     const int env = env_first + g;
-    const int ov = envm[ENVM_WORDS * g + ENVM_OVF];
+    const int ov = s.env_word(g, ENVM_OVF);
     // the last tick of the launch env g ran, counted from the tick its current controller decision was applied at
-    const int last = envm[ENVM_WORDS * g + ENVM_TB] + ((ov != NO_OVERFLOW) ? ov : p.K - 1) - envm[ENVM_WORDS * g + ENVM_SEG];
+    const int last = s.env_word(g, ENVM_TB) + ((ov != NO_OVERFLOW) ? ov : p.K - 1) - s.env_word(g, ENVM_SEG);
     unsigned char *wire_rec = use_wire ? p.wire + (step_env0 + env) * p.wire_stride : nullptr;
-    const bool ls_act = learn_switch && s.act[i];
-    const int ph_f = s.phase[i] ^ (ls_act ? (last & 1) : 0);
-    const int el_f = ls_act ? 0 : s.elapsed[i] + last;
+    int ph_f = s.phase[i], el_f = s.elapsed[i];
+    light_after(ph_f, el_f, learn_switch && s.act[i], last);
     if (last_step) {
       p.phase[ibase + i] = (uint8_t)ph_f;
       p.elapsed[ibase + i] = el_f;
     }
     float rew = (float)(-10 * s.ovf[i]);  // OVERFLOW_PENALTY summed over the ticks: small integers, exact, +0 when none
     if (clear_remi) {
-      // remi, traffic_env.py:64-78, over the 4 approaches of intersection ii in road order
-      rew = 0.f;
-      const bool pd = s.pdst[i] != 0;
-      for (int dd = 0; dd < 4; dd++) {
-        const int e = g * p.R + dd * p.V + ii;
-        const bool green = ((dd < 2) ? 1 : 0) != ph_f;
-        const bool w = s.wait[e] > 0;
-        if (w && !green && !pd) rew = __fsub_rn(rew, 0.5f);
-        else if (pd && green && !w) rew = __fadd_rn(rew, 0.5f);
-      }
+      rew = remi_reward(ph_f, s.pdst[i] != 0, [&](int dd) { return s.wait[g * p.R + dd * p.V + ii] > 0; });
       s.pdst[i] = 0;
     }
     if (last_step) p.passed_dst[ibase + i] = s.pdst[i];
@@ -898,7 +918,10 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
       gen_local += __shfl_xor_sync(FULL, gen_local, o);
       exit_local += __shfl_xor_sync(FULL, exit_local, o);
     }
-    if (lane == 0) { atomicAdd(&s.misc[2], veh_local); atomicAdd(&s.misc[4], gen_local); atomicAdd(&s.misc[6], exit_local); }
+    if (lane == 0) {
+      atomicAdd(&s.misc[CTA_VEH_UPDATES], veh_local); atomicAdd(&s.misc[CTA_GENERATED], gen_local);
+      atomicAdd(&s.misc[CTA_EXITED], exit_local);
+    }
   }
   if (last_step && !out_of_play) {
     // pack ring indices back into the row headers, restore the virtual leader's x (then: flush)
@@ -908,12 +931,12 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
     fence_proxy_async();  // my generic-proxy writes to the planes become visible to the bulk-copy engine
   }
   __syncthreads();
-  if (tid < ng && !envm[ENVM_WORDS * tid + ENVM_SKIP]) {          // thread g: the scalars of env g for this actor step
+  if (tid < ng && !s.env_word(tid, ENVM_SKIP)) {          // thread g: the scalars of env g for this actor step
     const int g = tid, env = env_first + g;
-    const int ov = envm[ENVM_WORDS * g + ENVM_OVF];
+    const int ov = s.env_word(g, ENVM_OVF);
     const bool overflowed = ov != NO_OVERFLOW;
     const int ticks_run = overflowed ? ov + 1 : p.K;   // >= 1
-    const int ticks_total = envm[ENVM_WORDS * g + ENVM_TB] + ticks_run;   // ticks env g has run in this launch
+    const int ticks_total = s.env_word(g, ENVM_TB) + ticks_run;   // ticks env g has run in this launch
     EnvScalars *esg = p.env + env;
     // (wire_layout(p.r, p.I).done, spelled out: through the function the compiler schedules this kernel differently)
     if (use_wire) p.wire[(step_env0 + env) * p.wire_stride + 2 * p.r + 8 * p.I] = overflowed ? 1 : 0;
@@ -939,12 +962,12 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
       }
       atomicAdd(&p.stats->ticks, (unsigned long long)ticks_total);
     } else {   // re-arm the stamps of env g for the next actor step
-      envm[ENVM_WORDS * g + ENVM_TB] = ticks_total;
-      envm[ENVM_WORDS * g + ENVM_OVF] = NO_OVERFLOW;   // (raised only after the first barrier of a tick: safe to reset here)
+      s.env_word(g, ENVM_TB) = ticks_total;
+      s.env_word(g, ENVM_OVF) = NO_OVERFLOW;   // (raised only after the first barrier of a tick: safe to reset here)
     }
   }
   if (last_step) break;
-  if (tid == 0) s.misc[0] = nactive;   // (decremented only after the first barrier of a tick: safe to reset here)
+  if (tid == 0) s.misc[CTA_RUNNING] = nactive;   // (decremented only after the first barrier of a tick: safe to reset here)
   }
 
   // ------------------------------------------------------------ flush
@@ -955,11 +978,11 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
       bulk_store(p.v + off, s.vs + g * p.R * CAP, plane_bytes);
       if (VALIDATE) bulk_store(p.w + off, s.ws + g * p.R * CAP, plane_bytes);
     }
-    atomicAdd(&p.stats->vehicle_updates, (unsigned long long)s.misc[2]);
-    if (s.misc[3]) atomicAdd(&p.stats->overflows, (unsigned long long)s.misc[3]);
-    atomicAdd(&p.stats->cars_generated, (unsigned long long)s.misc[4]);
-    if (s.misc[5]) atomicAdd(&p.stats->seq_fallback_ticks, (unsigned long long)s.misc[5]);
-    if (s.misc[6]) atomicAdd(&p.stats->cars_exited, (unsigned long long)s.misc[6]);
+    atomicAdd(&p.stats->vehicle_updates, (unsigned long long)s.misc[CTA_VEH_UPDATES]);
+    if (s.misc[CTA_OVERFLOWS]) atomicAdd(&p.stats->overflows, (unsigned long long)s.misc[CTA_OVERFLOWS]);
+    atomicAdd(&p.stats->cars_generated, (unsigned long long)s.misc[CTA_GENERATED]);
+    if (s.misc[CTA_ORD_ENV_TICKS]) atomicAdd(&p.stats->seq_fallback_ticks, (unsigned long long)s.misc[CTA_ORD_ENV_TICKS]);
+    if (s.misc[CTA_EXITED]) atomicAdd(&p.stats->cars_exited, (unsigned long long)s.misc[CTA_EXITED]);
     bulk_commit_wait();  // the flush has left shared memory before the CTA retires
   }
 }
@@ -1006,7 +1029,7 @@ __global__ void te_reset_kernel(StepParams p, const uint8_t *mask, const uint8_t
     if (!doit) continue;
     float *x = p.x + (size_t)env * p.Rp * CAP, *v = p.v + (size_t)env * p.Rp * CAP;
     for (int road = tid; road < p.Rp; road += blockDim.x) {
-      const int det = (__float_as_uint(x[road * CAP]) >> 16) & 0xff;  // `detected` survives a reset
+      const int det = unpack_meta(__float_as_uint(x[road * CAP])).detected;  // `detected` survives a reset
       x[road * CAP] = __uint_as_float(pack_meta(1, 1, det));
       v[road * CAP] = __int_as_float(0);
       x[road * CAP + 1] = __int_as_float(0x7f800000);
@@ -1044,17 +1067,8 @@ __global__ void te_remi_kernel(StepParams p, float *reward) {
   const int env = blockIdx.x;
   float *v = p.v + (size_t)env * p.Rp * CAP;
   for (int i = threadIdx.x; i < p.I; i += blockDim.x) {
-    const int ph = p.phase[(size_t)env * p.I + i];
-    const bool pd = p.passed_dst[(size_t)env * p.I + i] != 0;
-    float rew = 0.f;
-    for (int dd = 0; dd < 4; dd++) {
-      const int e = dd * p.V + i;
-      const bool green = ((dd < 2) ? 1 : 0) != ph;
-      const bool w = __float_as_int(v[e * CAP]) > 0;
-      if (w && !green && !pd) rew = __fsub_rn(rew, 0.5f);
-      else if (pd && green && !w) rew = __fadd_rn(rew, 0.5f);
-    }
-    reward[(size_t)env * p.I + i] = rew;
+    reward[(size_t)env * p.I + i] = remi_reward(p.phase[(size_t)env * p.I + i], p.passed_dst[(size_t)env * p.I + i] != 0,
+                                                [&](int dd) { return __float_as_int(v[(dd * p.V + i) * CAP]) > 0; });
   }
   __syncthreads();
   for (int i = threadIdx.x; i < p.I; i += blockDim.x) p.passed_dst[(size_t)env * p.I + i] = 0;
@@ -1066,21 +1080,15 @@ __global__ void te_cars_kernel(StepParams p, int *out) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (long long)p.num_envs * p.R) return;
   const int env = (int)(i / p.R), road = (int)(i % p.R);
-  const uint32_t w0 = __float_as_uint(p.x[((size_t)env * p.Rp + road) * CAP]);
-  out[i] = ring_count(w0 & 0xff, (w0 >> 8) & 0xff);
+  out[i] = ring_count(__float_as_uint(p.x[((size_t)env * p.Rp + road) * CAP]));
 }
 
-// greedy controller (algorithms/greedy.py:14-16): cars_on_roads()[row, col, :] . [1,1,-1,-1] < 0
+// the greedy controller's actions from the row headers in HBM
 __global__ void te_greedy_kernel(StepParams p, uint8_t *actions) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (long long)p.num_envs * p.I) return;
   const int env = (int)(i / p.I), it = (int)(i % p.I);
-  int cnt[4];
-  for (int dd = 0; dd < 4; dd++) {
-    const uint32_t w0 = __float_as_uint(p.x[((size_t)env * p.Rp + dd * p.V + it) * CAP]);
-    cnt[dd] = ring_count(w0 & 0xff, (w0 >> 8) & 0xff);
-  }
-  actions[i] = (cnt[0] + cnt[1] - cnt[2] - cnt[3]) < 0 ? 1 : 0;
+  actions[i] = (uint8_t)greedy_action([&](int dd) { return ring_count(__float_as_uint(p.x[((size_t)env * p.Rp + dd * p.V + it) * CAP])); });
 }
 
 // ---- test hooks
@@ -1088,20 +1096,20 @@ __global__ void te_test_powf_kernel(const float *x, float y, float *out, long lo
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) out[i] = powf_glibc(x[i], y, &g_powf_tables);
 }
-__global__ void te_test_idm_kernel(IdmConst c, const IdmConst *cg, const float *xl, const float *vl, const float *ll, const float *x,
+__global__ void te_test_idm_kernel(IdmConst c, const float *xl, const float *vl, const float *ll, const float *x,
                                    const float *v, float *xo, float *vo, long long n, int unchecked) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) {
     float xx = x[i], vv = v[i];
-    if (unchecked) idm_update<true, false>(c, cg, &g_powf_tables, xl[i], vl[i], ll[i], xx, vv);   // tame operands only
-    else if (c.pow2 && c.delta_is_four) idm_update<true, true>(c, cg, &g_powf_tables, xl[i], vl[i], ll[i], xx, vv);
-    else idm_update<false, true>(c, cg, &g_powf_tables, xl[i], vl[i], ll[i], xx, vv);
+    if (unchecked) idm_update<true, false>(c, &g_powf_tables, xl[i], vl[i], ll[i], xx, vv);   // tame operands only
+    else if (c.pow2 && c.delta_is_four) idm_update<true, true>(c, &g_powf_tables, xl[i], vl[i], ll[i], xx, vv);
+    else idm_update<false, true>(c, &g_powf_tables, xl[i], vl[i], ll[i], xx, vv);
     xo[i] = xx; vo[i] = vv;
   }
 }
 // Arithmetic-only ceiling: every lane runs `iters` dependent IDM updates of one car behind a leader that
 // drives at constant speed (registers only, full-precision path: both divisions and powf every time).
-__global__ void te_idm_peak_kernel(IdmConst c, const IdmConst *cg, int iters, float *sink, int ilp2) {
+__global__ void te_idm_peak_kernel(IdmConst c, int iters, float *sink, int ilp2) {
   __shared__ PowfTables tabs;
   for (int i = threadIdx.x; i < (int)(sizeof(PowfTables) / 8); i += blockDim.x)
     reinterpret_cast<unsigned long long *>(&tabs)[i] = reinterpret_cast<const unsigned long long *>(&g_powf_tables)[i];
@@ -1112,7 +1120,7 @@ __global__ void te_idm_peak_kernel(IdmConst c, const IdmConst *cg, int iters, fl
   const float vl = 9.f, step = __fmul_rn(vl, c.rate);
   if (ilp2 == 5) {   // what the step kernels run on a tame handle: archetype flags known at compile time, no validity predicate
     for (int i = 0; i < iters; i++) {
-      idm_update<true, false>(c, cg, &tabs, xl, vl, c.len, x, v);
+      idm_update<true, false>(c, &tabs, xl, vl, c.len, x, v);
       xl = __fadd_rn(xl, step);
     }
     sink[gid] = x + v;
@@ -1120,7 +1128,7 @@ __global__ void te_idm_peak_kernel(IdmConst c, const IdmConst *cg, int iters, fl
   }
   if (ilp2 == 4) {   // the same with the validity predicate and the generic fallback (a handle that saw a wild car)
     for (int i = 0; i < iters; i++) {
-      idm_update<true, true>(c, cg, &tabs, xl, vl, c.len, x, v);
+      idm_update<true, true>(c, &tabs, xl, vl, c.len, x, v);
       xl = __fadd_rn(xl, step);
     }
     sink[gid] = x + v;
@@ -1149,15 +1157,15 @@ __global__ void te_idm_peak_kernel(IdmConst c, const IdmConst *cg, int iters, fl
     // latency study: TWO independent cars per lane (one straight-line block: the compiler interleaves the chains)
     float x2 = 1.f, v2 = 6.f + 0.001f * (float)(gid & 511), xl2 = 40.f + 0.01f * (float)(gid & 127);
     for (int i = 0; i < iters; i++) {
-      idm_update<false, true>(c, cg, &tabs, xl, vl, c.len, x, v);
-      idm_update<false, true>(c, cg, &tabs, xl2, vl, c.len, x2, v2);
+      idm_update<false, true>(c, &tabs, xl, vl, c.len, x, v);
+      idm_update<false, true>(c, &tabs, xl2, vl, c.len, x2, v2);
       xl = __fadd_rn(xl, step); xl2 = __fadd_rn(xl2, step);
     }
     sink[gid] = x + v + x2 + v2;
     return;
   }
   for (int i = 0; i < iters; i++) {
-    idm_update<false, true>(c, cg, &tabs, xl, vl, c.len, x, v);
+    idm_update<false, true>(c, &tabs, xl, vl, c.len, x, v);
     xl = __fadd_rn(xl, step);
   }
   sink[gid] = x + v;
