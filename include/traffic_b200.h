@@ -257,14 +257,12 @@ int te_last_kernel_ms(te_handle *h, float *ms);
    unchanged.  Used by bench.py to report what the flush achieves against the HBM peak. */
 int te_stage_bandwidth(te_handle *h, int32_t repeats, double *gbytes_per_sec);
 
-/* Arithmetic-only ceiling of the path: vehicle-updates/s of a micro-kernel in which every lane of a fully
-   occupied GPU does nothing but dependent IDM updates (traffic_env.py:50-62) in registers.  Used by bench.py
-   as the compute roofline of the step kernel. */
-int te_idm_peak(int device, const float *archetype, float rate, int32_t iters, double *updates_per_sec);
-/* The same for one form of the update and one occupancy.  form: -1 = the form the step kernels run for this archetype on
-   a tame handle, 0 = general checked form (te_idm_peak), 4 = compile-time archetype flags + validity predicate, 5 = the
-   same without the predicate (tame handles), 1..3 = latency studies (two calls per lane; split fast path with one / two
-   cars per lane).  warps_per_sm: 0 = 2048 resident threads per SM, else one CTA of that many warps per SM (1..32). */
+/* Arithmetic-only ceiling of the path: vehicle-updates/s of a micro-kernel in which every lane does nothing but
+   dependent IDM updates (traffic_env.py:50-62) in registers.  Used by bench.py as the compute roofline of the step
+   kernel.  form: -1 = the form the step kernels run for this archetype on a tame handle (5 or 0), 0 = the general form
+   (checked: archetype flags tested, validity predicate and generic fallback), 5 = the tame form (the reference's
+   archetype flags known at compile time, no predicate; needs T and rate powers of two and delta = 4); any other form is
+   an error.  warps_per_sm: 0 = 2048 resident threads per SM, else one CTA of that many warps per SM (1..32). */
 int te_idm_peak_form(int device, const float *archetype, float rate, int32_t iters, int32_t form, int32_t warps_per_sm,
                      double *updates_per_sec);
 
@@ -274,7 +272,8 @@ int te_test_powf(int device, const float *x, float y, float *out, int64_t n);
 /* One IDM update per element (traffic_env.py:50-62): follower (x,v) behind leader (xl,vl,ll). */
 int te_test_idm(int device, float rate, const float *archetype, const float *xl, const float *vl, const float *ll,
                 const float *x, const float *v, float *x_out, float *v_out, int64_t n);
-/* The same through the unchecked form (valid for tame operands and the reference's archetype flags only). */
+/* The same through the tame form (valid for tame operands only).  An error when the archetype and tick length would not
+   run it (T and rate powers of two, delta = 4, archetype inside the tame ranges). */
 int te_test_idm_tame(int device, float rate, const float *archetype, const float *xl, const float *vl, const float *ll,
                      const float *x, const float *v, float *x_out, float *v_out, int64_t n);
 /* powf(r, 4) over every non-negative finite float r: out[0] = #r where RN_f32((r*r)*(r*r)) differs from the
@@ -282,9 +281,6 @@ int te_test_idm_tame(int device, float rate, const float *archetype, const float
    rounding boundary, out[2] = #r the shortcut filter with threshold tau declines, out[3] = #r it accepts although
    the results differ (the proof obligation: must be 0). */
 int te_test_powf4_exhaustive(int device, uint64_t tau, uint64_t out[4]);
-/* v / cst for every non-negative finite float v: out[0] = #v where the multiply + 2 FMA sequence differs from
-   the IEEE quotient, out[1] = those with a normal quotient, out[2] = bits of the largest such v. */
-int te_test_fdiv_const_exhaustive(int device, float cst, uint64_t out[3]);
 /* Philox4x32-10 block: out[4] for counter ctr[4], key[2]. */
 int te_test_philox(int device, const uint32_t *ctr, const uint32_t *key, uint32_t *out);
 

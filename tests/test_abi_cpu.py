@@ -64,3 +64,18 @@ def test_gap_cdf_table_properties():
         assert abs(t[0] / 2 ** 32 - (1 - np.exp(-0.5 * rate))) < 1e-9
         mean_gap = float(((2 ** 32 - t.astype(np.float64)) / 2 ** 32).sum())  # sum_k P(gap > k)
         assert abs(mean_gap - (1 / rate)) < 0.15 + 0.02 / rate
+
+
+def test_idm_peak_form_rejects_unknown_forms():
+    """The micro-kernel times form 5 (tame), form 0 (general) or, for -1, the one the step kernels run; any other form
+    is refused with a message naming the accepted ones, before a device is touched."""
+    import numpy as np
+    from traffic_env_b200 import _lib
+    L = _lib.load()
+    arch = np.array(_lib.default_config().archetype, np.float32)
+    for form in (1, 2, 3, 4, 6):
+        out = C.c_double(-1.0)
+        assert L.te_idm_peak_form(0, arch.ctypes.data, 0.5, 100, form, 0, C.byref(out)) < 0
+        msg = L.te_last_error().decode()
+        assert "form %d" % form in msg and "-1 = " in msg and "0 = general" in msg and "5 = tame" in msg, msg
+        assert out.value == -1.0

@@ -221,7 +221,7 @@ def gpu_idm_tame(rate, arch, xl, vl, ll, x, v):
 
 
 def test_idm_unchecked_form_on_tame_operands():
-    """The form the step kernels run while the handle is tame (idm_update<true, false>: no validity predicate, no generic
+    """The form the step kernels run while the handle is tame (idm_update<true>: no validity predicate, no generic
     fallback) against the checked form and the oracle, over the whole tame domain and its edges: speeds of 0, 2^-100,
     the handle's speed cap (twice the fastest speed of the dynamics) and log-uniform in between, positions up to 2^40 in magnitude, gaps from overlapping (negative) through
     zero and the -1e-8 neighbourhood to 2^40 and the free road (+inf leader), leader lengths 0 and up to 2^19; and that
@@ -270,3 +270,13 @@ def test_idm_unchecked_form_on_tame_operands():
     assert np.isfinite(ux).all() and (np.abs(ux) < 2.0 ** 40 + 2.0 ** 21).all()
     assert ((uv == 0) | ((uv >= lo) & (uv <= hi))).all() and not np.signbit(uv).any()
     assert (uv <= np.maximum(v, np.float32(13.89 + 3.0 * 0.5)) * np.float32(1 + 1e-6)).all()
+
+
+def test_idm_tame_hook_refuses_an_archetype_without_the_tame_form():
+    """te_test_idm_tame runs the compile-time-archetype form, which is only right where the step kernels would run it:
+    T = 3 is not a power of two, so the hook refuses instead of returning wrong numbers."""
+    from traffic_env_b200._lib import TrafficB200Error
+    arch = np.array([0.0, 11.11, 4.0, 3.0, 4.0, 13.89, 6.0, 3.0, 1.0, 0.0], np.float32)
+    z = np.zeros(16, np.float32)
+    with pytest.raises(TrafficB200Error, match="te_test_idm_tame"):
+        gpu_idm_tame(0.5, arch, z + 40.0, z, z + 4.0, z, z + 5.0)

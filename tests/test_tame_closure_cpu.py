@@ -1,4 +1,4 @@
-"""CPU: the closure argument behind the kernels' tame mode (te_math.cuh, idm_update<FA, CHECKED = false>), checked on the
+"""CPU: the closure argument behind the kernels' tame mode (te_math.cuh, idm_update<TAME = true>), checked on the
 oracle alone - the oracle is the reference's arithmetic, so this needs no GPU.  For operands inside the tame domain
 (finite |x| < 2^40, speeds zero or in [2^-100, cap], leader finite or +inf) one IDM update must give a tame car again:
 finite position, speed zero or in [2^-100, cap] and never above max(v, v0 + a rate).  The cap comes from the library's

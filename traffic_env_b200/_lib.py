@@ -23,7 +23,7 @@ EXPORTS = [
     "te_reset", "te_set_arrivals", "te_step", "te_step_masked", "te_step_multi", "te_step_multi_wire", "te_step_wire",
     "te_pool_create", "te_pool_destroy", "te_pool_step", "te_pool_reset", "te_pool_cars", "te_pool_counters", "te_pool_last_error", "te_wire_layout", "te_expand_wire", "te_step_raw", "te_remi_reward", "te_cars_on_roads",
     "te_greedy_actions", "te_get_state", "te_set_state", "te_get_stats", "te_get_trip_times",
-    "te_synchronize", "te_host_alloc", "te_host_free", "te_last_kernel_ms", "te_stage_bandwidth", "te_idm_peak", "te_idm_peak_form", "te_test_powf", "te_test_idm", "te_test_idm_tame", "te_is_tame", "te_tame_speed_cap", "te_set_controller_spacing", "te_test_powf4_exhaustive", "te_test_fdiv_const_exhaustive", "te_test_philox",
+    "te_synchronize", "te_host_alloc", "te_host_free", "te_last_kernel_ms", "te_stage_bandwidth", "te_idm_peak_form", "te_test_powf", "te_test_idm", "te_test_idm_tame", "te_is_tame", "te_tame_speed_cap", "te_set_controller_spacing", "te_test_powf4_exhaustive", "te_test_philox",
 ]
 
 
@@ -112,7 +112,6 @@ def load():
     L.te_host_alloc.argtypes = [C.c_uint64, C.POINTER(vp)]
     L.te_host_free.argtypes = [vp]
     L.te_stage_bandwidth.argtypes = [vp, i32, C.POINTER(C.c_double)]
-    L.te_idm_peak.argtypes = [C.c_int, vp, C.c_float, i32, C.POINTER(C.c_double)]
     L.te_idm_peak_form.argtypes = [C.c_int, vp, C.c_float, i32, i32, i32, C.POINTER(C.c_double)]
     L.te_test_powf.argtypes = [C.c_int, vp, C.c_float, vp, i64]
     L.te_test_idm.argtypes = [C.c_int, C.c_float, vp, vp, vp, vp, vp, vp, vp, vp, i64]
@@ -121,7 +120,6 @@ def load():
     L.te_tame_speed_cap.argtypes = [vp, C.c_float, C.c_float, C.POINTER(C.c_float)]
     L.te_is_tame.argtypes = [vp, C.POINTER(i32), C.POINTER(C.c_float)]
     L.te_test_powf4_exhaustive.argtypes = [C.c_int, C.c_uint64, vp]
-    L.te_test_fdiv_const_exhaustive.argtypes = [C.c_int, C.c_float, vp]
     L.te_test_philox.argtypes = [C.c_int, vp, vp, vp]
     for name in EXPORTS:
         if name not in ("te_default_config", "te_last_error", "te_pool_last_error"):

@@ -200,7 +200,7 @@ struct te_handle {
   dev_buf<unsigned char> d_wire; pinned_buf<unsigned char> h_wire;   // [steps][E][wire_stride] device / page-locked host
   int wire_stride = 0, host_slices = 1;
   int wire_steps = 1, float_steps = 1;   // actor steps the wire records / float staging have room for
-  bool tame = false;     // every car the device has seen is tame (te_math.cuh: CHECKED = false may run)
+  bool tame = false;     // every car the device has seen is tame (te_math.cuh: idm_update<TAME = true> may run)
   float v_cap = 0.f;     // speed bound of the tame domain for this archetype (tame_archetype)
   int ctrl_spacing = 0;  // TE_CTRL_GREEDY: a new decision every so many actor steps inside a te_step_multi launch (0: one per launch)
   int actions_cap = 1;   // decisions d_actions has room for
@@ -215,16 +215,16 @@ struct te_handle {
 // x 2 CTAs, 101.7 KB each; 3x3 grid: 64 threads x 16 CTAs).
 typedef void (*step_kernel_t)(const StepParams);
 struct StepVariant { step_kernel_t fn; int maxt; };
-// threads = rows of the CTA; fa = the car loop compiled for the reference's archetype (IdmConst.pow2 && delta_is_four,
-// tame handles); grouped = several env instances per CTA (small grids with the reference's archetype, te_create).
+// threads = rows of the CTA; tame = the car loop compiled in the tame form (runs_tame_form); grouped = several env
+// instances per CTA (small grids with the reference's archetype, te_create).
 // 20 instantiations of the step kernel: the set is kept small for the sake of build time.
-static StepVariant step_variant_for(int threads, bool validate, bool fa, bool grouped) {
+static StepVariant step_variant_for(int threads, bool validate, bool tame, bool grouped) {
   if (validate) {  // + the birth-tick plane in shared memory: one CTA fewer per SM
     if (threads <= 256) return {te_step_kernel<256, 2, true, false, false>, 256};
     if (threads <= 512) return {te_step_kernel<512, 1, true, false, false>, 512};
     return {te_step_kernel<768, 1, true, false, false>, 768};
   }
-  if (grouped) {   // (only built for the fast archetype: te_create keeps G = 1 otherwise)
+  if (grouped) {   // (only built in the tame form: te_create keeps G = 1 otherwise)
     if (threads <= 64) return {te_step_kernel<64, 16, false, true, true>, 64};
     // default 3x3 grid: two envs (2 x 48 roads) on three warps, 20 envs per SM at 64 registers (72 registers and 9 CTAs
     // per SM measured 2.4 % slower)
@@ -233,7 +233,7 @@ static StepVariant step_variant_for(int threads, bool validate, bool fa, bool gr
     if (threads <= 160) return {te_step_kernel<160, 6, false, true, true>, 160};
     return {te_step_kernel<256, 4, false, true, true>, 256};
   }
-  if (fa) {
+  if (tame) {
     if (threads <= 64) return {te_step_kernel<64, 16, false, true, false>, 64};
     if (threads <= 128) return {te_step_kernel<128, 8, false, true, false>, 128};
     if (threads <= 256) return {te_step_kernel<256, 4, false, true, false>, 256};
@@ -248,8 +248,6 @@ static StepVariant step_variant_for(int threads, bool validate, bool fa, bool gr
   if (threads <= 768) return {te_step_kernel<768, 1, false, false, false>, 768};
   return {te_step_kernel<1024, 1, false, false, false>, 1024};
 }
-static bool fast_arch(const te_handle *h);
-
 // The double literals of the IDM update live in constant memory (te_math.cuh: g_mc); one upload per device.
 static cudaError_t upload_math_consts() {
   const MathConsts m = math_consts_host();
@@ -273,9 +271,10 @@ static void fill_idm(IdmConst &c, const float *a, float rate) {
   c.pow2 = is_pow2_f(a[7]) && is_pow2_f(rate) && !getenv("TE_NO_POW2_SHORTCUT");
 }
 
-// The FA kernels are compiled for the reference's archetype AND without the per-car validity predicate:
-// they may only run while the handle is tame.
-static bool fast_arch(const te_handle *h) { return h->base.idm.pow2 && h->base.idm.delta_is_four && h->tame; }
+// The one rule for which form of the IDM update runs (te_math.cuh: idm_update<TAME>).  The tame kernels are compiled for
+// the reference's archetype AND without the per-car validity predicate: they may only run while the handle (or, for the
+// test hooks, the archetype) is tame.
+static bool runs_tame_form(const IdmConst &c, bool tame) { return c.pow2 && c.delta_is_four && tame; }
 
 // Archetype ranges under which tame car state stays tame and every fast sequence of idm_update is exact (te_math.cuh).
 // *v_cap = the speed bound of the tame domain for this archetype: twice the fastest speed the dynamics can produce
@@ -372,7 +371,7 @@ static int select_layout(te_handle *h) {
   if (h->Rp > 1024) { return fail("te_create: %d roads exceed one CTA (max 1024)", h->Rp); }
   const bool validate = (cfg->flags & TE_VALIDATE) != 0;
   h->G = 1; h->threads = h->Rp;
-  if (!validate && h->R < 128 && fast_arch(h)) {
+  if (!validate && h->R < 128 && runs_tame_form(h->base.idm, h->tame)) {
     double best = (double)(h->Rp - h->R) / h->Rp;
     for (int g = 2; g <= 4 && g * h->R <= 256; g++) {
       const int th = (g * h->R + 31) / 32 * 32;
@@ -383,7 +382,7 @@ static int select_layout(te_handle *h) {
   h->warps = h->threads / GROUP_ROADS;
   p.G = h->G;
   CU(cudaDeviceGetAttribute(&h->smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
-  const StepVariant sv = step_variant_for(h->threads, validate, fast_arch(h), h->G > 1);
+  const StepVariant sv = step_variant_for(h->threads, validate, runs_tame_form(h->base.idm, h->tame), h->G > 1);
   if (h->threads > sv.maxt) { return fail("te_create: %d roads exceed the largest%s kernel variant (%d)", h->threads, validate ? " validate-mode" : "", sv.maxt); }
   const int smem_max = smem_bytes(sv.maxt, validate, MAX_K, h->n_entry, h->G);
   if (smem_max > h->smem_optin) { return fail("te_create: env needs %d B of shared memory, device allows %d", smem_max, h->smem_optin); }
@@ -824,7 +823,7 @@ static int launch_step(te_handle *h, const StepReq &q) {
     CU(cudaGetLastError());
   }
   const bool validate = (h->cfg.flags & TE_VALIDATE) != 0;
-  const StepVariant sv = step_variant_for(h->threads, validate, fast_arch(h), h->G > 1);
+  const StepVariant sv = step_variant_for(h->threads, validate, runs_tame_form(h->base.idm, h->tame), h->G > 1);
   const int smem = smem_bytes(sv.maxt, validate, K * nsteps, h->n_entry, h->G);
   CU(cudaEventRecord(h->ev0.get(), st));
   if (route != Route::DEVICE) return launch_sliced(h, q, route, p, sv, smem, st);
@@ -1129,9 +1128,9 @@ extern "C" int te_stage_bandwidth(te_handle *h, int32_t repeats, double *gbytes_
   StepParams p = h->base;
   p.K = 10;
   cudaStream_t st = h->stream.get();
-  te_stage_kernel<<<h->cfg.num_envs, h->Rp, stage_smem, st>>>(p, validate);  // warm-up (state is rewritten unchanged)
+  te_stage_kernel<<<h->cfg.num_envs, h->Rp, stage_smem, st>>>(p);  // warm-up (state is rewritten unchanged)
   CU(cudaEventRecord(h->ev0.get(), st));
-  for (int i = 0; i < repeats; i++) te_stage_kernel<<<h->cfg.num_envs, h->Rp, stage_smem, st>>>(p, validate);
+  for (int i = 0; i < repeats; i++) te_stage_kernel<<<h->cfg.num_envs, h->Rp, stage_smem, st>>>(p);
   CU(cudaEventRecord(h->ev1.get(), st));
   CU(cudaEventSynchronize(h->ev1.get()));
   CU(cudaGetLastError());
@@ -1173,28 +1172,39 @@ extern "C" int te_test_powf(int device, const float *x, float y, float *out, int
   return 0;
 }
 
+// tame_archetype for the hooks below, which have no handle: the default config's road length.
+static bool archetype_is_tame(const float *a, float rate) {
+  te_config cfg; te_default_config(&cfg);
+  memcpy(cfg.archetype, a, sizeof(cfg.archetype)); cfg.rate = rate;
+  float cap;
+  return tame_archetype(&cfg, &cap);
+}
+
 static int test_idm(int device, float rate, const float *a, const float *xl, const float *vl, const float *ll,
-                    const float *x, const float *v, float *x_out, float *v_out, int64_t n, int unchecked);
+                    const float *x, const float *v, float *x_out, float *v_out, int64_t n, bool tame);
 extern "C" int te_test_idm(int device, float rate, const float *a, const float *xl, const float *vl, const float *ll,
                            const float *x, const float *v, float *x_out, float *v_out, int64_t n) {
-  return test_idm(device, rate, a, xl, vl, ll, x, v, x_out, v_out, n, 0);
+  return test_idm(device, rate, a, xl, vl, ll, x, v, x_out, v_out, n, false);
 }
 extern "C" int te_test_idm_tame(int device, float rate, const float *a, const float *xl, const float *vl, const float *ll,
                                 const float *x, const float *v, float *x_out, float *v_out, int64_t n) {
-  return test_idm(device, rate, a, xl, vl, ll, x, v, x_out, v_out, n, 1);
+  return test_idm(device, rate, a, xl, vl, ll, x, v, x_out, v_out, n, true);
 }
 static int test_idm(int device, float rate, const float *a, const float *xl, const float *vl, const float *ll,
-                    const float *x, const float *v, float *x_out, float *v_out, int64_t n, int unchecked) {
-  CU(cudaSetDevice(device));
-  CU(upload_math_consts());
+                    const float *x, const float *v, float *x_out, float *v_out, int64_t n, bool tame) {
   IdmConst c;
   fill_idm(c, a, rate);
+  if (tame && !runs_tame_form(c, archetype_is_tame(a, rate)))
+    return fail("te_test_idm_tame: the tame form needs T and rate powers of two, delta = 4 and an archetype inside the "
+                "tame ranges");
+  CU(cudaSetDevice(device));
+  CU(upload_math_consts());
   dev_buf<float> d[7];
   const float *src[5] = {xl, vl, ll, x, v};
   for (int i = 0; i < 7; i++) CU(alloc(d[i], n));
   for (int i = 0; i < 5; i++) CU(cudaMemcpy(d[i].get(), src[i], n * 4, cudaMemcpyHostToDevice));
   te_test_idm_kernel<<<(unsigned)((n + 255) / 256), 256>>>(c, d[0].get(), d[1].get(), d[2].get(), d[3].get(),
-                                                           d[4].get(), d[5].get(), d[6].get(), n, unchecked);
+                                                           d[4].get(), d[5].get(), d[6].get(), n, tame);
   CU(cudaGetLastError());
   CU(cudaMemcpy(x_out, d[5].get(), n * 4, cudaMemcpyDeviceToHost));
   CU(cudaMemcpy(v_out, d[6].get(), n * 4, cudaMemcpyDeviceToHost));
@@ -1203,20 +1213,17 @@ static int test_idm(int device, float rate, const float *a, const float *xl, con
 
 extern "C" int te_idm_peak_form(int device, const float *a, float rate, int32_t iters, int32_t form, int32_t warps_per_sm,
                                 double *updates_per_sec) {
-  if (!a || !updates_per_sec || iters < 1 || form < -1 || form > 5 || warps_per_sm < 0 || warps_per_sm > 32)
+  if (!a || !updates_per_sec || iters < 1 || warps_per_sm < 0 || warps_per_sm > 32)
     return fail("te_idm_peak_form: bad argument");
-  CU(cudaSetDevice(device));
-  CU(upload_math_consts());
+  if (form != -1 && form != 0 && form != 5)
+    return fail("te_idm_peak_form: unknown form %d (accepted: -1 = the form the step kernels run for this archetype, "
+                "0 = general, 5 = tame)", form);
   IdmConst c;
   fill_idm(c, a, rate);
-  if (form < 0) {   // the form the step kernels run for this archetype
-    te_config cfg; te_default_config(&cfg);
-    memcpy(cfg.archetype, a, sizeof(cfg.archetype)); cfg.rate = rate;
-    float cap;
-    const bool fa = c.pow2 && c.delta_is_four;
-    form = fa ? (tame_archetype(&cfg, &cap) ? 5 : 4) : 0;
-  }
-  if (form >= 1 && !(c.pow2 && c.delta_is_four)) return fail("te_idm_peak_form: forms 1..5 need the power-of-two archetype");
+  if (form == 5 && !runs_tame_form(c, true)) return fail("te_idm_peak_form: form 5 needs the power-of-two, delta = 4 archetype");
+  const bool tame = form == 5 || (form == -1 && runs_tame_form(c, archetype_is_tame(a, rate)));
+  CU(cudaSetDevice(device));
+  CU(upload_math_consts());
   int sms = 0;
   CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
   int threads = 256, blocks = sms * 8;  // warps_per_sm == 0: 2048 resident threads per SM
@@ -1225,20 +1232,17 @@ extern "C" int te_idm_peak_form(int device, const float *a, float rate, int32_t 
   CU(alloc(sink, (size_t)threads * blocks));
   event_ptr e0, e1;
   CU(create(e0, cudaEventDefault)); CU(create(e1, cudaEventDefault));
-  te_idm_peak_kernel<<<blocks, threads>>>(c, iters / 4 + 1, sink.get(), form);  // warm-up
+  void (*kernel)(IdmConst, int, float *) = tame ? te_idm_peak_kernel<true> : te_idm_peak_kernel<false>;
+  kernel<<<blocks, threads>>>(c, iters / 4 + 1, sink.get());  // warm-up
   CU(cudaEventRecord(e0.get()));
-  te_idm_peak_kernel<<<blocks, threads>>>(c, iters, sink.get(), form);
+  kernel<<<blocks, threads>>>(c, iters, sink.get());
   CU(cudaEventRecord(e1.get()));
   CU(cudaEventSynchronize(e1.get()));
   CU(cudaGetLastError());
   float ms = 0.f;
   CU(cudaEventElapsedTime(&ms, e0.get(), e1.get()));
-  *updates_per_sec = (double)threads * blocks * iters * ((form == 1 || form == 3) ? 2 : 1) / (ms * 1e-3);
+  *updates_per_sec = (double)threads * blocks * iters / (ms * 1e-3);
   return 0;
-}
-
-extern "C" int te_idm_peak(int device, const float *a, float rate, int32_t iters, double *updates_per_sec) {
-  return te_idm_peak_form(device, a, rate, iters, 0, 0, updates_per_sec);
 }
 
 extern "C" int te_test_powf4_exhaustive(int device, uint64_t tau, uint64_t out[4]) {
@@ -1250,19 +1254,6 @@ extern "C" int te_test_powf4_exhaustive(int device, uint64_t tau, uint64_t out[4
   te_powf4_exhaustive_kernel<<<148 * 16, 256>>>((unsigned long long)tau, d.get());
   CU(cudaGetLastError());
   CU(cudaMemcpy(out, d.get(), 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-  return 0;
-}
-
-extern "C" int te_test_fdiv_const_exhaustive(int device, float cst, uint64_t out[3]) {
-  if (!out) return fail("te_test_fdiv_const_exhaustive: null argument");
-  CU(cudaSetDevice(device));
-  dev_buf<unsigned long long> d;
-  CU(alloc(d, 3));
-  CU(cudaMemset(d.get(), 0, 3 * sizeof(unsigned long long)));
-  volatile float y = 1.0f / cst;
-  te_fdiv_const_exhaustive_kernel<<<148 * 16, 256>>>(cst, y, d.get());
-  CU(cudaGetLastError());
-  CU(cudaMemcpy(out, d.get(), 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
   return 0;
 }
 

@@ -421,7 +421,7 @@ __device__ __forceinline__ int light_ylim(const Smem &s, int i, int road, int V,
 }
 
 // GROUPED = false: one env per CTA (p.G == 1), everything about env groups folds away at compile time.
-template <int MAXT, int MINB, bool VALIDATE, bool FA, bool GROUPED>
+template <int MAXT, int MINB, bool VALIDATE, bool TAME, bool GROUPED>
 __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   constexpr SmemLayout L = make_layout(MAXT, VALIDATE);
@@ -737,8 +737,8 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
           float xn = lds_f32(addr), vn = lds_f32_off<VOFF>(addr);
           const float xl = px, vl = pv, ll = pl;
           px = xn; pv = vn; pl = c.len;
-          // the FA kernels run the unchecked arithmetic; te_api.cu only launches them on tame handles
-          idm_update<FA, !FA>(c, s.tabs, xl, vl, ll, xn, vn);
+          // the tame kernels run the unchecked arithmetic; te_api.cu only launches them on tame handles
+          idm_update<TAME>(c, s.tabs, xl, vl, ll, xn, vn);
           sts_f32(addr, xn); sts_f32_off<VOFF>(addr, vn);
           // wrapped ring, low segment (slot < leading): the reference tests x, not v (traffic_env.py:210).
           // THRESH = 0.2 is compared in double by the reference; 0.2f is the smallest float above 0.2, so for every
@@ -990,9 +990,8 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
 // Staging only: the step kernel's bulk-TMA stage-in and flush of one env's ring planes with no ticks in
 // between (same CTA shape and shared-memory footprint, so the same number of copies is in flight per SM).
 // Measures the HBM bandwidth the load/flush phases of te_step_kernel run at.
-__global__ void te_stage_kernel(const StepParams p, int validate) {
+__global__ void te_stage_kernel(const StepParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  (void)validate;
   const int env = blockIdx.x;
   const uint32_t plane_bytes = (uint32_t)p.R * CAP * 4;   // the real roads, like the step kernel
   float *xs = reinterpret_cast<float *>(smem_raw), *vs = reinterpret_cast<float *>(smem_raw + plane_bytes);
@@ -1097,19 +1096,22 @@ __global__ void te_test_powf_kernel(const float *x, float y, float *out, long lo
   if (i < n) out[i] = powf_glibc(x[i], y, &g_powf_tables);
 }
 __global__ void te_test_idm_kernel(IdmConst c, const float *xl, const float *vl, const float *ll, const float *x,
-                                   const float *v, float *xo, float *vo, long long n, int unchecked) {
+                                   const float *v, float *xo, float *vo, long long n, int tame) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) {
     float xx = x[i], vv = v[i];
-    if (unchecked) idm_update<true, false>(c, &g_powf_tables, xl[i], vl[i], ll[i], xx, vv);   // tame operands only
-    else if (c.pow2 && c.delta_is_four) idm_update<true, true>(c, &g_powf_tables, xl[i], vl[i], ll[i], xx, vv);
-    else idm_update<false, true>(c, &g_powf_tables, xl[i], vl[i], ll[i], xx, vv);
+    if (tame) idm_update<true>(c, &g_powf_tables, xl[i], vl[i], ll[i], xx, vv);   // tame operands only
+    else idm_update<false>(c, &g_powf_tables, xl[i], vl[i], ll[i], xx, vv);
     xo[i] = xx; vo[i] = vv;
   }
 }
-// Arithmetic-only ceiling: every lane runs `iters` dependent IDM updates of one car behind a leader that
-// drives at constant speed (registers only, full-precision path: both divisions and powf every time).
-__global__ void te_idm_peak_kernel(IdmConst c, int iters, float *sink, int ilp2) {
+// Arithmetic-only ceiling: every lane runs `iters` dependent IDM updates of one car behind a leader that drives at
+// constant speed (registers only), in the form a step kernel with the same TAME runs.  One instantiation per form, so
+// that each timed loop is compiled on its own.  __maxnreg__(40) keeps the register budget the rates in DESIGN.md
+// section 4 were measured with: 48 warps per SM at warps_per_sm = 0 (six 256-thread CTAs) and the same loop schedule.
+// Left to itself ptxas gives the tame form 30 registers and a schedule that runs 5 % slower at 32 warps per SM.
+template <bool TAME>
+__global__ void __maxnreg__(40) te_idm_peak_kernel(IdmConst c, int iters, float *sink) {
   __shared__ PowfTables tabs;
   for (int i = threadIdx.x; i < (int)(sizeof(PowfTables) / 8); i += blockDim.x)
     reinterpret_cast<unsigned long long *>(&tabs)[i] = reinterpret_cast<const unsigned long long *>(&g_powf_tables)[i];
@@ -1118,54 +1120,8 @@ __global__ void te_idm_peak_kernel(IdmConst c, int iters, float *sink, int ilp2)
   float x = 0.f, v = 5.f + 0.001f * (float)(gid & 1023);
   float xl = 30.f + 0.01f * (float)(gid & 255);
   const float vl = 9.f, step = __fmul_rn(vl, c.rate);
-  if (ilp2 == 5) {   // what the step kernels run on a tame handle: archetype flags known at compile time, no validity predicate
-    for (int i = 0; i < iters; i++) {
-      idm_update<true, false>(c, &tabs, xl, vl, c.len, x, v);
-      xl = __fadd_rn(xl, step);
-    }
-    sink[gid] = x + v;
-    return;
-  }
-  if (ilp2 == 4) {   // the same with the validity predicate and the generic fallback (a handle that saw a wild car)
-    for (int i = 0; i < iters; i++) {
-      idm_update<true, true>(c, &tabs, xl, vl, c.len, x, v);
-      xl = __fadd_rn(xl, step);
-    }
-    sink[gid] = x + v;
-    return;
-  }
-  if (ilp2 >= 2) {
-    // latency study: the split fast path (idm_study_part1 / part2), one car per lane (ilp2 == 2) or two cars whose first
-    // parts share a basic block (ilp2 == 3)
-    float x2 = 1.f, v2 = 6.f + 0.001f * (float)(gid & 511), xl2 = 40.f + 0.01f * (float)(gid & 127);
-    for (int i = 0; i < iters; i++) {
-      const IdmMid ma = idm_study_part1(c, xl, vl, c.len, x, v);
-      if (ilp2 == 3) {
-        const IdmMid mb = idm_study_part1(c, xl2, vl, c.len, x2, v2);
-        idm_study_part2(c, &tabs, ma, x, v);
-        idm_study_part2(c, &tabs, mb, x2, v2);
-        xl2 = __fadd_rn(xl2, step);
-      } else {
-        idm_study_part2(c, &tabs, ma, x, v);
-      }
-      xl = __fadd_rn(xl, step);
-    }
-    sink[gid] = x + v + x2 + v2;
-    return;
-  }
-  if (ilp2) {
-    // latency study: TWO independent cars per lane (one straight-line block: the compiler interleaves the chains)
-    float x2 = 1.f, v2 = 6.f + 0.001f * (float)(gid & 511), xl2 = 40.f + 0.01f * (float)(gid & 127);
-    for (int i = 0; i < iters; i++) {
-      idm_update<false, true>(c, &tabs, xl, vl, c.len, x, v);
-      idm_update<false, true>(c, &tabs, xl2, vl, c.len, x2, v2);
-      xl = __fadd_rn(xl, step); xl2 = __fadd_rn(xl2, step);
-    }
-    sink[gid] = x + v + x2 + v2;
-    return;
-  }
   for (int i = 0; i < iters; i++) {
-    idm_update<false, true>(c, &tabs, xl, vl, c.len, x, v);
+    idm_update<TAME>(c, &tabs, xl, vl, c.len, x, v);
     xl = __fadd_rn(xl, step);
   }
   sink[gid] = x + v;
@@ -1194,27 +1150,6 @@ __global__ void te_powf4_exhaustive_kernel(unsigned long long tau, unsigned long
     if (powf4_fast_d((double)r, pd2) && !(pd2 == (double)ref && __float_as_uint(__double2float_rn(pd2)) == __float_as_uint(ref))) bad++;
   }
   atomicAdd(&out[0], diff); atomicMax(&out[1], maxd); atomicAdd(&out[2], slow); atomicAdd(&out[3], bad);
-}
-
-// Exhaustive check of the float division by a constant: for EVERY non-negative finite float v, is
-// fma(fma(-c, v*y, v), y, v*y) with y = RN_f32(1/c) equal to RN_f32(v / c)?  out[0] = #mismatches,
-// out[1] = #mismatches whose quotient is a normal float, out[2] = largest v (bits) that mismatches.
-__global__ void te_fdiv_const_exhaustive_kernel(float cst, float y, unsigned long long *out) {
-  const unsigned long long stride = (unsigned long long)gridDim.x * blockDim.x;
-  unsigned long long bad = 0, bad_normal = 0, maxv = 0;
-  for (unsigned long long ix = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; ix < 0x7f800000ull; ix += stride) {
-    const float v = __uint_as_float((uint32_t)ix);
-    const float ref = __fdiv_rn(v, cst);
-    const float q = __fmul_rn(v, y);
-    const float r = __fmaf_rn(-cst, q, v);
-    const float got = __fmaf_rn(r, y, q);
-    if (__float_as_uint(ref) != __float_as_uint(got)) {
-      bad++;
-      if (__float_as_uint(ref) >= 0x00800000u) bad_normal++;
-      if (ix > maxv) maxv = ix;
-    }
-  }
-  atomicAdd(&out[0], bad); atomicAdd(&out[1], bad_normal); atomicMax(&out[2], maxv);
 }
 
 __global__ void te_test_philox_kernel(const uint32_t *ctr, const uint32_t *key, uint32_t *out) {

@@ -446,8 +446,9 @@ class VecTrafficEnv(object):
 
 def idm_arithmetic_peak(device=0, rate=0.5, archetype=None, iters=4000, form=-1, warps_per_sm=None):
     """vehicle-updates/s of the IDM arithmetic alone, registers only, every lane busy (te_idm_peak_form).  form -1: the
-    form the step kernels run for this archetype on a tame handle; 0: the general checked form (the denominator of the
-    round-1 figures).  warps_per_sm None: the better of 32 warps per SM (the step kernels' occupancy) and 64."""
+    form the step kernels run for this archetype on a tame handle (5 or 0); 0: the general checked form (the denominator
+    of the round-1 figures); 5: the tame form.  Any other form raises.  warps_per_sm None: the better of 32 warps per SM
+    (the step kernels' occupancy) and 64."""
     L = _lib.load()
     arch = np.ascontiguousarray(ARCHETYPE if archetype is None else archetype, dtype=np.float32)
     best = 0.0
