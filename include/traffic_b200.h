@@ -220,6 +220,38 @@ int te_set_state(te_handle *h, int32_t env_begin, int32_t count, const int32_t *
                  const float *x, const float *v, const int32_t *obs, const int32_t *waiting,
                  const uint8_t *passed_dst, const float *steps);
 
+/* Snapshot records: the complete state of one env in one fixed-size, 16-byte-aligned blob, for bit-exact rewind,
+   checkpoint / resume and cloning of envs.  A record holds a header (magic, format version, m, n, validate bit), the R
+   real rows of the x and v ring planes exactly as the device holds them (slot 0 of a row is the packed header word:
+   leading | lastcar << 8 | detected << 16 in the x plane, waiting in the v plane), the birth-tick plane w (TE_VALIDATE
+   handles only), phase / passed_dst (u8) and elapsed (i32) of the I intersections, and the env's private scalars (episode
+   tick counter, position in the Philox arrival stream, injected-schedule clock, reset counter, episode step / done flag /
+   return statistics).  About 71 KB per 10x10 env, 7.8 KB per 3x3 env.  A record carries no env id.
+   Continuation: arrivals and reset phases are keyed by (seed, env_id_base + slot) and a record restores only the
+   position in that stream, so a loaded env continues exactly as the saved env would have when it sits in the same slot
+   of a handle with the same configuration, seed and env_id_base; loaded into another slot it has the same state and
+   continues that slot's own stream from the saved draw index (independent noise, what branching rollouts want).
+   Not part of a record: the handle's te_stats counters, the trip-time buffer, the injected schedule itself and the
+   controller spacing. */
+typedef struct te_snapshot_layout_t {
+  int32_t stride;                              /* bytes per record */
+  int32_t x, v, w, phase, elapsed, passed_dst; /* byte offsets inside a record; w = -1 without TE_VALIDATE */
+  int32_t scalars;                             /* library-private bytes from here on */
+} te_snapshot_layout_t;
+int te_snapshot_layout(const te_handle *h, te_snapshot_layout_t *out);
+/* env_ids is always a host array; NULL = envs [0, count).  records: count * stride bytes in `memspace` (16-byte aligned
+   in device memory).  te_save_envs gathers the listed envs into records (duplicates allowed).  TE_DEVICE: asynchronous,
+   ordered on `stream` after earlier work on it (explicit env_ids are copied from the caller's pageable array, which may
+   make the call wait for that stream); TE_HOST: synchronous. */
+int te_save_envs(te_handle *h, const int32_t *env_ids, int32_t count, void *records, int memspace, void *stream);
+/* te_load_envs scatters record j into env env_ids[j] (each id at most once); synchronous in both memspaces (`stream` is
+   not used), like te_set_state.  Every record is checked on the device before anything is written - magic, version,
+   m / n, the validate bit, every row's leading and lastcar in [1, 20) with the header word's top byte zero, phase and
+   passed_dst in {0, 1} - and on a failure the call returns an error naming the first bad record and field and leaves
+   every env untouched.  On a tame handle the same pass applies te_set_state's tame predicate to every live car and
+   leading slot: one wild car moves the handle to the checked kernels for good, exactly as te_set_state does. */
+int te_load_envs(te_handle *h, const int32_t *env_ids, int32_t count, const void *records, int memspace, void *stream);
+
 /* *tame = 1 while the handle runs the unchecked arithmetic: its archetype is inside the supported ranges and every car ever
    handed to te_set_state was tame - x finite with |x| < 2^40, v zero or in [2^-100, *v_cap], *v_cap = twice the fastest
    speed the archetype's dynamics can produce.  Tame state stays tame under the step, and no operand of the IDM update can

@@ -24,6 +24,7 @@ EXPORTS = [
     "te_pool_create", "te_pool_destroy", "te_pool_step", "te_pool_reset", "te_pool_cars", "te_pool_counters", "te_pool_last_error", "te_wire_layout", "te_expand_wire", "te_step_raw", "te_remi_reward", "te_cars_on_roads",
     "te_greedy_actions", "te_get_state", "te_set_state", "te_get_stats", "te_get_trip_times",
     "te_synchronize", "te_host_alloc", "te_host_free", "te_last_kernel_ms", "te_stage_bandwidth", "te_idm_peak_form", "te_test_powf", "te_test_idm", "te_test_idm_tame", "te_is_tame", "te_tame_speed_cap", "te_set_controller_spacing", "te_test_powf4_exhaustive", "te_test_philox",
+    "te_snapshot_layout", "te_save_envs", "te_load_envs",
 ]
 
 
@@ -54,6 +55,10 @@ class TeStats(C.Structure):
 class TeWireLayout(C.Structure):
     _fields_ = [(k, C.c_int32) for k in ("stride", "passed", "detected", "light", "reward", "done", "max_k_ticks",
                                             "host_float_dma")]
+
+
+class TeSnapshotLayout(C.Structure):
+    _fields_ = [(k, C.c_int32) for k in ("stride", "x", "v", "w", "phase", "elapsed", "passed_dst", "scalars")]
 
 
 class TrafficB200Error(RuntimeError):
@@ -121,6 +126,9 @@ def load():
     L.te_is_tame.argtypes = [vp, C.POINTER(i32), C.POINTER(C.c_float)]
     L.te_test_powf4_exhaustive.argtypes = [C.c_int, C.c_uint64, vp]
     L.te_test_philox.argtypes = [C.c_int, vp, vp, vp]
+    L.te_snapshot_layout.argtypes = [vp, C.POINTER(TeSnapshotLayout)]
+    L.te_save_envs.argtypes = [vp, vp, i32, vp, C.c_int, vp]
+    L.te_load_envs.argtypes = [vp, vp, i32, vp, C.c_int, vp]
     for name in EXPORTS:
         if name not in ("te_default_config", "te_last_error", "te_pool_last_error"):
             getattr(L, name).restype = C.c_int

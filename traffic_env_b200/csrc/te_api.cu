@@ -205,6 +205,9 @@ struct te_handle {
   int ctrl_spacing = 0;  // TE_CTRL_GREEDY: a new decision every so many actor steps inside a te_step_multi launch (0: one per launch)
   int actions_cap = 1;   // decisions d_actions has room for
   bool float_dma = false;  // te_step(TE_HOST) with float outputs: let the copy engine write the float arrays (no host expansion)
+  // snapshot records (te_save_envs / te_load_envs): device staging of host records, and the check pass's status word
+  dev_buf<unsigned char> d_snap; size_t snap_cap = 0;
+  dev_buf<SnapStatus> d_snap_status;
   std::unique_ptr<ExpandPool> pool;
   ~te_handle() { cudaSetDevice(device); }
 };
@@ -1046,6 +1049,142 @@ extern "C" int te_set_state(te_handle *h, int32_t env_begin, int32_t count, cons
   CU(cudaStreamSynchronize(st));
   CU(cudaDeviceSynchronize());
   if (wild && h->tame) {      // from now on: the kernels with the per-car validity predicate, one env per CTA
+    h->tame = false;
+    if (int rc = select_layout(h)) return rc;
+  }
+  return 0;
+}
+
+// ---- snapshot records (te_kernels.cuh: snap_layout)
+static SnapLayout snap_layout_of(const te_handle *h) { return snap_layout(h->R, h->I, (h->cfg.flags & TE_VALIDATE) != 0); }
+
+extern "C" int te_snapshot_layout(const te_handle *h, te_snapshot_layout_t *out) {
+  if (!h || !out) return fail("te_snapshot_layout: null argument");
+  const SnapLayout L = snap_layout_of(h);
+  *out = {L.stride, L.x, L.v, L.w, L.phase, L.elapsed, L.passed_dst, L.scalars};
+  return 0;
+}
+
+// Shared argument checks of te_save_envs / te_load_envs: ids in range (and, for a load, each at most once).
+static int snap_check_args(const te_handle *h, const char *who, const int32_t *env_ids, int32_t count, const void *records,
+                           int memspace, bool unique) {
+  if (!h) return fail("%s: null handle", who);
+  if (count < 0) return fail("%s: count %d is negative", who, count);
+  if (count > 0 && !records) return fail("%s: null records", who);
+  if (memspace != TE_HOST && memspace != TE_DEVICE) return fail("%s: unknown memspace %d", who, memspace);
+  if (memspace == TE_DEVICE && ((uintptr_t)records & 15)) return fail("%s: device records must be 16-byte aligned", who);
+  const int E = h->cfg.num_envs;
+  if (!env_ids) {
+    if (count > E) return fail("%s: count %d exceeds the %d envs of the handle", who, count, E);
+    return 0;
+  }
+  std::vector<uint8_t> seen(unique ? E : 0, 0);
+  for (int32_t j = 0; j < count; j++) {
+    const int e = env_ids[j];
+    if (e < 0 || e >= E) return fail("%s: env_ids[%d] = %d is outside [0, %d)", who, j, e, E);
+    if (unique && seen[e]++) return fail("%s: env %d is listed twice (env_ids[%d])", who, e, j);
+  }
+  return 0;
+}
+
+// The kernel arguments of `count` records, and the grid that covers them.
+static SnapArgs snap_args(const te_handle *h, int32_t count, unsigned *blocks) {
+  SnapArgs a = {};
+  a.L = snap_layout_of(h);
+  const int units = (a.L.w >= 0 ? 3 : 2) * h->R * CAP / 4;
+  a.per_cta = std::max(1, std::min(16, SNAP_UNITS_PER_CTA / units));
+  a.count = count; a.m = h->cfg.m; a.n = h->cfg.n;
+  a.check_tame = h->tame ? 1 : 0; a.v_cap = h->v_cap;
+  *blocks = (unsigned)((count + a.per_cta - 1) / a.per_cta);
+  return a;
+}
+
+// A device copy of a host id list, allocated (and later freed) in the order of `st`: a save queued on a stream keeps
+// its own ids while the caller goes on.
+static int upload_ids(const int32_t *env_ids, int32_t count, cudaStream_t st, int **out) {
+  *out = nullptr;
+  if (!env_ids) return 0;
+  CU(cudaMallocAsync((void **)out, (size_t)count * sizeof(int), st));
+  CU(cudaMemcpyAsync(*out, env_ids, (size_t)count * sizeof(int), cudaMemcpyHostToDevice, st));
+  return 0;
+}
+
+// Device staging for records in host memory (the device is idle when this is called).
+static int snap_staging(te_handle *h, size_t bytes) {
+  if (bytes > h->snap_cap) {
+    h->snap_cap = 0;
+    if (int rc = grow(h->d_snap, bytes)) return rc;
+    h->snap_cap = bytes;
+  }
+  return 0;
+}
+
+extern "C" int te_save_envs(te_handle *h, const int32_t *env_ids, int32_t count, void *records, int memspace, void *stream) {
+  if (int rc = snap_check_args(h, "te_save_envs", env_ids, count, records, memspace, false)) return rc;
+  if (count == 0) return 0;
+  CU(cudaSetDevice(h->device));
+  unsigned blocks = 0;
+  const SnapArgs a = snap_args(h, count, &blocks);
+  const size_t bytes = (size_t)count * a.L.stride;
+  cudaStream_t st = pick_stream(h, stream);
+  unsigned char *dst = (unsigned char *)records;
+  if (memspace == TE_HOST) {   // like te_get_state: steps may be queued on caller-provided streams
+    CU(cudaDeviceSynchronize());
+    st = h->stream.get();
+    if (int rc = snap_staging(h, bytes)) return rc;
+    dst = h->d_snap.get();
+  }
+  int *d_ids = nullptr;
+  if (int rc = upload_ids(env_ids, count, st, &d_ids)) return rc;
+  te_snap_save_kernel<<<blocks, SNAP_THREADS, 0, st>>>(h->base, a, d_ids, dst);
+  CU(cudaGetLastError());
+  if (d_ids) CU(cudaFreeAsync(d_ids, st));
+  if (memspace == TE_HOST) {
+    CU(cudaMemcpyAsync(records, dst, bytes, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+  }
+  return 0;
+}
+
+extern "C" int te_load_envs(te_handle *h, const int32_t *env_ids, int32_t count, const void *records, int memspace,
+                            void *stream) {
+  (void)stream;   // synchronous: the records are checked before anything is written
+  if (int rc = snap_check_args(h, "te_load_envs", env_ids, count, records, memspace, true)) return rc;
+  if (count == 0) return 0;
+  CU(cudaSetDevice(h->device));
+  CU(cudaDeviceSynchronize());   // steps queued on caller-provided streams have finished with the state
+  unsigned blocks = 0;
+  const SnapArgs a = snap_args(h, count, &blocks);
+  const size_t bytes = (size_t)count * a.L.stride;
+  cudaStream_t st = h->stream.get();
+  const unsigned char *src = (const unsigned char *)records;
+  if (memspace == TE_HOST) {
+    if (int rc = snap_staging(h, bytes)) return rc;
+    CU(cudaMemcpyAsync(h->d_snap.get(), records, bytes, cudaMemcpyHostToDevice, st));
+    src = h->d_snap.get();
+  }
+  if (!h->d_snap_status) CU(alloc(h->d_snap_status, 1));
+  SnapStatus status = {~0ull, 0u, 0u};
+  CU(cudaMemcpyAsync(h->d_snap_status.get(), &status, sizeof(status), cudaMemcpyHostToDevice, st));
+  te_snap_check_kernel<<<blocks, SNAP_THREADS, 0, st>>>(h->base, a, src, h->d_snap_status.get());
+  CU(cudaGetLastError());
+  CU(cudaMemcpyAsync(&status, h->d_snap_status.get(), sizeof(status), cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
+  if (status.first_bad != ~0ull) {
+    static const char *const what[] = {"magic", "format version", "dimensions (m, n)", "validate bit", "leading",
+                                       "lastcar", "row header (top byte)", "phase", "passed_dst"};
+    const long long j = (long long)(status.first_bad >> 4);
+    const unsigned field = (unsigned)(status.first_bad & 15);
+    return fail("te_load_envs: record %lld (for env %d): bad %s; no env was changed", j, env_ids ? env_ids[j] : (int)j,
+                field < sizeof(what) / sizeof(what[0]) ? what[field] : "field");
+  }
+  int *d_ids = nullptr;
+  if (int rc = upload_ids(env_ids, count, st, &d_ids)) return rc;
+  te_snap_load_kernel<<<blocks, SNAP_THREADS, 0, st>>>(h->base, a, d_ids, src);
+  CU(cudaGetLastError());
+  if (d_ids) CU(cudaFreeAsync(d_ids, st));
+  CU(cudaStreamSynchronize(st));
+  if (status.wild && h->tame) {   // as te_set_state: from now on the checked, one-env-per-CTA kernels
     h->tame = false;
     if (int rc = select_layout(h)) return rc;
   }

@@ -1095,6 +1095,186 @@ __global__ void te_greedy_kernel(StepParams p, uint8_t *actions) {
   actions[i] = (uint8_t)greedy_action([&](int dd) { return ring_count(__float_as_uint(p.x[((size_t)env * p.Rp + dd * p.V + it) * CAP])); });
 }
 
+// ---- snapshot records (te_save_envs / te_load_envs): the complete state of one env in one fixed-size blob.
+//   header u32[8]: magic | version | m | n | flags (bit 0: validate) | R | I | 0
+//   x[R][20], v[R][20] (and w[R][20] on validate handles) exactly as HBM holds the real rows, slot-0 header words included
+//   u8 phase[I], u8 passed_dst[I], i32 elapsed[I], EnvScalars - each region padded with zeros to 16 bytes
+// Every offset is a multiple of 16, so the planes move as 16-byte vectors; padding rows (R..Rp) are not carried: the step
+// kernel rebuilds them in shared memory.
+constexpr uint32_t SNAP_MAGIC = 0x4e534554u;   // "TESN"
+constexpr uint32_t SNAP_VERSION = 1;
+constexpr int SNAP_HEADER_BYTES = 32;
+constexpr int SNAP_THREADS = 256;
+constexpr int SNAP_UNITS_PER_CTA = 4096;        // 16-byte plane vectors a CTA moves (several envs per CTA on small grids)
+struct SnapLayout { int stride, x, v, w, phase, elapsed, passed_dst, scalars; };   // bytes; w = -1 without validate
+__host__ __device__ constexpr SnapLayout snap_layout(int R, int I, bool validate) {
+  const int plane = R * CAP * 4;
+  const int x = SNAP_HEADER_BYTES, v = x + plane, w = validate ? v + plane : -1;
+  const int phase = v + plane + (validate ? plane : 0);
+  const int passed_dst = phase + align_up(I, 16);
+  const int elapsed = passed_dst + align_up(I, 16);
+  const int scalars = elapsed + align_up(4 * I, 16);
+  return {scalars + align_up((int)sizeof(EnvScalars), 16), x, v, w, phase, elapsed, passed_dst, scalars};
+}
+static_assert(sizeof(EnvScalars) % 4 == 0 && (CAP * 4) % 16 == 0, "snapshot record alignment");
+
+// First failed check of te_load_envs: (record << 4) | field, the lowest one wins (atomicMin).
+enum : int { SNAP_BAD_MAGIC = 0, SNAP_BAD_VERSION, SNAP_BAD_DIMS, SNAP_BAD_VALIDATE, SNAP_BAD_LEADING, SNAP_BAD_LASTCAR,
+             SNAP_BAD_HEADER, SNAP_BAD_PHASE, SNAP_BAD_PASSED_DST };
+struct SnapStatus {
+  unsigned long long first_bad;   // ~0: every record passed
+  unsigned int wild;              // some live car or leading slot is outside the tame domain (te_set_state's predicate)
+  unsigned int pad;
+};
+struct SnapArgs {
+  SnapLayout L;
+  int count, per_cta, m, n;
+  int check_tame;                 // the handle is tame: look for wild cars
+  float v_cap;
+};
+
+// Record j of a launch: the env it comes from / goes to.
+__device__ __forceinline__ int snap_env(const int *ids, int j) { return ids ? ids[j] : j; }
+
+// The bulk of a record: its 2 (3) planes of R * 20 floats, 16 bytes per unit.  Units of the CTA's records are dealt to
+// the threads round-robin, four in flight per thread.  SAVE: state -> record, else record -> state.
+template <bool SAVE>
+__device__ __forceinline__ void snap_planes(const StepParams &p, const SnapArgs &a, const int *ids, unsigned char *recs,
+                                            int j0, int nj) {
+  const int planes = a.L.w >= 0 ? 3 : 2;
+  const int n16 = p.R * CAP / 4;
+  const int per_rec = planes * n16, total = nj * per_rec;
+  for (int i0 = threadIdx.x; i0 < total; i0 += 4 * SNAP_THREADS) {
+    uint4 val[4];
+    uint4 *dst[4];
+#pragma unroll
+    for (int u = 0; u < 4; u++) {
+      const int i = i0 + u * SNAP_THREADS;
+      dst[u] = nullptr;
+      if (i < total) {
+        const int jj = i / per_rec, rem = i - jj * per_rec, pl = rem / n16, k = rem - pl * n16;
+        const int j = j0 + jj;
+        float *plane = pl == 0 ? p.x : (pl == 1 ? p.v : p.w);
+        uint4 *st = reinterpret_cast<uint4 *>(plane + (size_t)snap_env(ids, j) * p.Rp * CAP) + k;
+        uint4 *rc = reinterpret_cast<uint4 *>(recs + (size_t)j * a.L.stride + (pl == 0 ? a.L.x : (pl == 1 ? a.L.v : a.L.w))) + k;
+        val[u] = SAVE ? *st : *rc;
+        dst[u] = SAVE ? rc : st;
+      }
+    }
+#pragma unroll
+    for (int u = 0; u < 4; u++)
+      if (dst[u]) *dst[u] = val[u];
+  }
+}
+
+// te_save_envs: gather the listed envs into records (records [count][stride], 16-byte aligned).
+__global__ void __launch_bounds__(SNAP_THREADS) te_snap_save_kernel(const StepParams p, const SnapArgs a, const int *ids,
+                                                                    unsigned char *recs) {
+  const int j0 = blockIdx.x * a.per_cta, nj = min(a.per_cta, a.count - j0);
+  snap_planes<true>(p, a, ids, recs, j0, nj);
+  // header and the small per-intersection / per-env regions, one 32-bit word per thread, padding written as zeros
+  const int hw = SNAP_HEADER_BYTES / 4, sw = (a.L.stride - a.L.phase) / 4, per = hw + sw;
+  for (int i = threadIdx.x; i < nj * per; i += SNAP_THREADS) {
+    const int jj = i / per, k = i - jj * per, j = j0 + jj, env = snap_env(ids, j);
+    uint32_t *rec = reinterpret_cast<uint32_t *>(recs + (size_t)j * a.L.stride);
+    if (k < hw) {
+      const uint32_t h[8] = {SNAP_MAGIC, SNAP_VERSION, (uint32_t)a.m, (uint32_t)a.n, p.w ? 1u : 0u, (uint32_t)p.R,
+                             (uint32_t)p.I, 0u};
+      rec[k] = h[k];
+      continue;
+    }
+    const int o = a.L.phase + 4 * (k - hw);   // byte offset inside the record
+    uint32_t word = 0;
+    if (o < a.L.elapsed) {                    // phase / passed_dst bytes
+      const bool ph = o < a.L.passed_dst;
+      const int b = o - (ph ? a.L.phase : a.L.passed_dst);
+      const uint8_t *src = (ph ? p.phase : p.passed_dst) + (size_t)env * p.I;
+      for (int t = 0; t < 4; t++)
+        if (b + t < p.I) word |= (uint32_t)src[b + t] << (8 * t);
+    } else if (o < a.L.scalars) {
+      const int idx = (o - a.L.elapsed) / 4;
+      if (idx < p.I) word = (uint32_t)p.elapsed[(size_t)env * p.I + idx];
+    } else {
+      const int idx = (o - a.L.scalars) / 4;
+      if (idx < (int)(sizeof(EnvScalars) / 4)) word = reinterpret_cast<const uint32_t *>(p.env + env)[idx];
+    }
+    rec[a.L.phase / 4 + (k - hw)] = word;
+  }
+}
+
+// te_set_state's tame predicate (te_api.cu: tame_car and the leading-slot rule), on the device
+__device__ __forceinline__ bool snap_tame_car(float x, float v, float v_cap) {
+  return isfinite(x) && fabsf(x) < 0x1p40f && isfinite(v) && (v == 0.f ? !signbit(v) : (v >= 0x1p-100f && v <= v_cap));
+}
+__device__ __forceinline__ bool snap_tame_leader(float x) {
+  return x == __int_as_float(0x7f800000) || (isfinite(x) && fabsf(x) < 0x1p40f);
+}
+
+// te_load_envs, first pass: check every record (nothing is written to the state).  One item per 16-byte quad of the x
+// plane (ring indices from the row's header word; live cars and the leading slot of that quad against the tame predicate
+// when the handle is tame), per intersection (phase, passed_dst) and per record (header).
+__global__ void __launch_bounds__(SNAP_THREADS) te_snap_check_kernel(const StepParams p, const SnapArgs a,
+                                                                     const unsigned char *recs, SnapStatus *status) {
+  const int j0 = blockIdx.x * a.per_cta, nj = min(a.per_cta, a.count - j0);
+  const int nq = p.R * CAP / 4, items = nq + p.I + 1;
+  bool wild = false;
+  for (int i = threadIdx.x; i < nj * items; i += SNAP_THREADS) {
+    const int jj = i / items, it = i - jj * items, j = j0 + jj;
+    const unsigned char *rec = recs + (size_t)j * a.L.stride;
+    int bad = -1;
+    if (it < nq) {
+      const int rd = it / (CAP / 4), q = it - rd * (CAP / 4);
+      const uint32_t hw = *reinterpret_cast<const uint32_t *>(rec + a.L.x + rd * CAP * 4);
+      const int ld = (int)(hw & 0xff), lc = (int)((hw >> 8) & 0xff);
+      const bool ld_ok = ld >= 1 && ld < CAP, lc_ok = lc >= 1 && lc < CAP, top_ok = (hw >> 24) == 0;
+      if (q == 0) bad = !ld_ok ? SNAP_BAD_LEADING : (!lc_ok ? SNAP_BAD_LASTCAR : (!top_ok ? SNAP_BAD_HEADER : -1));
+      if (a.check_tame && ld_ok && lc_ok) {
+        const float4 xq = *reinterpret_cast<const float4 *>(rec + a.L.x + rd * CAP * 4 + q * 16);
+        const float4 vq = *reinterpret_cast<const float4 *>(rec + a.L.v + rd * CAP * 4 + q * 16);
+        const float xs[4] = {xq.x, xq.y, xq.z, xq.w}, vs[4] = {vq.x, vq.y, vq.z, vq.w};
+        const int cnt = ring_count(ld, lc);
+#pragma unroll
+        for (int t = 0; t < 4; t++) {
+          const int s = 4 * q + t;
+          if (s == 0) continue;                  // the header word
+          int d = s - ld;
+          if (d < 0) d += RING;                  // ring distance behind the leading slot: 0 = leading, 1..cnt = live cars
+          if (d == 0) wild |= !snap_tame_leader(xs[t]);
+          else if (d <= cnt) wild |= !snap_tame_car(xs[t], vs[t], a.v_cap);
+        }
+      }
+    } else if (it < nq + p.I) {
+      const int b = it - nq;
+      if (rec[a.L.phase + b] > 1) bad = SNAP_BAD_PHASE;
+      else if (rec[a.L.passed_dst + b] > 1) bad = SNAP_BAD_PASSED_DST;
+    } else {
+      const uint32_t *h = reinterpret_cast<const uint32_t *>(rec);
+      if (h[0] != SNAP_MAGIC) bad = SNAP_BAD_MAGIC;
+      else if (h[1] != SNAP_VERSION) bad = SNAP_BAD_VERSION;
+      else if (h[2] != (uint32_t)a.m || h[3] != (uint32_t)a.n || h[5] != (uint32_t)p.R || h[6] != (uint32_t)p.I) bad = SNAP_BAD_DIMS;
+      else if (h[4] != (p.w ? 1u : 0u)) bad = SNAP_BAD_VALIDATE;
+    }
+    if (bad >= 0) atomicMin(&status->first_bad, ((unsigned long long)j << 4) | (unsigned)bad);
+  }
+  if (__syncthreads_or(wild) && threadIdx.x == 0) status->wild = 1;
+}
+
+// te_load_envs, second pass (every record checked): scatter record j into env ids[j].  The header is not stored.
+__global__ void __launch_bounds__(SNAP_THREADS) te_snap_load_kernel(const StepParams p, const SnapArgs a, const int *ids,
+                                                                    const unsigned char *recs) {
+  const int j0 = blockIdx.x * a.per_cta, nj = min(a.per_cta, a.count - j0);
+  snap_planes<false>(p, a, ids, const_cast<unsigned char *>(recs), j0, nj);
+  const int ns = (int)(sizeof(EnvScalars) / 4), per = 3 * p.I + ns;
+  for (int i = threadIdx.x; i < nj * per; i += SNAP_THREADS) {
+    const int jj = i / per, k = i - jj * per, j = j0 + jj, env = snap_env(ids, j);
+    const unsigned char *rec = recs + (size_t)j * a.L.stride;
+    if (k < p.I) p.phase[(size_t)env * p.I + k] = rec[a.L.phase + k];
+    else if (k < 2 * p.I) p.passed_dst[(size_t)env * p.I + k - p.I] = rec[a.L.passed_dst + k - p.I];
+    else if (k < 3 * p.I) p.elapsed[(size_t)env * p.I + k - 2 * p.I] = reinterpret_cast<const int *>(rec + a.L.elapsed)[k - 2 * p.I];
+    else reinterpret_cast<uint32_t *>(p.env + env)[k - 3 * p.I] = reinterpret_cast<const uint32_t *>(rec + a.L.scalars)[k - 3 * p.I];
+  }
+}
+
 // ---- test hooks
 __global__ void te_test_powf_kernel(const float *x, float y, float *out, long long n) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;

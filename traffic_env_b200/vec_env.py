@@ -400,6 +400,58 @@ class VecTrafficEnv(object):
                  ("obs", np.int32), ("waiting", np.int32), ("passed_dst", np.uint8), ("steps", np.float32))]
         check(self._L.te_set_state(self._h, env_begin, count, *[a.ctypes.data for a in arrs]))
 
+    # ------------------------------------------------------------ snapshot records
+    @property
+    def snapshot_layout(self):
+        """Byte layout of one snapshot record (te_snapshot_layout): stride and the offsets of x, v, w (-1 without
+        validate), phase, elapsed, passed_dst and the library-private scalars."""
+        lay = _lib.TeSnapshotLayout()
+        check(self._L.te_snapshot_layout(self._h, C.byref(lay)))
+        return lay
+
+    def _env_ids(self, env_ids, count=None):
+        """(int32 id array or None, count) for te_save_envs / te_load_envs; None stands for envs [0, count)."""
+        if env_ids is None:
+            return None, self.num_envs if count is None else count
+        ids = np.ascontiguousarray(np.asarray(env_ids, dtype=np.int64).reshape(-1), dtype=np.int32)
+        return ids, ids.size
+
+    def save_envs(self, env_ids=None, out=None, stream=None):
+        """Snapshot records of the listed envs (all when env_ids is None; duplicates allowed), one row of
+        snapshot_layout.stride bytes per id.  out None: a new uint8[count, stride] host array (synchronous); a host array:
+        filled in place; a CUDA torch tensor or a raw device pointer: written on the device, asynchronously on `stream`
+        (a cudaStream_t as int, None = the handle's stream) after the steps queued there before it."""
+        ids, count = self._env_ids(env_ids)
+        stride = self.snapshot_layout.stride
+        if out is None or isinstance(out, np.ndarray):
+            if out is None:
+                out = np.empty((count, stride), np.uint8)
+            assert out.flags.c_contiguous and out.nbytes == count * stride, "out must be C-contiguous [count, stride] bytes"
+            check(self._L.te_save_envs(self._h, _ptr(ids), count, out.ctypes.data, TE_HOST, None))
+            return out
+        if not isinstance(out, int):
+            assert out.is_cuda and out.is_contiguous() and out.numel() * out.element_size() >= count * stride, \
+                "out must be a contiguous CUDA tensor of at least count * stride bytes"
+        check(self._L.te_save_envs(self._h, _ptr(ids), count, out if isinstance(out, int) else _ptr(out), TE_DEVICE,
+                                   stream))
+        return out
+
+    def load_envs(self, records, env_ids=None):
+        """Load snapshot records (a host array or CUDA torch tensor of [count, stride] bytes) into the listed envs, record j
+        into env env_ids[j] (envs [0, count) when env_ids is None).  Synchronous; every record is checked first, and a bad
+        one raises TrafficB200Error with every env left as it was."""
+        stride = self.snapshot_layout.stride
+        if isinstance(records, np.ndarray):
+            rec = np.ascontiguousarray(records).view(np.uint8).reshape(-1)
+            mem, ptr, nbytes = TE_HOST, rec.ctypes.data, rec.nbytes
+        else:
+            assert records.is_cuda and records.is_contiguous(), "device records must be a contiguous CUDA tensor"
+            mem, ptr, nbytes = TE_DEVICE, _ptr(records), records.numel() * records.element_size()
+        ids, count = self._env_ids(env_ids, nbytes // stride)
+        if nbytes < count * stride or (env_ids is None and nbytes != count * stride):
+            raise ValueError("records hold %d bytes; %d records of %d bytes expected" % (nbytes, count, stride))
+        check(self._L.te_load_envs(self._h, _ptr(ids), count, ptr, mem, None))
+
     def trip_times(self, clear=True):
         """Validate mode: (env ids, trip times in seconds) of the cars that left the map since the last clear."""
         n = C.c_int64()
