@@ -253,7 +253,7 @@ int te_save_envs(te_handle *h, const int32_t *env_ids, int32_t count, void *reco
 int te_load_envs(te_handle *h, const int32_t *env_ids, int32_t count, const void *records, int memspace, void *stream);
 
 /* *tame = 1 while the handle runs the unchecked arithmetic: its archetype is inside the supported ranges and every car ever
-   handed to te_set_state was tame - x finite with |x| < 2^40, v zero or in [2^-100, *v_cap], *v_cap = twice the fastest
+   handed to te_set_state was tame - x finite with |x| < 2^40 and not -0, v zero or in [2^-100, *v_cap], *v_cap = twice the fastest
    speed the archetype's dynamics can produce.  Tame state stays tame under the step, and no operand of the IDM update can
    then leave the domain on which its fast sequences are exact, so the per-car validity predicate and the generic
    fallback are not compiled into the kernels that run (DESIGN.md section 4).  One wild car in te_set_state switches the

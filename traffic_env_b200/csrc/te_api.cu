@@ -289,8 +289,9 @@ static bool tame_archetype(const te_config *cfg, float *v_cap) {
   auto in = [](double v, double lo, double hi) { return std::isfinite(v) && v >= lo && v <= hi; };
   const double tiny = ldexp(1.0, -10), big = ldexp(1.0, 19);
   *v_cap = 0.f;
-  if (!(in(a[0], -ldexp(1.0, 30), ldexp(1.0, 30)) && (a[1] == 0.f || in(a[1], tiny, big)) && in(a[2], 0.0, big) &&
-        in(a[3], tiny, big) && in(a[4], tiny, 64.0) && in(a[5], tiny, big) && in(a[6], tiny, big) && in(a[7], tiny, big) &&
+  // (x_new = -0: cars would enter at a position tame_car rejects)
+  if (!(in(a[0], -ldexp(1.0, 30), ldexp(1.0, 30)) && !(a[0] == 0.f && std::signbit(a[0])) &&
+        (a[1] == 0.f || in(a[1], tiny, big)) && in(a[2], 0.0, big) && in(a[3], tiny, big) && in(a[4], tiny, 64.0) && in(a[5], tiny, big) && in(a[6], tiny, big) && in(a[7], tiny, big) &&
         in(a[8], tiny, big) && in(cfg->rate, tiny, 1024.0) && in(cfg->length, tiny, ldexp(1.0, 30))))
     return false;
   const double cap = 2.0 * std::max((double)a[1], (double)a[5] + (double)a[3] * cfg->rate);
@@ -302,8 +303,9 @@ static bool tame_archetype(const te_config *cfg, float *v_cap) {
   *v_cap = (float)cap;
   return true;
 }
+// x = -0 is not tame: the tame kernels move a car with dx <= 0 by keeping x, where the reference adds +-0 (te_math.cuh)
 static bool tame_car(float x, float v, float v_cap) {
-  return std::isfinite(x) && fabsf(x) < ldexpf(1.f, 40) && std::isfinite(v) &&
+  return std::isfinite(x) && fabsf(x) < ldexpf(1.f, 40) && !(x == 0.f && std::signbit(x)) && std::isfinite(v) &&
          (v == 0.f ? !std::signbit(v) : (v >= ldexpf(1.f, -100) && v <= v_cap));
 }
 static int select_layout(te_handle *h);

@@ -38,7 +38,7 @@ constexpr int CAP = 20;            // CAPACITY, traffic_env.py:24
 constexpr int RING = CAP - 1;      // live ring positions 1..19
 constexpr int YELLOW_TICKS = 6;    // traffic_env.py:21
 constexpr int GROUP_ROADS = 32;    // one road per lane of the owning warp
-constexpr int WARP_AREA = 704;     // per-warp tables of the car loop: 32 x (16 B road entry + 4 B counters + 2 B list start)
+constexpr int WARP_AREA = 720;     // per-warp tables of the car loop: 33 x 16 B road entry, 32 x (4 B counters + 2 B list start)
 constexpr int MAX_K = 64;
 
 enum : int { F_LEARN_SWITCH = 1, F_REMI = 2, F_AUTO_RESET = 4, F_VALIDATE = 8, F_ORDERED = 16 };
@@ -167,7 +167,7 @@ enum : int { CTA_RUNNING = 0,         // envs still running (an env stops after 
 constexpr int MAX_G = 8;           // most env instances one CTA can hold (te_api.cu: select_layout)
 
 struct SmemLayout {
-  int xs, vs, ws, tabs, mbar, tailx, meta, wait, elapsed, ovf, rew, misc, envm, warp, phase, act, pdst, cnt;
+  int sink, xs, vs, ws, tabs, mbar, tailx, meta, wait, elapsed, ovf, rew, misc, envm, warp, phase, act, pdst, cnt;
 };
 
 __host__ __device__ constexpr int align_up(int a, int b) { return (a + b - 1) / b * b; }
@@ -176,7 +176,11 @@ __host__ __device__ constexpr SmemLayout make_layout(int maxt, bool validate) {
   SmemLayout L = {};
   const int icap = align_up(maxt / 4, 4);               // 4 I = r < R <= Rp <= maxt
   int o = 0;
+  // The car loop's sink slot: x at L.sink, below every row, and v at the same distance from it as the v plane from the
+  // x plane, in the 16 bytes between the two planes.
+  L.sink = o; o += 16;
   L.xs = o; o += maxt * CAP * 4;
+  o += 16;
   L.vs = o; o += maxt * CAP * 4;
   L.ws = o; o += validate ? maxt * CAP * 4 : 0;
   L.tabs = o;                                           // (the powf tables stay in global memory: only the rare full-powf path reads them)
@@ -471,6 +475,9 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
   if (tid == 0) {
     s.misc[CTA_RUNNING] = nactive; s.misc[CTA_ORD_TICK] = -1; s.misc[CTA_VEH_UPDATES] = 0; s.misc[CTA_OVERFLOWS] = 0;
     s.misc[CTA_GENERATED] = 0; s.misc[CTA_ORD_ENV_TICKS] = 0; s.misc[CTA_EXITED] = 0;
+    // the sink car (see the car loop): x = NaN, v = +0
+    reinterpret_cast<float *>(smem_raw + L.sink)[0] = __int_as_float(0x7fffffff);
+    reinterpret_cast<float *>(smem_raw + L.sink + (L.vs - L.xs))[0] = 0.f;
   }
   if (tid < G) {
     s.env_word(tid, ENVM_OVF) = NO_OVERFLOW; s.env_word(tid, ENVM_ORD) = -1; s.env_word(tid, ENVM_TB) = 0;
@@ -570,6 +577,15 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
     s.xs[tid * CAP] = __uint_as_float(pack_meta(1, 1, 0)); s.vs[tid * CAP] = __int_as_float(0);
     s.xs[tid * CAP + 1] = INF; s.vs[tid * CAP + 1] = 0.f;
   }
+  {
+    // Every road-table entry starts with addresses above the sink slot (here: the table's own), so that every entry the
+    // car loop can load - the one past the last listed road included - has them: a lane on the sink never crosses and
+    // its waiting test reads x.  The tick loop only writes row addresses, above the sink too; entry 32 (the one past 32
+    // listed roads) keeps this one.
+    const uint32_t t_a = smem_u32(s.warp + warp * WARP_AREA);
+    sts_v4(t_a + 16u * lane, make_uint4(t_a, t_a, t_a, 0u));
+    if (lane == 0) sts_v4(t_a + 16u * 32, make_uint4(t_a, t_a, t_a, 0u));
+  }
 
   // ---- row -> (warp, lane) assignment for this launch, balanced by car count: counting sort of the rows by
   // their current number of cars (0..18), then dealt to the warps in snake order, so every warp simulates
@@ -627,11 +643,13 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
   // (all three are reached from ONE 32-bit shared address, rt_a, with immediates: no generic pointers kept per table)
   const uint32_t rt_a = smem_u32(s.warp + warp * WARP_AREA);             // rt: non-empty roads of the warp, in lane order:
                                                                          // shared addresses of x[leading], x[lastcar], x[19]; leader x
-  constexpr int WCNT_OFF = 32 * 16;                                      // wcnt: waiting | detected << 16 per listed road
+                                                                         // (entry 32: only ever the prologue's, see there)
+  constexpr int WCNT_OFF = 33 * 16;                                      // wcnt: waiting | detected << 16 per listed road
   constexpr int WST_OFF = WCNT_OFF + 32 * 4;                             // wst: first list position of each listed road (u16)
   const uint32_t wcnt_a = rt_a + WCNT_OFF;
   const uint32_t xrow_a = smem_u32(xr);                                  // shared address of x[my row][0]
   constexpr int VOFF = L.vs - L.xs;                                      // v plane relative to the x plane
+  const uint32_t sink_a = smem_u32(smem_raw + L.sink);                   // x of the sink car (v at + VOFF)
   const unsigned lt_mask = (1u << lane) - 1u;
   __syncthreads();
 
@@ -715,8 +733,9 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
       const int target = lane * q;
       const int cnt = min(q, total - target);                  // cars of my run (<= 0: none)
       // run state: address of my car's x slot; x[leading], x[lastcar], x[19] of its road; table cursors;
-      // (px, pv, pl) = pre-update x, v and length of the car ahead (virtual leader: v = 0, l = 0, SURVEY 8a quirks)
-      uint32_t addr = 0, ldaddr = 0, lcaddr = 0, endaddr = 0, jaddr = rt_a, caddr = wcnt_a;
+      // (px, pv, pl) = pre-update x, v and length of the car ahead (virtual leader: v = 0, l = 0, SURVEY 8a quirks).
+      // A lane without a run starts on the sink (below), with the table's own address as its road addresses.
+      uint32_t addr = sink_a, ldaddr = rt_a, lcaddr = rt_a, endaddr = rt_a, jaddr = rt_a, caddr = wcnt_a;
       float px = 0.f, pv = 0.f, pl = 0.f;
       if (cnt > 0) {
         int lo = 0;
@@ -735,33 +754,37 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
       }
       __syncwarp();  // every run has read the leader of its first car before any lane overwrites a slot
       // a uniform trip count: a per-lane one (the lanes of the shorter runs leaving early) measured 4.5 % / 8 % slower
-      // (10x10 / 3x3): lanes drifting apart cost more than the re-convergence
+      // (10x10 / 3x3): lanes drifting apart cost more than the re-convergence.
+      // A lane whose run is over, or empty, does not branch around the body: it updates the sink car, one slot shared
+      // by every such lane of the CTA (x = NaN, v = +0, set up in the prologue).  Whatever its leader, its update writes
+      // back x = NaN and v = +0 (te_math.cuh: idm_update), and v = +0 keeps it on the powf shortcut.  Its slot lies below
+      // every row (addr < ldaddr), so its waiting test reads x: NaN < 0.2f and NaN > det_thr_f are false, and its red.add
+      // adds 0.  It never crosses: lcaddr is always a row or table address, above the sink.
       for (int i = 0; i < q; i++) {
-        if (i < cnt) {
-          float xn = lds_f32(addr), vn = lds_f32_off<VOFF>(addr);
-          const float xl = px, vl = pv, ll = pl;
-          px = xn; pv = vn; pl = c.len;
-          // the tame kernels run the unchecked arithmetic; te_api.cu only launches them on tame handles
-          idm_update<TAME>(c, s.tabs, xl, vl, ll, xn, vn);
-          sts_f32(addr, xn); sts_f32_off<VOFF>(addr, vn);
-          // wrapped ring, low segment (slot < leading): the reference tests x, not v (traffic_env.py:210).
-          // THRESH = 0.2 is compared in double by the reference; 0.2f is the smallest float above 0.2, so for every
-          // float w: (double)w < 0.2  <=>  w < 0.2f.  Same for the detector threshold with det_thr_f (see StepParams).
-          // My car's counts go straight to its road's counters, so moving on to the next road hands nothing over.
-          uint32_t cw = (((addr < ldaddr) ? xn : vn) < 0.2f) ? 1u : 0u;
-          if (xn > p.det_thr_f) cw += 0x10000u;
-          red_add_shared(caddr, cw);
-          // Past the road's last car: move on to the next listed road.  Some lane of the warp does so in nearly every
-          // iteration, so the cursors and the run state are updated by predicated instructions, not in a branch.
-          const bool cross = addr == lcaddr;
-          if (cross) { jaddr += 16u; caddr += 4u; }
-          uint4 e = make_uint4(ldaddr, lcaddr, endaddr, __float_as_uint(px));
-          lds_v4_if(cross, jaddr, e);  // (past the last listed road: a stale entry that is never used, cnt ends the run)
-          ldaddr = e.x; lcaddr = e.y; endaddr = e.z; px = __uint_as_float(e.w);
-          pv = cross ? 0.f : pv; pl = cross ? 0.f : pl;
-          const uint32_t from = cross ? ldaddr : addr;  // the slot before my next car
-          addr = (from == endaddr) ? from - 4u * (RING - 1) : from + 4u;
-        }
+        float xn = lds_f32(addr), vn = lds_f32_off<VOFF>(addr);
+        const float xl = px, vl = pv, ll = pl;
+        px = xn; pv = vn; pl = c.len;
+        // the tame kernels run the unchecked arithmetic; te_api.cu only launches them on tame handles
+        idm_update<TAME>(c, s.tabs, xl, vl, ll, xn, vn, i < cnt);
+        sts_f32(addr, xn); sts_f32_off<VOFF>(addr, vn);
+        // wrapped ring, low segment (slot < leading): the reference tests x, not v (traffic_env.py:210).
+        // THRESH = 0.2 is compared in double by the reference; 0.2f is the smallest float above 0.2, so for every
+        // float w: (double)w < 0.2  <=>  w < 0.2f.  Same for the detector threshold with det_thr_f (see StepParams).
+        // My car's counts go straight to its road's counters, so moving on to the next road hands nothing over.
+        uint32_t cw = (((addr < ldaddr) ? xn : vn) < 0.2f) ? 1u : 0u;
+        if (xn > p.det_thr_f) cw += 0x10000u;
+        red_add_shared(caddr, cw);
+        // Past the road's last car: move on to the next listed road.  Some lane of the warp does so in nearly every
+        // iteration, so the cursors and the run state are updated by predicated instructions, not in a branch.
+        const bool cross = addr == lcaddr;
+        if (cross) { jaddr += 16u; caddr += 4u; }
+        uint4 e = make_uint4(ldaddr, lcaddr, endaddr, __float_as_uint(px));
+        lds_v4_if(cross, jaddr, e);  // (past the last listed road: an entry from an earlier tick or the prologue's; the sink follows)
+        ldaddr = e.x; lcaddr = e.y; endaddr = e.z; px = __uint_as_float(e.w);
+        pv = cross ? 0.f : pv; pl = cross ? 0.f : pl;
+        const uint32_t from = cross ? ldaddr : addr;  // the slot before my next car
+        addr = (from == endaddr) ? from - 4u * (RING - 1) : from + 4u;
+        addr = (i + 1 < cnt) ? addr : sink_a;
       }
       __syncwarp();
     }
@@ -1204,7 +1227,7 @@ __global__ void __launch_bounds__(SNAP_THREADS) te_snap_save_kernel(const StepPa
 
 // te_set_state's tame predicate (te_api.cu: tame_car and the leading-slot rule), on the device
 __device__ __forceinline__ bool snap_tame_car(float x, float v, float v_cap) {
-  return isfinite(x) && fabsf(x) < 0x1p40f && isfinite(v) && (v == 0.f ? !signbit(v) : (v >= 0x1p-100f && v <= v_cap));
+  return isfinite(x) && fabsf(x) < 0x1p40f && __float_as_uint(x) != 0x80000000u && isfinite(v) && (v == 0.f ? !signbit(v) : (v >= 0x1p-100f && v <= v_cap));
 }
 __device__ __forceinline__ bool snap_tame_leader(float x) {
   return x == __int_as_float(0x7f800000) || (isfinite(x) && fabsf(x) < 0x1p40f);
