@@ -212,8 +212,16 @@ int te_greedy_actions(te_handle *h, uint8_t *actions, int memspace, void *stream
 
 /* Full state of envs [env_begin, env_begin+count) in the reference's layout, host pointers, any may be
    NULL: leading/lastcar int32[count,R]; x, v float[count,R,20] (only live slots and the leading slot are
-   meaningful, as in the reference); obs int32[count,2r+2I]; waiting int32[count,r];
-   passed_dst uint8[count,I]; steps float[count]. */
+   meaningful, as in the reference; slot 0 reads NaN); obs int32[count,2r+2I] (passed 0, detected, phase, elapsed);
+   waiting int32[count,r]; passed_dst uint8[count,I]; steps float[count].
+   Both calls go through the envs' snapshot records (te_save_envs / te_load_envs), in host memory, and are synchronous:
+   they first wait for steps queued on any stream.  They use the handle's device staging for host records, which grows
+   to count * stride bytes and is kept (about 1.17 GB for all 16384 envs of a 10x10 handle).
+   te_set_state writes what te_get_state reads (every array but steps is required; steps NULL keeps the tick counter)
+   and keeps the rest of each env: birth ticks, arrival-stream position, clocks and return statistics.  Slot 0 of x and
+   v is not read.  Phase and passed_dst are stored as 0 / 1 (any non-zero byte is 1).  It fails, with every env left
+   as it was, unless every leading / lastcar is in [1, 20) and every detected count in [0, 255].  Its records pass
+   te_load_envs's check, tame-car rule included (te_is_tame). */
 int te_get_state(te_handle *h, int32_t env_begin, int32_t count, int32_t *leading, int32_t *lastcar, float *x,
                  float *v, int32_t *obs, int32_t *waiting, uint8_t *passed_dst, float *steps);
 int te_set_state(te_handle *h, int32_t env_begin, int32_t count, const int32_t *leading, const int32_t *lastcar,
@@ -245,19 +253,20 @@ int te_snapshot_layout(const te_handle *h, te_snapshot_layout_t *out);
    make the call wait for that stream); TE_HOST: synchronous. */
 int te_save_envs(te_handle *h, const int32_t *env_ids, int32_t count, void *records, int memspace, void *stream);
 /* te_load_envs scatters record j into env env_ids[j] (each id at most once); synchronous in both memspaces (`stream` is
-   not used), like te_set_state.  Every record is checked on the device before anything is written - magic, version,
-   m / n, the validate bit, every row's leading and lastcar in [1, 20) with the header word's top byte zero, phase and
-   passed_dst in {0, 1} - and on a failure the call returns an error naming the first bad record and field and leaves
-   every env untouched.  On a tame handle the same pass applies te_set_state's tame predicate to every live car and
-   leading slot: one wild car moves the handle to the checked kernels for good, exactly as te_set_state does. */
+   not used): it first waits for steps queued on any stream.  Every record is checked on the device before anything is
+   written - magic, version, m / n, the validate bit, every row's leading and lastcar in [1, 20) with the header word's
+   top byte zero, phase and passed_dst in {0, 1} - and on a failure the call returns an error naming the first bad record
+   and field and leaves every env untouched.  On a tame handle the same pass applies the tame-car rule (te_is_tame) to
+   every live car and leading slot: one wild car moves the handle to the checked kernels for good. */
 int te_load_envs(te_handle *h, const int32_t *env_ids, int32_t count, const void *records, int memspace, void *stream);
 
 /* *tame = 1 while the handle runs the unchecked arithmetic: its archetype is inside the supported ranges and every car ever
-   handed to te_set_state was tame - x finite with |x| < 2^40 and not -0, v zero or in [2^-100, *v_cap], *v_cap = twice the fastest
-   speed the archetype's dynamics can produce.  Tame state stays tame under the step, and no operand of the IDM update can
-   then leave the domain on which its fast sequences are exact, so the per-car validity predicate and the generic
-   fallback are not compiled into the kernels that run (DESIGN.md section 4).  One wild car in te_set_state switches the
-   handle to the checked kernels for good.  v_cap may be NULL. */
+   handed to te_load_envs or te_set_state was tame - x finite with |x| < 2^40 and not -0, v zero or in [2^-100, *v_cap],
+   *v_cap = twice the fastest speed the archetype's dynamics can produce; a leading slot's x finite with |x| < 2^40, or
+   +inf.  Tame state stays tame under the step, and no operand of the IDM update can then leave the domain on which its
+   fast sequences are exact, so the per-car validity predicate and the generic fallback are not compiled into the
+   kernels that run (DESIGN.md section 4).  One wild car in te_load_envs or te_set_state switches the handle to the
+   checked kernels for good.  v_cap may be NULL. */
 int te_is_tame(const te_handle *h, int32_t *tame, float *v_cap);
 /* The speed cap of the tame domain for an archetype / tick length / road length, 0 when the archetype is outside the
    supported ranges (host arithmetic only: needs no device). */

@@ -18,10 +18,21 @@ def test_argument_errors_are_reported():
         env.step(np.zeros((4, 9)), k=65)
     with pytest.raises(TrafficB200Error, match="out of bounds"):
         env.get_state(2, 3)
+    before = env.save_envs()
     st = env.get_state()
-    st["leading"][0, 0] = 0
+    st["leading"][3, 0] = 0                                  # the last env only: the earlier ones are not written either
     with pytest.raises(TrafficB200Error, match="ring index"):
         env.set_state(st)
+    assert env.save_envs().tobytes() == before.tobytes()
+    st = env.get_state()
+    st["obs"][3, env.train_roads] = 256                      # detected of road 0: one byte of the row header
+    with pytest.raises(TrafficB200Error, match="detected"):
+        env.set_state(st)
+    assert env.save_envs().tobytes() == before.tobytes()
+    st = env.get_state()
+    st["passed_dst"][1, 2] = 2
+    env.set_state(st)
+    assert env.get_state()["passed_dst"][1, 2] == 1
     with pytest.raises(TrafficB200Error, match="TE_VALIDATE"):
         env.trip_times()
     obs, rew, done = env.step(np.zeros((4, 9)))              # still usable after the errors

@@ -78,8 +78,11 @@ def test_sampled_envs_replay_on_oracle(big):
 
 def test_state_round_trip_is_idempotent(big):
     env, _ = big
+    ids = range(100, 164)
+    rec = env.save_envs(ids)
     a = env.get_state(100, 64)
     env.set_state(a, env_begin=100)
     b = env.get_state(100, 64)
     for k in ("leading", "lastcar", "obs", "waiting", "passed_dst"):
         assert (a[k] == b[k]).all(), k
+    assert env.save_envs(ids).tobytes() == rec.tobytes()

@@ -54,6 +54,8 @@ def test_rewind_replays_bit_for_bit(name, kw, multi):
     if validate:
         env.trip_times(clear=True)
     rec = env.save_envs()
+    env.set_state(env.get_state())                     # keeps everything it does not set (w plane, scalars, clocks)
+    assert env.save_envs().tobytes() == rec.tobytes(), name + ": get_state / set_state round trip"
     ep0 = env.stats()["episodes"]
     first = run_window(env, 7, multi)
     st1, rec1 = env.get_state(), env.save_envs()

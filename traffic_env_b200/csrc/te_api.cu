@@ -9,11 +9,13 @@
 #include <cstdio>
 #include <cstdlib>
 #include <algorithm>
+#include <cstddef>
 #include <cstring>
 #include <atomic>
 #include <condition_variable>
 #include <memory>
 #include <mutex>
+#include <numeric>
 #include <string>
 #include <thread>
 #include <vector>
@@ -205,7 +207,8 @@ struct te_handle {
   int ctrl_spacing = 0;  // TE_CTRL_GREEDY: a new decision every so many actor steps inside a te_step_multi launch (0: one per launch)
   int actions_cap = 1;   // decisions d_actions has room for
   bool float_dma = false;  // te_step(TE_HOST) with float outputs: let the copy engine write the float arrays (no host expansion)
-  // snapshot records (te_save_envs / te_load_envs): device staging of host records, and the check pass's status word
+  // snapshot records (te_save_envs / te_load_envs, and te_get_state / te_set_state through them): device staging of host
+  // records, and the check pass's status word
   dev_buf<unsigned char> d_snap; size_t snap_cap = 0;
   dev_buf<SnapStatus> d_snap_status;
   std::unique_ptr<ExpandPool> pool;
@@ -289,7 +292,7 @@ static bool tame_archetype(const te_config *cfg, float *v_cap) {
   auto in = [](double v, double lo, double hi) { return std::isfinite(v) && v >= lo && v <= hi; };
   const double tiny = ldexp(1.0, -10), big = ldexp(1.0, 19);
   *v_cap = 0.f;
-  // (x_new = -0: cars would enter at a position tame_car rejects)
+  // (x_new = -0: cars would enter at a position tame_car (te_kernels.cuh) rejects)
   if (!(in(a[0], -ldexp(1.0, 30), ldexp(1.0, 30)) && !(a[0] == 0.f && std::signbit(a[0])) &&
         (a[1] == 0.f || in(a[1], tiny, big)) && in(a[2], 0.0, big) && in(a[3], tiny, big) && in(a[4], tiny, 64.0) && in(a[5], tiny, big) && in(a[6], tiny, big) && in(a[7], tiny, big) &&
         in(a[8], tiny, big) && in(cfg->rate, tiny, 1024.0) && in(cfg->length, tiny, ldexp(1.0, 30))))
@@ -302,11 +305,6 @@ static bool tame_archetype(const te_config *cfg, float *v_cap) {
   if (!((double)a[3] * (q_max * q_max + pow(cap / a[5], (double)a[4]) + 1.0) < ldexp(1.0, 126))) return false;
   *v_cap = (float)cap;
   return true;
-}
-// x = -0 is not tame: the tame kernels move a car with dx <= 0 by keeping x, where the reference adds +-0 (te_math.cuh)
-static bool tame_car(float x, float v, float v_cap) {
-  return std::isfinite(x) && fabsf(x) < ldexpf(1.f, 40) && !(x == 0.f && std::signbit(x)) && std::isfinite(v) &&
-         (v == 0.f ? !std::signbit(v) : (v >= ldexpf(1.f, -100) && v <= v_cap));
 }
 static int select_layout(te_handle *h);
 
@@ -365,7 +363,7 @@ static std::vector<uint32_t> build_gap_cdf(double cars_per_tick) {
 extern "C" int te_destroy(te_handle *h) { delete h; return 0; }
 
 // Threads per CTA, env instances per CTA and the kernel variant of a handle; called by te_create and again when a
-// handle stops being tame (te_set_state with a wild car: the checked, one-env-per-CTA kernels take over).
+// handle stops being tame (a wild car in loaded records, load_records: the checked, one-env-per-CTA kernels take over).
 static int select_layout(te_handle *h) {
   const te_config *cfg = &h->cfg;
   StepParams &p = h->base;
@@ -950,113 +948,6 @@ extern "C" int te_greedy_actions(te_handle *h, uint8_t *actions, int memspace, v
   return 0;
 }
 
-extern "C" int te_get_state(te_handle *h, int32_t env_begin, int32_t count, int32_t *leading, int32_t *lastcar, float *x,
-                            float *v, int32_t *obs, int32_t *waiting, uint8_t *passed_dst, float *steps) {
-  if (!h) return fail("te_get_state: null handle");
-  if (env_begin < 0 || count < 0 || env_begin + count > h->cfg.num_envs) return fail("te_get_state: env range out of bounds");
-  CU(cudaSetDevice(h->device));
-  CU(cudaDeviceSynchronize());
-  const size_t row = (size_t)h->Rp * CAP;
-  std::vector<float> hx(row * count), hv(row * count);
-  std::vector<int> hel((size_t)h->I * count);
-  std::vector<uint8_t> hph((size_t)h->I * count), hpd((size_t)h->I * count);
-  std::vector<EnvScalars> hes(count);
-  CU(cudaMemcpy(hx.data(), h->x.get() + env_begin * row, hx.size() * 4, cudaMemcpyDeviceToHost));
-  CU(cudaMemcpy(hv.data(), h->v.get() + env_begin * row, hv.size() * 4, cudaMemcpyDeviceToHost));
-  CU(cudaMemcpy(hel.data(), h->elapsed.get() + (size_t)env_begin * h->I, hel.size() * 4, cudaMemcpyDeviceToHost));
-  CU(cudaMemcpy(hph.data(), h->phase.get() + (size_t)env_begin * h->I, hph.size(), cudaMemcpyDeviceToHost));
-  CU(cudaMemcpy(hpd.data(), h->passed_dst.get() + (size_t)env_begin * h->I, hpd.size(), cudaMemcpyDeviceToHost));
-  CU(cudaMemcpy(hes.data(), h->env.get() + env_begin, hes.size() * sizeof(EnvScalars), cudaMemcpyDeviceToHost));
-  const int R = h->R, r = h->r, I = h->I, ol = 2 * r + 2 * I;
-  for (int e = 0; e < count; e++) {
-    for (int rd = 0; rd < R; rd++) {
-      uint32_t w0; memcpy(&w0, &hx[e * row + (size_t)rd * CAP], 4);
-      int wt; memcpy(&wt, &hv[e * row + (size_t)rd * CAP], 4);
-      const RowHeader m = unpack_meta(w0);
-      if (leading) leading[(size_t)e * R + rd] = m.leading;
-      if (lastcar) lastcar[(size_t)e * R + rd] = m.lastcar;
-      if (obs && rd < r) { obs[(size_t)e * ol + rd] = 0; obs[(size_t)e * ol + r + rd] = m.detected; }
-      if (waiting && rd < r) waiting[(size_t)e * r + rd] = wt;
-      if (x) { memcpy(&x[((size_t)e * R + rd) * CAP], &hx[e * row + (size_t)rd * CAP], CAP * 4); x[((size_t)e * R + rd) * CAP] = NAN; }
-      if (v) { memcpy(&v[((size_t)e * R + rd) * CAP], &hv[e * row + (size_t)rd * CAP], CAP * 4); v[((size_t)e * R + rd) * CAP] = NAN; }
-    }
-    for (int i = 0; i < I; i++) {
-      if (obs) { obs[(size_t)e * ol + 2 * r + i] = hph[(size_t)e * I + i]; obs[(size_t)e * ol + 2 * r + I + i] = hel[(size_t)e * I + i]; }
-      if (passed_dst) passed_dst[(size_t)e * I + i] = hpd[(size_t)e * I + i];
-    }
-    if (steps) steps[e] = hes[e].steps;
-  }
-  return 0;
-}
-
-extern "C" int te_set_state(te_handle *h, int32_t env_begin, int32_t count, const int32_t *leading, const int32_t *lastcar,
-                            const float *x, const float *v, const int32_t *obs, const int32_t *waiting,
-                            const uint8_t *passed_dst, const float *steps) {
-  if (!h) return fail("te_set_state: null handle");
-  if (env_begin < 0 || count < 0 || env_begin + count > h->cfg.num_envs) return fail("te_set_state: env range out of bounds");
-  if (!leading || !lastcar || !x || !v || !obs || !waiting || !passed_dst) return fail("te_set_state: all state arrays are required");
-  CU(cudaSetDevice(h->device));
-  CU(cudaDeviceSynchronize());
-  const size_t row = (size_t)h->Rp * CAP;
-  const int R = h->R, r = h->r, I = h->I, ol = 2 * r + 2 * I;
-  std::vector<float> hx(row * count, 0.f), hv(row * count, 0.f);
-  std::vector<int> hel((size_t)I * count);
-  std::vector<uint8_t> hph((size_t)I * count), hpd((size_t)I * count);
-  std::vector<EnvScalars> hes(count);
-  CU(cudaMemcpy(hes.data(), h->env.get() + env_begin, hes.size() * sizeof(EnvScalars), cudaMemcpyDeviceToHost));
-  bool wild = false;
-  for (int e = 0; e < count; e++) {
-    for (int rd = 0; rd < h->Rp; rd++) {
-      uint32_t w0 = pack_meta(1, 1, 0); int wt = 0;
-      float *xr = &hx[e * row + (size_t)rd * CAP], *vr = &hv[e * row + (size_t)rd * CAP];
-      if (rd < R) {
-        const int ld = leading[(size_t)e * R + rd], lc = lastcar[(size_t)e * R + rd];
-        if (ld < 1 || ld >= CAP || lc < 1 || lc >= CAP) return fail("te_set_state: ring index out of range");
-        // every live car (and the leading slot's x, the virtual leader: finite or +inf) must be tame for the unchecked
-        // arithmetic; one wild car moves the whole handle to the checked kernels for good
-        for (int sl = ld; sl != lc;) {
-          sl = sl + 1 >= CAP ? 1 : sl + 1;
-          if (!tame_car(x[((size_t)e * R + rd) * CAP + sl], v[((size_t)e * R + rd) * CAP + sl], h->v_cap)) wild = true;
-        }
-        {
-          const float lx = x[((size_t)e * R + rd) * CAP + ld];
-          if (!(lx == INFINITY || (std::isfinite(lx) && fabsf(lx) < ldexpf(1.f, 40)))) wild = true;
-        }
-        memcpy(xr, &x[((size_t)e * R + rd) * CAP], CAP * 4);
-        memcpy(vr, &v[((size_t)e * R + rd) * CAP], CAP * 4);
-        const int det = rd < r ? obs[(size_t)e * ol + r + rd] : 0;
-        w0 = pack_meta(ld, lc, det);
-        wt = rd < r ? waiting[(size_t)e * r + rd] : 0;
-      } else {
-        xr[1] = INFINITY;
-      }
-      memcpy(xr, &w0, 4); memcpy(vr, &wt, 4);
-    }
-    for (int i = 0; i < I; i++) {
-      hph[(size_t)e * I + i] = obs[(size_t)e * ol + 2 * r + i] != 0;
-      hel[(size_t)e * I + i] = obs[(size_t)e * ol + 2 * r + I + i];
-      hpd[(size_t)e * I + i] = passed_dst[(size_t)e * I + i];
-    }
-    if (steps) hes[e].steps = steps[e];
-  }
-  // uploads go through the handle's stream and the device is synchronised afterwards, so they are ordered against
-  // steps on ANY stream (the step streams are non-blocking: the legacy default stream does not order against them)
-  cudaStream_t st = h->stream.get();
-  CU(cudaMemcpyAsync(h->x.get() + env_begin * row, hx.data(), hx.size() * 4, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(h->v.get() + env_begin * row, hv.data(), hv.size() * 4, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(h->elapsed.get() + (size_t)env_begin * I, hel.data(), hel.size() * 4, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(h->phase.get() + (size_t)env_begin * I, hph.data(), hph.size(), cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(h->passed_dst.get() + (size_t)env_begin * I, hpd.data(), hpd.size(), cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(h->env.get() + env_begin, hes.data(), hes.size() * sizeof(EnvScalars), cudaMemcpyHostToDevice, st));
-  CU(cudaStreamSynchronize(st));
-  CU(cudaDeviceSynchronize());
-  if (wild && h->tame) {      // from now on: the kernels with the per-car validity predicate, one env per CTA
-    h->tame = false;
-    if (int rc = select_layout(h)) return rc;
-  }
-  return 0;
-}
-
 // ---- snapshot records (te_kernels.cuh: snap_layout)
 static SnapLayout snap_layout_of(const te_handle *h) { return snap_layout(h->R, h->I, (h->cfg.flags & TE_VALIDATE) != 0); }
 
@@ -1101,17 +992,21 @@ static SnapArgs snap_args(const te_handle *h, int32_t count, unsigned *blocks) {
   return a;
 }
 
-// A device copy of a host id list, allocated (and later freed) in the order of `st`: a save queued on a stream keeps
-// its own ids while the caller goes on.
-static int upload_ids(const int32_t *env_ids, int32_t count, cudaStream_t st, int **out) {
+// A device copy of a host id list.  A synchronous call passes `staged`, room in the handle's staging; an asynchronous
+// save gets a copy allocated (and later freed) in the order of `st`, so that it keeps its own ids while the caller goes
+// on.  (The synchronous calls do not allocate: the default pool returns freed memory at every synchronisation, and mapping
+// it again costs each call ~0.4 ms, at times tens of ms.)
+static int upload_ids(const int32_t *env_ids, int32_t count, cudaStream_t st, int *staged, int **out) {
   *out = nullptr;
   if (!env_ids) return 0;
-  CU(cudaMallocAsync((void **)out, (size_t)count * sizeof(int), st));
+  *out = staged;
+  if (!staged) CU(cudaMallocAsync((void **)out, (size_t)count * sizeof(int), st));
   CU(cudaMemcpyAsync(*out, env_ids, (size_t)count * sizeof(int), cudaMemcpyHostToDevice, st));
   return 0;
 }
 
-// Device staging for records in host memory (the device is idle when this is called).
+// Device staging for records in host memory and for the ids of synchronous calls (the device is idle when this is
+// called).
 static int snap_staging(te_handle *h, size_t bytes) {
   if (bytes > h->snap_cap) {
     h->snap_cap = 0;
@@ -1121,8 +1016,11 @@ static int snap_staging(te_handle *h, size_t bytes) {
   return 0;
 }
 
-extern "C" int te_save_envs(te_handle *h, const int32_t *env_ids, int32_t count, void *records, int memspace, void *stream) {
-  if (int rc = snap_check_args(h, "te_save_envs", env_ids, count, records, memspace, false)) return rc;
+// te_save_envs, and te_get_state / te_set_state, which read and patch host records; `who` names the caller's entry
+// point in every error message.
+static int save_records(te_handle *h, const char *who, const int32_t *env_ids, int32_t count, void *records, int memspace,
+                        void *stream) {
+  if (int rc = snap_check_args(h, who, env_ids, count, records, memspace, false)) return rc;
   if (count == 0) return 0;
   CU(cudaSetDevice(h->device));
   unsigned blocks = 0;
@@ -1130,17 +1028,19 @@ extern "C" int te_save_envs(te_handle *h, const int32_t *env_ids, int32_t count,
   const size_t bytes = (size_t)count * a.L.stride;
   cudaStream_t st = pick_stream(h, stream);
   unsigned char *dst = (unsigned char *)records;
-  if (memspace == TE_HOST) {   // like te_get_state: steps may be queued on caller-provided streams
+  int *staged_ids = nullptr;
+  if (memspace == TE_HOST) {   // steps may be queued on caller-provided streams
     CU(cudaDeviceSynchronize());
     st = h->stream.get();
-    if (int rc = snap_staging(h, bytes)) return rc;
+    if (int rc = snap_staging(h, bytes + (env_ids ? (size_t)count * sizeof(int) : 0))) return rc;   // records | ids
     dst = h->d_snap.get();
+    staged_ids = reinterpret_cast<int *>(dst + bytes);
   }
   int *d_ids = nullptr;
-  if (int rc = upload_ids(env_ids, count, st, &d_ids)) return rc;
+  if (int rc = upload_ids(env_ids, count, st, staged_ids, &d_ids)) return rc;
   te_snap_save_kernel<<<blocks, SNAP_THREADS, 0, st>>>(h->base, a, d_ids, dst);
   CU(cudaGetLastError());
-  if (d_ids) CU(cudaFreeAsync(d_ids, st));
+  if (d_ids && !staged_ids) CU(cudaFreeAsync(d_ids, st));
   if (memspace == TE_HOST) {
     CU(cudaMemcpyAsync(records, dst, bytes, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
@@ -1148,10 +1048,10 @@ extern "C" int te_save_envs(te_handle *h, const int32_t *env_ids, int32_t count,
   return 0;
 }
 
-extern "C" int te_load_envs(te_handle *h, const int32_t *env_ids, int32_t count, const void *records, int memspace,
-                            void *stream) {
-  (void)stream;   // synchronous: the records are checked before anything is written
-  if (int rc = snap_check_args(h, "te_load_envs", env_ids, count, records, memspace, true)) return rc;
+// te_load_envs and te_set_state: synchronous, the records are checked before anything is written.
+static int load_records(te_handle *h, const char *who, const int32_t *env_ids, int32_t count, const void *records,
+                        int memspace) {
+  if (int rc = snap_check_args(h, who, env_ids, count, records, memspace, true)) return rc;
   if (count == 0) return 0;
   CU(cudaSetDevice(h->device));
   CU(cudaDeviceSynchronize());   // steps queued on caller-provided streams have finished with the state
@@ -1160,8 +1060,9 @@ extern "C" int te_load_envs(te_handle *h, const int32_t *env_ids, int32_t count,
   const size_t bytes = (size_t)count * a.L.stride;
   cudaStream_t st = h->stream.get();
   const unsigned char *src = (const unsigned char *)records;
+  const size_t ids_at = memspace == TE_HOST ? bytes : 0;   // staging: host records, then ids
+  if (int rc = snap_staging(h, ids_at + (env_ids ? (size_t)count * sizeof(int) : 0))) return rc;
   if (memspace == TE_HOST) {
-    if (int rc = snap_staging(h, bytes)) return rc;
     CU(cudaMemcpyAsync(h->d_snap.get(), records, bytes, cudaMemcpyHostToDevice, st));
     src = h->d_snap.get();
   }
@@ -1177,20 +1078,109 @@ extern "C" int te_load_envs(te_handle *h, const int32_t *env_ids, int32_t count,
                                        "lastcar", "row header (top byte)", "phase", "passed_dst"};
     const long long j = (long long)(status.first_bad >> 4);
     const unsigned field = (unsigned)(status.first_bad & 15);
-    return fail("te_load_envs: record %lld (for env %d): bad %s; no env was changed", j, env_ids ? env_ids[j] : (int)j,
+    return fail("%s: record %lld (for env %d): bad %s; no env was changed", who, j, env_ids ? env_ids[j] : (int)j,
                 field < sizeof(what) / sizeof(what[0]) ? what[field] : "field");
   }
   int *d_ids = nullptr;
-  if (int rc = upload_ids(env_ids, count, st, &d_ids)) return rc;
+  if (int rc = upload_ids(env_ids, count, st, reinterpret_cast<int *>(h->d_snap.get() + ids_at), &d_ids)) return rc;
   te_snap_load_kernel<<<blocks, SNAP_THREADS, 0, st>>>(h->base, a, d_ids, src);
   CU(cudaGetLastError());
-  if (d_ids) CU(cudaFreeAsync(d_ids, st));
   CU(cudaStreamSynchronize(st));
-  if (status.wild && h->tame) {   // as te_set_state: from now on the checked, one-env-per-CTA kernels
+  if (status.wild && h->tame) {   // from now on: the kernels with the per-car validity predicate, one env per CTA
     h->tame = false;
     if (int rc = select_layout(h)) return rc;
   }
   return 0;
+}
+
+extern "C" int te_save_envs(te_handle *h, const int32_t *env_ids, int32_t count, void *records, int memspace, void *stream) {
+  return save_records(h, "te_save_envs", env_ids, count, records, memspace, stream);
+}
+
+extern "C" int te_load_envs(te_handle *h, const int32_t *env_ids, int32_t count, const void *records, int memspace,
+                            void *stream) {
+  (void)stream;
+  return load_records(h, "te_load_envs", env_ids, count, records, memspace);
+}
+
+// te_get_state / te_set_state: the reference's view of envs [env_begin, env_begin + count), decoded from and encoded
+// into their snapshot records on the host.
+extern "C" int te_get_state(te_handle *h, int32_t env_begin, int32_t count, int32_t *leading, int32_t *lastcar, float *x,
+                            float *v, int32_t *obs, int32_t *waiting, uint8_t *passed_dst, float *steps) {
+  if (!h) return fail("te_get_state: null handle");
+  if (env_begin < 0 || count < 0 || env_begin + count > h->cfg.num_envs) return fail("te_get_state: env range out of bounds");
+  const SnapLayout L = snap_layout_of(h);
+  std::vector<int32_t> ids(count);
+  std::iota(ids.begin(), ids.end(), env_begin);
+  std::vector<unsigned char> recs((size_t)count * L.stride);
+  if (int rc = save_records(h, "te_get_state", ids.data(), count, recs.data(), TE_HOST, nullptr)) return rc;
+  const int R = h->R, r = h->r, I = h->I, ol = 2 * r + 2 * I;
+  for (int e = 0; e < count; e++) {
+    const unsigned char *rec = recs.data() + (size_t)e * L.stride;
+    for (int rd = 0; rd < R; rd++) {
+      const unsigned char *xr = rec + L.x + rd * CAP * 4, *vr = rec + L.v + rd * CAP * 4;
+      const size_t er = (size_t)e * R + rd;
+      uint32_t w0; memcpy(&w0, xr, 4);
+      int wt; memcpy(&wt, vr, 4);
+      const RowHeader m = unpack_meta(w0);
+      if (leading) leading[er] = m.leading;
+      if (lastcar) lastcar[er] = m.lastcar;
+      if (obs && rd < r) { obs[(size_t)e * ol + rd] = 0; obs[(size_t)e * ol + r + rd] = m.detected; }
+      if (waiting && rd < r) waiting[(size_t)e * r + rd] = wt;
+      if (x) { memcpy(&x[er * CAP], xr, CAP * 4); x[er * CAP] = NAN; }
+      if (v) { memcpy(&v[er * CAP], vr, CAP * 4); v[er * CAP] = NAN; }
+    }
+    for (int i = 0; i < I; i++) {
+      int el; memcpy(&el, rec + L.elapsed + 4 * i, 4);
+      if (obs) { obs[(size_t)e * ol + 2 * r + i] = rec[L.phase + i]; obs[(size_t)e * ol + 2 * r + I + i] = el; }
+      if (passed_dst) passed_dst[(size_t)e * I + i] = rec[L.passed_dst + i];
+    }
+    if (steps) memcpy(&steps[e], rec + L.scalars + offsetof(EnvScalars, steps), 4);
+  }
+  return 0;
+}
+
+// Saves the range, overwrites what the caller gives and loads the records back: the rest of each env (birth ticks,
+// arrival-stream position, clocks, return statistics) is kept, and the load's check pass decides whether a car is wild.
+extern "C" int te_set_state(te_handle *h, int32_t env_begin, int32_t count, const int32_t *leading, const int32_t *lastcar,
+                            const float *x, const float *v, const int32_t *obs, const int32_t *waiting,
+                            const uint8_t *passed_dst, const float *steps) {
+  if (!h) return fail("te_set_state: null handle");
+  if (env_begin < 0 || count < 0 || env_begin + count > h->cfg.num_envs) return fail("te_set_state: env range out of bounds");
+  if (!leading || !lastcar || !x || !v || !obs || !waiting || !passed_dst) return fail("te_set_state: all state arrays are required");
+  const int R = h->R, r = h->r, I = h->I, ol = 2 * r + 2 * I;
+  for (int e = 0; e < count; e++)   // every check before anything is written
+    for (int rd = 0; rd < R; rd++) {
+      const int ld = leading[(size_t)e * R + rd], lc = lastcar[(size_t)e * R + rd];
+      if (ld < 1 || ld >= CAP || lc < 1 || lc >= CAP)
+        return fail("te_set_state: ring index out of range (env %d, road %d)", env_begin + e, rd);
+      const int det = rd < r ? obs[(size_t)e * ol + r + rd] : 0;
+      if (det < 0 || det > 255)   // a byte of the row header word
+        return fail("te_set_state: env %d road %d: detected = %d is outside [0, 255]", env_begin + e, rd, det);
+    }
+  const SnapLayout L = snap_layout_of(h);
+  std::vector<int32_t> ids(count);
+  std::iota(ids.begin(), ids.end(), env_begin);
+  std::vector<unsigned char> recs((size_t)count * L.stride);
+  if (int rc = save_records(h, "te_set_state", ids.data(), count, recs.data(), TE_HOST, nullptr)) return rc;
+  for (int e = 0; e < count; e++) {
+    unsigned char *rec = recs.data() + (size_t)e * L.stride;
+    for (int rd = 0; rd < R; rd++) {
+      unsigned char *xr = rec + L.x + rd * CAP * 4, *vr = rec + L.v + rd * CAP * 4;
+      const size_t er = (size_t)e * R + rd;
+      const uint32_t w0 = pack_meta(leading[er], lastcar[er], rd < r ? obs[(size_t)e * ol + r + rd] : 0);
+      const int wt = rd < r ? waiting[(size_t)e * r + rd] : 0;
+      memcpy(xr, &w0, 4); memcpy(xr + 4, &x[er * CAP + 1], (CAP - 1) * 4);
+      memcpy(vr, &wt, 4); memcpy(vr + 4, &v[er * CAP + 1], (CAP - 1) * 4);
+    }
+    for (int i = 0; i < I; i++) {
+      rec[L.phase + i] = obs[(size_t)e * ol + 2 * r + i] != 0;
+      memcpy(rec + L.elapsed + 4 * i, &obs[(size_t)e * ol + 2 * r + I + i], 4);
+      rec[L.passed_dst + i] = passed_dst[(size_t)e * I + i] != 0;
+    }
+    if (steps) memcpy(rec + L.scalars + offsetof(EnvScalars, steps), &steps[e], 4);
+  }
+  return load_records(h, "te_set_state", ids.data(), count, recs.data(), TE_HOST);
 }
 
 extern "C" int te_tame_speed_cap(const float *archetype, float rate, float length, float *v_cap) {

@@ -1146,7 +1146,7 @@ enum : int { SNAP_BAD_MAGIC = 0, SNAP_BAD_VERSION, SNAP_BAD_DIMS, SNAP_BAD_VALID
              SNAP_BAD_HEADER, SNAP_BAD_PHASE, SNAP_BAD_PASSED_DST };
 struct SnapStatus {
   unsigned long long first_bad;   // ~0: every record passed
-  unsigned int wild;              // some live car or leading slot is outside the tame domain (te_set_state's predicate)
+  unsigned int wild;              // some live car or leading slot is outside the tame domain (tame_car / tame_leader)
   unsigned int pad;
 };
 struct SnapArgs {
@@ -1225,11 +1225,13 @@ __global__ void __launch_bounds__(SNAP_THREADS) te_snap_save_kernel(const StepPa
   }
 }
 
-// te_set_state's tame predicate (te_api.cu: tame_car and the leading-slot rule), on the device
-__device__ __forceinline__ bool snap_tame_car(float x, float v, float v_cap) {
+// The tame-car rule (te_math.cuh, idm_update), its one definition: the check pass of every load (te_load_envs,
+// te_set_state) applies it.  x = -0 is not tame: the tame kernels move a car with dx <= 0 by keeping x, where the
+// reference adds +-0.
+__device__ __forceinline__ bool tame_car(float x, float v, float v_cap) {
   return isfinite(x) && fabsf(x) < 0x1p40f && __float_as_uint(x) != 0x80000000u && isfinite(v) && (v == 0.f ? !signbit(v) : (v >= 0x1p-100f && v <= v_cap));
 }
-__device__ __forceinline__ bool snap_tame_leader(float x) {
+__device__ __forceinline__ bool tame_leader(float x) {
   return x == __int_as_float(0x7f800000) || (isfinite(x) && fabsf(x) < 0x1p40f);
 }
 
@@ -1262,8 +1264,8 @@ __global__ void __launch_bounds__(SNAP_THREADS) te_snap_check_kernel(const StepP
           if (s == 0) continue;                  // the header word
           int d = s - ld;
           if (d < 0) d += RING;                  // ring distance behind the leading slot: 0 = leading, 1..cnt = live cars
-          if (d == 0) wild |= !snap_tame_leader(xs[t]);
-          else if (d <= cnt) wild |= !snap_tame_car(xs[t], vs[t], a.v_cap);
+          if (d == 0) wild |= !tame_leader(xs[t]);
+          else if (d <= cnt) wild |= !tame_car(xs[t], vs[t], a.v_cap);
         }
       }
     } else if (it < nq + p.I) {
