@@ -134,13 +134,18 @@ int te_set_arrivals(te_handle *h, const int64_t *offsets, const int16_t *roads, 
    of an env stops after the tick that overflowed.  TE_DEVICE: one kernel launch on `stream`, asynchronous.
    TE_HOST: synchronous; the batch is launched in slices; each finished slice's results travel to the host as compact
    wire records (see te_step_wire) while the next slices run, and helper threads of the handle expand them into the
-   caller's arrays (TE_HOST_SLICES / TE_HOST_THREADS environment variables tune slices and threads). */
+   caller's arrays (TE_HOST_SLICES / TE_HOST_THREADS environment variables tune slices and threads).  Steps of more
+   than 13 ticks (too long for a record), and every step of a handle with host_float_dma set (te_wire_layout), travel
+   instead as float arrays that the copy engine writes into the caller's arrays. */
 int te_step(te_handle *h, const uint8_t *actions, int32_t k_ticks, float *obs, float *reward, uint8_t *done,
             int memspace, void *stream);
 
 /* te_step for a SUBSET of the envs: envs whose env_mask byte is zero are not stepped - their state, arrival stream and
    rows of obs / reward / done stay untouched.  For learners that step their env slots at different times (A3C worker
-   threads, a3c.py:66-72: traffic_env_b200.pool.EnvPool steps whichever slots have an action ready). */
+   threads, a3c.py:66-72: traffic_env_b200.pool.EnvPool steps whichever slots have an action ready).  TE_HOST: steps of
+   up to 13 ticks travel as wire records and only the stepped envs' are expanded; longer ones travel as float arrays into
+   a page-locked staging of the handle (grown to E * (8r + 12I + 1) bytes and kept), from which the stepped envs' rows
+   are copied to the caller's arrays. */
 int te_step_masked(te_handle *h, const uint8_t *actions, const uint8_t *env_mask, int32_t k_ticks, float *obs, float *reward,
                    uint8_t *done, int memspace, void *stream);
 
@@ -271,6 +276,26 @@ int te_is_tame(const te_handle *h, int32_t *tame, float *v_cap);
 /* The speed cap of the tame domain for an archetype / tick length / road length, 0 when the archetype is outside the
    supported ranges (host arithmetic only: needs no device). */
 int te_tame_speed_cap(const float *archetype, float rate, float length, float *v_cap);
+
+/* Which instantiation of the step kernel, te_step_kernel<MAXT, MINB, VALIDATE, TAME, GROUPED>, runs a configuration.
+   max_threads = MAXT, the row capacity of a CTA; min_blocks = MINB, the CTAs per SM its register cap is set for;
+   validate: compiled for TE_VALIDATE (birth-tick plane); tame: compiled without the per-car validity predicate and
+   generic fallback (te_is_tame); grouped: several env instances per CTA.  The layout: roads R of one env, roads_padded
+   (its rows in HBM), envs_per_cta G and threads per CTA (G * R rounded up to whole warps, or roads_padded when G = 1). */
+typedef struct te_step_variant_t {
+  int32_t max_threads, min_blocks, validate, tame, grouped;
+  int32_t roads, roads_padded, envs_per_cta, threads; /* 0 in te_step_variants */
+} te_step_variant_t;
+/* The compiled instantiations: *count receives their number, the first min(cap, *count) are written to out (NULL when
+   cap = 0).  Needs no device. */
+int te_step_variants(te_step_variant_t *out, int32_t cap, int32_t *count);
+/* What te_create picks for cfg (the same rules, in one place), and with wild = 1 what the handle runs once a wild car
+   has been loaded (te_is_tame).  Fails where te_create fails for the configuration itself (not for the device), e.g.
+   for grids too large for one CTA, or for the validate-mode kernels (the message names the largest variant).  Needs no
+   device. */
+int te_plan_step_variant(const te_config *cfg, int32_t wild, te_step_variant_t *out);
+/* What a handle runs now; changes when a wild car moves it to the checked kernels. */
+int te_get_step_variant(const te_handle *h, te_step_variant_t *out);
 
 /* Counters since te_create (device -> host; synchronises the device). */
 int te_get_stats(te_handle *h, te_stats *out);

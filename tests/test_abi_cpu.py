@@ -79,3 +79,24 @@ def test_idm_peak_form_rejects_unknown_forms():
         msg = L.te_last_error().decode()
         assert "form %d" % form in msg and "-1 = " in msg and "0 = general" in msg and "5 = tame" in msg, msg
         assert out.value == -1.0
+
+
+def test_step_variant_queries_need_no_device():
+    """te_step_variants and te_plan_step_variant answer from the host tables; te_get_step_variant needs a handle."""
+    from traffic_env_b200 import _lib
+    L = _lib.load()
+    n = C.c_int32(-1)
+    assert L.te_step_variants(None, 0, C.byref(n)) == 0 and n.value == 19
+    assert L.te_step_variants(None, 1, C.byref(n)) < 0
+    two = (_lib.TeStepVariant * 2)()
+    assert L.te_step_variants(two, 2, C.byref(n)) == 0 and n.value == 19 and two[1].max_threads > 0
+    out = _lib.TeStepVariant()
+    cfg = _lib.default_config()
+    assert L.te_plan_step_variant(C.byref(cfg), 0, C.byref(out)) == 0
+    assert (out.max_threads, out.min_blocks, out.tame, out.grouped, out.envs_per_cta, out.threads) == (96, 10, 1, 1, 2, 96)
+    assert L.te_plan_step_variant(C.byref(cfg), 1, C.byref(out)) == 0
+    assert (out.max_threads, out.tame, out.grouped, out.envs_per_cta, out.threads) == (64, 0, 0, 1, 64)
+    assert L.te_plan_step_variant(None, 0, C.byref(out)) < 0
+    cfg.struct_size = 8
+    assert L.te_plan_step_variant(C.byref(cfg), 0, C.byref(out)) < 0 and "size mismatch" in L.te_last_error().decode()
+    assert L.te_get_step_variant(None, C.byref(out)) < 0 and "null argument" in L.te_last_error().decode()

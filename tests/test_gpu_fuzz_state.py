@@ -41,7 +41,8 @@ def random_env_state(rng, R, r, I, L, dense):
     return dict(leading=leading, lastcar=lastcar, x=x, v=v, obs=obs, waiting=waiting, passed_dst=passed_dst)
 
 
-def load_oracle(o, st):
+def load_oracle(o, st, arch=ARCH):
+    """The state `st` (random_env_state) into OracleEnv `o`, whose cars have the archetype `arch` (the handle's)."""
     R = o.roads
     o.leading[:] = st["leading"]
     o.lastcar[:] = st["lastcar"]
@@ -52,7 +53,7 @@ def load_oracle(o, st):
         o.state[e, 0, s] = st["x"][e, s]
         while s != int(st["lastcar"][e]):
             s = 1 if s + 1 >= CAP else s + 1
-            o.state[e, :, s] = ARCH
+            o.state[e, :, s] = arch
             o.state[e, 0, s] = st["x"][e, s]
             o.state[e, 1, s] = st["v"][e, s]
     o.obs[:] = st["obs"]
@@ -60,18 +61,35 @@ def load_oracle(o, st):
     o.passed_dst[:] = st["passed_dst"]
 
 
-@pytest.mark.parametrize("m,n,L,E,dense,ordered", [
+FUZZ_ROWS = [
     (3, 3, 250.0, 96, True, False), (3, 3, 250.0, 96, False, False), (3, 3, 250.0, 64, True, True),
     (2, 3, 100.0, 64, True, False), (1, 1, 60.0, 32, True, False), (10, 10, 500.0, 6, True, False),
     (4, 2, 80.0, 48, False, True), (3, 2, 123.456, 64, True, False), (2, 2, 77.7, 48, True, False),
-    # one grid per kernel variant (row capacity 128 / 128 with Rp = 96 / 256 / 512 / 768 / 1024)
+    # one grid per tame kernel variant: tame 128 / grouped 160 / tame 256 / 512 / 768 / 1024
     (5, 5, 150.0, 8, True, False), (4, 4, 90.0, 8, True, False), (7, 7, 120.0, 4, True, False),
-    (10, 11, 100.0, 3, True, False), (13, 13, 100.0, 2, True, False), (15, 15, 100.0, 2, False, False)])
+    (10, 11, 100.0, 3, True, False), (13, 13, 100.0, 2, True, False), (15, 15, 100.0, 2, False, False),
+    # tame 64 (one env per CTA: sharing a CTA would save no lanes); grouped 256 with G = 4 and a last CTA holding two
+    # envs; grouped 64 with G = 3 and a last CTA holding one env
+    (4, 3, 90.0, 20, True, False), (2, 5, 80.0, 30, True, False), (1, 3, 70.0, 31, True, False)]
+# the step-kernel instantiation (kind, MAXT) each grid of FUZZ_ROWS runs
+FUZZ_VARIANTS = {(3, 3): ("grouped", 96), (2, 3): ("grouped", 160), (1, 1): ("grouped", 64), (10, 10): ("tame", 512),
+                 (4, 2): ("grouped", 96), (3, 2): ("grouped", 160), (2, 2): ("grouped", 96), (5, 5): ("tame", 128),
+                 (4, 4): ("grouped", 160), (7, 7): ("tame", 256), (10, 11): ("tame", 512), (13, 13): ("tame", 768),
+                 (15, 15): ("tame", 1024), (4, 3): ("tame", 64), (2, 5): ("grouped", 256), (1, 3): ("grouped", 64)}
+
+
+def variant_of(env):
+    v = env.step_variant()
+    return v["kind"], v["max_threads"]
+
+
+@pytest.mark.parametrize("m,n,L,E,dense,ordered", FUZZ_ROWS)
 def test_random_states_tick_by_tick(m, n, L, E, dense, ordered):
     from traffic_env_b200 import VecTrafficEnv
     rng = np.random.RandomState(1000 * m + 10 * n + int(dense) + 2 * int(ordered))
     T = 4
     env = VecTrafficEnv(m=m, n=n, length=L, num_envs=E, arrivals="injected", remi=False, ordered_transfers=ordered)
+    assert variant_of(env) == FUZZ_VARIANTS[(m, n)]
     R, r, I = env.roads, env.train_roads, env.intersections
     states = [random_env_state(rng, R, r, I, L, dense) for _ in range(E)]
     scheds = [[list(rng.choice(env.entrypoints, size=rng.randint(0, 4))) for _ in range(T)] for _ in range(E)]
@@ -109,6 +127,7 @@ def test_random_states_tick_by_tick(m, n, L, E, dense, ordered):
             gx, gv = live_walk(st["leading"][e], st["lastcar"][e], st["x"][e], st["v"][e])
             ox, ov = o.live_state()
             assert gx.tobytes() == ox.tobytes() and gv.tobytes() == ov.tobytes(), tag + " car state"
+    assert env.is_tame() and variant_of(env) == FUZZ_VARIANTS[(m, n)]
     stats = env.stats()
     assert stats["overflows"] == sum(o.overflows for o in oracles)
     assert stats["vehicle_updates"] == sum(o.vehicle_updates for o in oracles)

@@ -7,24 +7,32 @@ import pytest
 
 from oracle.oracle import OracleEnv
 from tests.golden_util import live_walk
-from tests.test_gpu_fuzz_state import load_oracle, random_env_state
+from tests.test_gpu_fuzz_state import load_oracle, random_env_state, variant_of
 
 pytestmark = pytest.mark.gpu
 
+# x, v, l, a, delta, v0, b, T, s0, w
+ARCH_ODD = [0.0, 9.5, 4.5, 2.2, 3.5, 15.3, 4.1, 1.7, 1.5, 0.0]        # nothing a power of two, delta != 4
+ARCH_DELTA4 = [0.0, 11.11, 4.0, 3.0, 4.0, 13.89, 6.0, 1.3, 1.0, 0.0]  # delta == 4 but T (and the rates used) not powers of two
+ARCH_POW2 = [0.0, 12.0, 5.0, 1.5, 2.0, 17.0, 3.0, 2.0, 2.0, 0.0]      # T, rate powers of two, delta != 4
+NONDEFAULT_ARCH_ROWS = [
+    (ARCH_ODD, 0.4, 3, 3, 250.0, 0.25, 24), (ARCH_DELTA4, 0.3, 2, 3, 140.0, 0.4, 24), (ARCH_POW2, 0.5, 4, 4, 200.0, 0.2, 24),
+    # the checked 256 / 768 / 1024 kernels, a few envs each
+    (ARCH_ODD, 0.4, 7, 7, 200.0, 0.25, 4), (ARCH_DELTA4, 0.3, 13, 13, 140.0, 0.4, 2), (ARCH_ODD, 0.4, 15, 15, 150.0, 0.25, 2)]
+NONDEFAULT_ARCH_VARIANTS = {(3, 3): ("checked", 64), (2, 3): ("checked", 64), (4, 4): ("checked", 128),
+                            (7, 7): ("checked", 256), (13, 13): ("checked", 768), (15, 15): ("checked", 1024)}
 
-@pytest.mark.parametrize("arch,rate,m,n,L,lcps", [
-    # x, v, l, a, delta, v0, b, T, s0, w
-    ([0.0, 9.5, 4.5, 2.2, 3.5, 15.3, 4.1, 1.7, 1.5, 0.0], 0.4, 3, 3, 250.0, 0.25),     # nothing a power of two, delta != 4
-    ([0.0, 11.11, 4.0, 3.0, 4.0, 13.89, 6.0, 1.3, 1.0, 0.0], 0.3, 2, 3, 140.0, 0.4),   # delta == 4 but T, rate not powers of two
-    ([0.0, 12.0, 5.0, 1.5, 2.0, 17.0, 3.0, 2.0, 2.0, 0.0], 0.5, 4, 4, 200.0, 0.2),     # T, rate powers of two, delta != 4
-])
-def test_nondefault_archetype_trajectories(arch, rate, m, n, L, lcps):
+
+@pytest.mark.parametrize("arch,rate,m,n,L,lcps,E", NONDEFAULT_ARCH_ROWS)
+def test_nondefault_archetype_trajectories(arch, rate, m, n, L, lcps, E):
     from traffic_env_b200 import VecTrafficEnv
     from traffic_env_b200.arrivals import gap_cdf
-    E, K, S = 24, 10, 45
+    K, S = 10, 45
     arch = np.asarray(arch, np.float32)
     env = VecTrafficEnv(m=m, n=n, length=L, num_envs=E, rate=rate, arrivals="philox", seed=77, local_cars_per_sec=lcps,
                         ticks_per_step=K, remi=True, archetype=arch)
+    # (is_tame() may hold: an archetype inside the tame ranges still runs the checked form unless it is the reference's)
+    assert variant_of(env) == NONDEFAULT_ARCH_VARIANTS[(m, n)]
     rng = np.random.RandomState(5)
     I = m * n
     init = rng.randint(2, size=(E, I))
@@ -409,7 +417,17 @@ def test_multi_step_argument_errors():
     assert o.shape == (8, 81)
 
 
-@pytest.mark.parametrize("m,n,L,E", [(3, 3, 250.0, 66), (10, 10, 120.0, 6), (1, 1, 60.0, 8)])
+WILD_CAR_ROWS = [(3, 3, 250.0, 66), (10, 10, 120.0, 6), (1, 1, 60.0, 8),
+                 # the checked 64 / 256 / 768 / 1024 kernels with the reference's archetype (pow2 and powf4 shortcuts on)
+                 (4, 3, 90.0, 12), (7, 7, 120.0, 4), (13, 13, 100.0, 2), (15, 15, 100.0, 2)]
+# (kind, MAXT) of the step kernel before and after the wild cars
+WILD_CAR_VARIANTS = {(3, 3): (("grouped", 96), ("checked", 64)), (10, 10): (("tame", 512), ("checked", 512)),
+                     (1, 1): (("grouped", 64), ("checked", 64)), (4, 3): (("tame", 64), ("checked", 64)),
+                     (7, 7): (("tame", 256), ("checked", 256)), (13, 13): (("tame", 768), ("checked", 768)),
+                     (15, 15): (("tame", 1024), ("checked", 1024))}
+
+
+@pytest.mark.parametrize("m,n,L,E", WILD_CAR_ROWS)
 def test_wild_car_moves_the_handle_to_the_checked_kernels(m, n, L, E):
     """A handle runs the kernels without the per-car validity predicate only while every car it was ever given is tame
     (te_is_tame, include/traffic_b200.h).  Tame random states first (is_tame stays set, two shared-CTA envs per CTA on
@@ -440,6 +458,7 @@ def test_wild_car_moves_the_handle_to_the_checked_kernels(m, n, L, E):
         env.set_arrivals(scheds, first_tick=T if wild else 0)     # (the envs' arrival clocks are at T after the first pass)
         env.set_state({k: np.stack([s[k] for s in states]) for k in states[0]} | {"steps": np.zeros(E, np.float32)})
         assert env.is_tame() == (not wild)
+        assert variant_of(env) == WILD_CAR_VARIANTS[(m, n)][int(wild)]
         oracles = []
         for e in range(E):
             o = OracleEnv(m, n, L, 0.5)
@@ -463,10 +482,15 @@ def test_wild_car_moves_the_handle_to_the_checked_kernels(m, n, L, E):
     assert not env.is_tame()
 
 
-@pytest.mark.parametrize("m,n,L,E,lcps,extra", [
+CONTROLLER_ROWS = [
     (3, 3, 250.0, 301, 0.5, {}), (10, 10, 500.0, 6, 0.3, {}), (2, 2, 120.0, 77, 0.9, {}), (4, 4, 150.0, 33, 0.4, {}),
     (3, 3, 250.0, 65, 0.5, {"learn_switch": True}), (3, 3, 250.0, 40, 0.15, {"validate": True}), (3, 3, 250.0, 50, 0.5, {"remi": False}),
-    (3, 3, 250.0, 64, 0.12, {"ticks_per_step": 4})])
+    (3, 3, 250.0, 64, 0.12, {"ticks_per_step": 4}),
+    # a non-tame archetype: the decisions are taken inside the checked 256 kernel
+    (7, 7, 150.0, 6, 0.9, {"archetype": ARCH_ODD, "rate": 0.4})]
+
+
+@pytest.mark.parametrize("m,n,L,E,lcps,extra", CONTROLLER_ROWS)
 def test_controller_decisions_inside_a_launch(m, n, L, E, lcps, extra):
     """te_set_controller_spacing: one te_step_multi launch that holds several greedy decisions (a new one every
     `spacing` actor steps, evaluated in the kernel on the live rings) produces exactly what one launch per decision
@@ -484,6 +508,8 @@ def test_controller_decisions_inside_a_launch(m, n, L, E, lcps, extra):
     init = np.random.RandomState(5).randint(2, size=(E, I))
     for env in (a, b, d, w):
         env.reset(init_phase=init)
+    if "archetype" in extra:
+        assert variant_of(a) == ("checked", 256)
     dev = torch.device("cuda", 0)
     NMAX = 64 // K
     d_act = torch.zeros((NMAX, E, I), dtype=torch.uint8, device=dev)

@@ -1,7 +1,8 @@
 """Every route the results of a step with host buffers can take (te_api.cu: pick_route) gives, bit for bit, what the
 same step gives on a handle stepped with device buffers: wire records expanded by the handle's threads, float arrays
-written by the copy engine (TE_HOST_FLOAT_DMA=1), steps too long for a record (k_ticks > 13), masked steps, and the
-records themselves - launched in one slice or in several (TE_HOST_SLICES)."""
+written by the copy engine (TE_HOST_FLOAT_DMA=1), steps too long for a record (k_ticks > 13), masked steps on both
+routes (the rows of envs not stepped keep what the caller's arrays held, on a fresh handle too), and the records
+themselves - launched in one slice or in several (TE_HOST_SLICES)."""
 import os
 
 import numpy as np
@@ -58,15 +59,34 @@ def test_host_routes_equal_device_buffers(float_dma, slices):
         for g, w, name in zip(got, want, ("obs", "reward", "done")):
             assert np.ascontiguousarray(g).tobytes() == np.ascontiguousarray(w).tobytes(), (what, name)
 
+    def full(k, what):
+        act = rng.randint(2, size=(E, I)).astype(np.uint8)
+        got = h.step(act, k=k)
+        d_act[0].copy_(torch.from_numpy(act))
+        d.step_device(d_act[0], d_obs[0], d_rew[0], d_done[0], k=k)
+        same(got, (w[0] for w in device_out(1)), (what, "step k=%d" % k))
+
+    def masked(k, what):
+        act = rng.randint(2, size=(E, I)).astype(np.uint8)
+        mask = rng.rand(E) < 0.5
+        h._obs[:] = -7.25                      # what the rows of the envs that are not stepped must keep
+        h._reward[:] = 99.5
+        h._done[:] = 7
+        obs, rew, done = h.step_masked(act, mask, k=k)
+        d_act[0].copy_(torch.from_numpy(act))
+        d_mask = torch.from_numpy(mask.astype(np.uint8)).to(dev)
+        check(d._L.te_step_masked(d._h, d_act[0].data_ptr(), d_mask.data_ptr(), k, d_obs.data_ptr(), d_rew.data_ptr(),
+                                  d_done.data_ptr(), TE_DEVICE, None))
+        want = device_out(1)
+        same((obs[mask], rew[mask], done[mask]), (w[0][mask] for w in want), (what, "step_masked k=%d" % k))
+        assert (obs[~mask] == np.float32(-7.25)).all() and (rew[~mask] == np.float32(99.5)).all() \
+            and (done[~mask] == 7).all(), (what, "step_masked k=%d: rows of envs not stepped" % k)
+
+    masked(20, "first call")                   # the float staging has never been written
     for rnd in range(3):
         tag = "round %d" % rnd
         for k in (10, 20):                     # 20 ticks: too long for a record, the float staging route
-            act = rng.randint(2, size=(E, I)).astype(np.uint8)
-            got = h.step(act, k=k)
-            d_act[0].copy_(torch.from_numpy(act))
-            d.step_device(d_act[0], d_obs[0], d_rew[0], d_done[0], k=k)
-            want = device_out(1)
-            same(got, (w[0] for w in want), (tag, "step k=%d" % k))
+            full(k, tag)
 
         act = rng.randint(2, size=(E, I)).astype(np.uint8)
         _, obs, rew, done = h.step_multi(3, actions=act, controller="given")
@@ -80,19 +100,14 @@ def test_host_routes_equal_device_buffers(float_dma, slices):
         assert act_h.tobytes() == d_act.cpu().numpy().tobytes(), (tag, "greedy actions")
 
         act = rng.randint(2, size=(E, I)).astype(np.uint8)
-        mask = rng.rand(E) < 0.5
-        h._obs[:] = -7.25                      # what the rows of the envs that are not stepped must keep
-        h._reward[:] = 99.5
-        h._done[:] = 7
-        obs, rew, done = h.step_masked(act, mask, k=10)
+        _, obs, rew, done = h.step_multi(3, actions=act, controller="given", k=20)    # the multi-step float route
         d_act[0].copy_(torch.from_numpy(act))
-        d_mask = torch.from_numpy(mask.astype(np.uint8)).to(dev)
-        check(d._L.te_step_masked(d._h, d_act[0].data_ptr(), d_mask.data_ptr(), 10, d_obs.data_ptr(), d_rew.data_ptr(),
-                                  d_done.data_ptr(), TE_DEVICE, None))
-        want = device_out(1)
-        same((obs[mask], rew[mask], done[mask]), (w[0][mask] for w in want), (tag, "step_masked"))
-        assert (obs[~mask] == np.float32(-7.25)).all() and (rew[~mask] == np.float32(99.5)).all() \
-            and (done[~mask] == 7).all(), (tag, "step_masked: rows of envs not stepped")
+        d.step_multi_device(3, d_act[0], d_obs, d_rew, d_done, controller="given", k=20)
+        same((obs, rew, done), device_out(3), (tag, "step_multi given k=20"))
+
+        masked(10, tag)
+        full(10, tag)
+        masked(20, tag)                        # the float route: its staging holds rows of envs this step leaves alone
 
         act = rng.randint(2, size=(E, I)).astype(np.uint8)
         h.step_wire(act, k=10)

@@ -185,7 +185,12 @@ def test_fused_learn_switch_matches_raw_ticks():
     assert checked == 60
 
 
-@pytest.mark.parametrize("m,n,L,E", [(10, 10, 50.0, 3), (6, 5, 90.0, 4)])
+# 11x11: 544 rows in the 768-row validate kernel; 13x13 fills it (14x14 and larger are refused)
+VALIDATE_ROWS = [(10, 10, 50.0, 3), (6, 5, 90.0, 4), (11, 11, 50.0, 2), (13, 13, 50.0, 2)]
+VALIDATE_VARIANTS = {(10, 10): 512, (6, 5): 256, (11, 11): 768, (13, 13): 768}
+
+
+@pytest.mark.parametrize("m,n,L,E", VALIDATE_ROWS)
 def test_validate_mode_larger_grids_vs_oracle(m, n, L, E):
     """TE_VALIDATE on the larger kernel variants (third shared-memory plane): trip times of cars leaving the map
     and the ring state against the oracle in validate mode, injected arrivals, 320 raw ticks."""
@@ -195,6 +200,8 @@ def test_validate_mode_larger_grids_vs_oracle(m, n, L, E):
     rng = np.random.RandomState(100 * m + n)
     T = 320
     env = VecTrafficEnv(m=m, n=n, length=L, num_envs=E, arrivals="injected", remi=False, validate=True)
+    v = env.step_variant()
+    assert (v["kind"], v["max_threads"]) == ("validate", VALIDATE_VARIANTS[(m, n)])
     I = env.intersections
     scheds = [[list(rng.choice(env.entrypoints, size=rng.poisson(1.5))) for _ in range(T)] for _ in range(E)]
     init = rng.randint(2, size=(E, I))

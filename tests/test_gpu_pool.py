@@ -14,9 +14,10 @@ pytestmark = pytest.mark.gpu
 KW = dict(m=3, n=3, length=250.0, arrivals="philox", local_cars_per_sec=0.3, ticks_per_step=10)
 
 
-def rollout(env, slot, seed, steps, out, delay=0.0):
+def rollout(env, slot, seed, steps, out, delay=0.0, k_ticks=10):
     """a3c.epoch restated: obs = env.reset(); y = policy(obs); new_obs, reward, done, _ = env.step(y) - with every
-    observation / reward / done compared, on the spot, with an OracleEnv driven by the same actions."""
+    observation / reward / done compared, on the spot, with an OracleEnv driven by the same actions (k_ticks: the pool's
+    ticks per actor step)."""
     from traffic_env_b200.arrivals import gap_cdf
     rng = np.random.RandomState(100 + slot)
     w = rng.standard_normal((env.observation_space.size, env.action_space.size)).astype(np.float32)
@@ -27,7 +28,7 @@ def rollout(env, slot, seed, steps, out, delay=0.0):
         ph, first = rng.randint(2, size=9), rng.randint(2, size=9)
         obs = env.reset(init_phase=ph, first_action=first)
         o.reset(ph)
-        oo, _, _ = o.actor_step_philox(first, 10, use_remi=True)
+        oo, _, _ = o.actor_step_philox(first, k_ticks, use_remi=True)
         assert obs.tobytes() == oo.tobytes(), "slot %d: reset observation" % slot
         return obs
     try:
@@ -36,7 +37,7 @@ def rollout(env, slot, seed, steps, out, delay=0.0):
         for t in range(steps):
             y = (obs @ w) < 0                      # bool vector, like tf.less in algorithms/util.py:114
             new_obs, reward, done, _ = env.step(y)
-            oo, orw, od = o.actor_step_philox(y, 10, use_remi=True)
+            oo, orw, od = o.actor_step_philox(y, k_ticks, use_remi=True)
             assert new_obs.tobytes() == oo.tobytes() and reward.tobytes() == orw.tobytes() and done == od, \
                 "slot %d diverges from the oracle at step %d" % (slot, t)
             assert new_obs.shape == (81,) and new_obs.dtype == np.float32 and reward.shape == (9,) and y.dtype == np.bool_
@@ -53,11 +54,12 @@ def rollout(env, slot, seed, steps, out, delay=0.0):
         env.close()
 
 
-def run_pool(T, steps, seed, delays=None):
+def run_pool(T, steps, seed, delays=None, k_ticks=10):
     from traffic_env_b200.pool import EnvPool
-    pool = EnvPool(T, seed=seed, **KW)
+    pool = EnvPool(T, seed=seed, **dict(KW, ticks_per_step=k_ticks))
     out = {}
-    threads = [threading.Thread(target=rollout, args=(pool.slot(i), i, seed, steps[i], out, (delays or {}).get(i, 0.0)))
+    threads = [threading.Thread(target=rollout, args=(pool.slot(i), i, seed, steps[i], out, (delays or {}).get(i, 0.0),
+                                                      k_ticks))
                for i in range(T)]
     t0 = time.perf_counter()
     for th in threads:
@@ -74,6 +76,15 @@ def test_every_slot_matches_the_oracle_from_threads():
     T, S = 8, 60
     pool, out, _ = run_pool(T, [S] * T, seed=3)
     # ready slots share launches: fewer launches than single-env steps, every step served
+    assert pool.stepped >= T * S and pool.launches <= pool.stepped
+    assert pool.vec.stats()["actor_steps"] == pool.stepped
+
+
+def test_every_slot_matches_the_oracle_on_the_float_route():
+    """20 ticks per actor step: too long for a wire record, so the pool's masked launches take the float route, which
+    must write no row of a slot it did not step (other slots' threads read theirs meanwhile)."""
+    T, S = 8, 60
+    pool, out, _ = run_pool(T, [S] * T, seed=3, k_ticks=20)
     assert pool.stepped >= T * S and pool.launches <= pool.stepped
     assert pool.vec.stats()["actor_steps"] == pool.stepped
 

@@ -24,7 +24,7 @@ EXPORTS = [
     "te_pool_create", "te_pool_destroy", "te_pool_step", "te_pool_reset", "te_pool_cars", "te_pool_counters", "te_pool_last_error", "te_wire_layout", "te_expand_wire", "te_step_raw", "te_remi_reward", "te_cars_on_roads",
     "te_greedy_actions", "te_get_state", "te_set_state", "te_get_stats", "te_get_trip_times",
     "te_synchronize", "te_host_alloc", "te_host_free", "te_last_kernel_ms", "te_stage_bandwidth", "te_idm_peak_form", "te_test_powf", "te_test_idm", "te_test_idm_tame", "te_is_tame", "te_tame_speed_cap", "te_set_controller_spacing", "te_test_powf4_exhaustive", "te_test_philox",
-    "te_snapshot_layout", "te_save_envs", "te_load_envs",
+    "te_snapshot_layout", "te_save_envs", "te_load_envs", "te_step_variants", "te_plan_step_variant", "te_get_step_variant",
 ]
 
 
@@ -59,6 +59,11 @@ class TeWireLayout(C.Structure):
 
 class TeSnapshotLayout(C.Structure):
     _fields_ = [(k, C.c_int32) for k in ("stride", "x", "v", "w", "phase", "elapsed", "passed_dst", "scalars")]
+
+
+class TeStepVariant(C.Structure):
+    _fields_ = [(k, C.c_int32) for k in ("max_threads", "min_blocks", "validate", "tame", "grouped", "roads", "roads_padded",
+                                            "envs_per_cta", "threads")]
 
 
 class TrafficB200Error(RuntimeError):
@@ -129,6 +134,9 @@ def load():
     L.te_snapshot_layout.argtypes = [vp, C.POINTER(TeSnapshotLayout)]
     L.te_save_envs.argtypes = [vp, vp, i32, vp, C.c_int, vp]
     L.te_load_envs.argtypes = [vp, vp, i32, vp, C.c_int, vp]
+    L.te_step_variants.argtypes = [vp, i32, C.POINTER(i32)]
+    L.te_plan_step_variant.argtypes = [C.POINTER(TeConfig), i32, C.POINTER(TeStepVariant)]
+    L.te_get_step_variant.argtypes = [vp, C.POINTER(TeStepVariant)]
     for name in EXPORTS:
         if name not in ("te_default_config", "te_last_error", "te_pool_last_error"):
             getattr(L, name).restype = C.c_int
@@ -151,6 +159,23 @@ def device_count():
         return int(n.value)
     except Exception:
         return 0
+
+
+def variant_dict(v):
+    """A te_step_variant_t as a dict, with `kind` = "validate" / "grouped" / "tame" / "checked"."""
+    d = {k: int(getattr(v, k)) for k, _ in TeStepVariant._fields_}
+    d["kind"] = "validate" if d["validate"] else "grouped" if d["grouped"] else "tame" if d["tame"] else "checked"
+    return d
+
+
+def step_variants():
+    """Every compiled instantiation of the step kernel (te_step_variants), as variant_dict()s; needs no device."""
+    L = load()
+    n = C.c_int32(0)
+    check(L.te_step_variants(None, 0, C.byref(n)))
+    out = (TeStepVariant * n.value)()
+    check(L.te_step_variants(out, n.value, C.byref(n)))
+    return [variant_dict(v) for v in out]
 
 
 def default_config():

@@ -168,6 +168,8 @@ struct ExpandPool {
   }
 };
 
+struct StepVariant;
+
 // Members go in reverse order of declaration: the helper threads stop before the page-locked records they read are
 // freed, and every event and buffer goes before the streams.
 struct te_handle {
@@ -197,11 +199,16 @@ struct te_handle {
   dev_buf<float> w; dev_buf<TripRecord> d_trips; dev_buf<unsigned long long> d_trip_count; long long trip_cap = 0;
   int warps = 0;
   int G = 1, threads = 0;        // env instances per CTA, threads per CTA (G * R rounded up to whole warps)
+  const StepVariant *sv = nullptr;   // the step kernel the handle runs now (select_layout)
+  te_step_variant_t plan = {};       // the same, as te_get_step_variant reports it
   int smem_optin = 0;
   // wire path of the host API
   dev_buf<unsigned char> d_wire; pinned_buf<unsigned char> h_wire;   // [steps][E][wire_stride] device / page-locked host
   int wire_stride = 0, host_slices = 1;
   int wire_steps = 1, float_steps = 1;   // actor steps the wire records / float staging have room for
+  // masked steps on the float route: page-locked [nsteps][E] obs | reward | done, of which only the stepped envs' rows
+  // are copied to the caller (launch_sliced)
+  pinned_buf<unsigned char> h_float; int h_float_steps = 0;
   bool tame = false;     // every car the device has seen is tame (te_math.cuh: idm_update<TAME = true> may run)
   float v_cap = 0.f;     // speed bound of the tame domain for this archetype (tame_archetype)
   int ctrl_spacing = 0;  // TE_CTRL_GREEDY: a new decision every so many actor steps inside a te_step_multi launch (0: one per launch)
@@ -220,39 +227,46 @@ struct te_handle {
 // should hold: 1024 resident threads per SM at 64 registers wherever shared memory allows it (10x10 grid: 512 threads
 // x 2 CTAs, 101.7 KB each; 3x3 grid: 64 threads x 16 CTAs).
 typedef void (*step_kernel_t)(const StepParams);
-struct StepVariant { step_kernel_t fn; int maxt; };
-// threads = rows of the CTA; tame = the car loop compiled in the tame form (runs_tame_form); grouped = several env
-// instances per CTA (small grids with the reference's archetype, te_create).
-// 20 instantiations of the step kernel: the set is kept small for the sake of build time.
-static StepVariant step_variant_for(int threads, bool validate, bool tame, bool grouped) {
-  if (validate) {  // + the birth-tick plane in shared memory: one CTA fewer per SM
-    if (threads <= 256) return {te_step_kernel<256, 2, true, false, false>, 256};
-    if (threads <= 512) return {te_step_kernel<512, 1, true, false, false>, 512};
-    return {te_step_kernel<768, 1, true, false, false>, 768};
+// te_step_kernel<MAXT, MINB, VALIDATE, TAME, GROUPED>: MAXT rows, MINB CTAs per SM for the register cap; TAME = the car
+// loop compiled in the tame form (runs_tame_form); GROUPED = several env instances per CTA (small grids with the
+// reference's archetype, plan_layout).
+struct StepVariant { step_kernel_t fn; int maxt, minb; bool validate, tame, grouped; };
+#define TE_STEP_VARIANT(MAXT, MINB, VALIDATE, TAME, GROUPED) \
+  {te_step_kernel<MAXT, MINB, VALIDATE, TAME, GROUPED>, MAXT, MINB, VALIDATE, TAME, GROUPED}
+// The 19 instantiations of the step kernel (te_step_variants), in increasing MAXT within each kind: the set is kept
+// small for the sake of build time.
+static const StepVariant STEP_VARIANTS[] = {
+    // validate: + the birth-tick plane in shared memory, one CTA fewer per SM
+    TE_STEP_VARIANT(256, 2, true, false, false), TE_STEP_VARIANT(512, 1, true, false, false),
+    TE_STEP_VARIANT(768, 1, true, false, false),
+    // grouped (only built in the tame form: plan_layout keeps G = 1 otherwise).  Default 3x3 grid: two envs (2 x 48 roads)
+    // on three warps, 20 envs per SM at 64 registers (72 registers and 9 CTAs per SM measured 2.4 % slower).  No grid
+    // yields 97..128 threads at G > 1, so those would run the 160 variant.
+    TE_STEP_VARIANT(64, 16, false, true, true), TE_STEP_VARIANT(96, 10, false, true, true),
+    TE_STEP_VARIANT(160, 6, false, true, true), TE_STEP_VARIANT(256, 4, false, true, true),
+    // tame, one env per CTA
+    TE_STEP_VARIANT(64, 16, false, true, false), TE_STEP_VARIANT(128, 8, false, true, false),
+    TE_STEP_VARIANT(256, 4, false, true, false), TE_STEP_VARIANT(512, 2, false, true, false),
+    TE_STEP_VARIANT(768, 1, false, true, false), TE_STEP_VARIANT(1024, 1, false, true, false),
+    // checked: per-car validity predicate and generic fallback
+    TE_STEP_VARIANT(64, 16, false, false, false), TE_STEP_VARIANT(128, 8, false, false, false),
+    TE_STEP_VARIANT(256, 4, false, false, false), TE_STEP_VARIANT(512, 2, false, false, false),
+    TE_STEP_VARIANT(768, 1, false, false, false), TE_STEP_VARIANT(1024, 1, false, false, false),
+};
+#undef TE_STEP_VARIANT
+static constexpr int NUM_STEP_VARIANTS = (int)(sizeof(STEP_VARIANTS) / sizeof(STEP_VARIANTS[0]));
+// The smallest variant of the kind with room for `threads` rows, else the largest of the kind (the caller compares
+// `threads` with its maxt).  Validate variants are neither tame nor grouped; grouped ones are tame.
+static const StepVariant &step_variant_for(int threads, bool validate, bool tame, bool grouped) {
+  if (validate) tame = grouped = false;
+  if (grouped) tame = true;
+  const StepVariant *last = nullptr;
+  for (const StepVariant &v : STEP_VARIANTS) {
+    if (v.validate != validate || v.tame != tame || v.grouped != grouped) continue;
+    if (threads <= v.maxt) return v;
+    last = &v;
   }
-  if (grouped) {   // (only built in the tame form: te_create keeps G = 1 otherwise)
-    if (threads <= 64) return {te_step_kernel<64, 16, false, true, true>, 64};
-    // default 3x3 grid: two envs (2 x 48 roads) on three warps, 20 envs per SM at 64 registers (72 registers and 9 CTAs
-    // per SM measured 2.4 % slower)
-    if (threads <= 96) return {te_step_kernel<96, 10, false, true, true>, 96};
-    if (threads <= 128) return {te_step_kernel<128, 8, false, true, true>, 128};
-    if (threads <= 160) return {te_step_kernel<160, 6, false, true, true>, 160};
-    return {te_step_kernel<256, 4, false, true, true>, 256};
-  }
-  if (tame) {
-    if (threads <= 64) return {te_step_kernel<64, 16, false, true, false>, 64};
-    if (threads <= 128) return {te_step_kernel<128, 8, false, true, false>, 128};
-    if (threads <= 256) return {te_step_kernel<256, 4, false, true, false>, 256};
-    if (threads <= 512) return {te_step_kernel<512, 2, false, true, false>, 512};
-    if (threads <= 768) return {te_step_kernel<768, 1, false, true, false>, 768};
-    return {te_step_kernel<1024, 1, false, true, false>, 1024};
-  }
-  if (threads <= 64) return {te_step_kernel<64, 16, false, false, false>, 64};
-  if (threads <= 128) return {te_step_kernel<128, 8, false, false, false>, 128};
-  if (threads <= 256) return {te_step_kernel<256, 4, false, false, false>, 256};
-  if (threads <= 512) return {te_step_kernel<512, 2, false, false, false>, 512};
-  if (threads <= 768) return {te_step_kernel<768, 1, false, false, false>, 768};
-  return {te_step_kernel<1024, 1, false, false, false>, 1024};
+  return *last;
 }
 // The double literals of the IDM update live in constant memory (te_math.cuh: g_mc); one upload per device.
 static cudaError_t upload_math_consts() {
@@ -362,58 +376,110 @@ static std::vector<uint32_t> build_gap_cdf(double cars_per_tick) {
 
 extern "C" int te_destroy(te_handle *h) { delete h; return 0; }
 
+// Rows of one env in HBM and in a one-env CTA: R roads padded to whole warps, or to whole groups of four warps when that
+// costs at most 20 % more rows.  Whole groups of four warps keep the SM's four schedulers evenly loaded (a 14-warp CTA
+// puts 4, 4, 3, 3 warps on them; two such CTAs 8, 8, 6, 6).  10x10 grid: 440 roads -> 512 threads, 16 warps, 64
+// registers: +1.7 % (measured A/B, 3 runs each).
+static int padded_rows(int R) {
+  const int rp32 = (R + GROUP_ROADS - 1) / GROUP_ROADS * GROUP_ROADS, rp128 = (R + 127) / 128 * 128;
+  return rp128 * 5 <= R * 6 ? rp128 : rp32;
+}
+
+// The configurations te_create accepts, apart from the device: physically sensible ones only (bit-parity with the
+// reference is established for these): finite positive tick length, road length, desired speed, acceleration and
+// braking; and a road longer than twice the farthest a car can travel in one tick, so that a car handed to the next road
+// cannot leave that road in the same tick (the reference's sequential road loop could pop it again; the parallel
+// transfer phase does not).
+static int check_config(const te_config *cfg, const char *who) {
+  if (cfg->struct_size != (int32_t)sizeof(te_config)) return fail("%s: te_config size mismatch (%d vs %zu)", who, cfg->struct_size, sizeof(te_config));
+  if (cfg->m < 1 || cfg->n < 1 || cfg->num_envs < 1) return fail("%s: bad dimensions", who);
+  const float *a = cfg->archetype;
+  auto pos = [](float f) { return std::isfinite(f) && f > 0.f; };
+  if (!pos(cfg->rate) || !pos(cfg->length)) return fail("%s: rate and length must be finite and positive", who);
+  if (!pos(a[5]) || !pos(a[3]) || !pos(a[6]) || !pos(a[4]) || !pos(a[7]))
+    return fail("%s: archetype v0, a, b, delta and T must be finite and positive", who);
+  for (int i = 0; i < TE_PARAMS; i++) if (!std::isfinite(a[i])) return fail("%s: archetype[%d] is not finite", who, i);
+  if (a[1] < 0.f || a[2] < 0.f || a[8] < 0.f) return fail("%s: archetype v, l and s0 must be non-negative", who);
+  const double vmax = std::max((double)a[5] + (double)a[3] * cfg->rate, (double)a[1]);
+  const double max_disp = cfg->rate * vmax + 0.5 * (double)a[3] * cfg->rate * cfg->rate;
+  if ((double)cfg->length <= 2.0 * max_disp)
+    return fail("%s: road length %.3f is not above twice the maximum displacement per tick (%.3f)", who, cfg->length, max_disp);
+  return 0;
+}
+
+// The one place that decides the CTA layout and the step kernel of a configuration (select_layout, te_plan_step_variant).
+// tame: every car the handle has seen is tame (tame_archetype, and no wild car loaded).  Touches no device.
+// One thread per road.  Small grids put G env instances on one CTA (its rows are the G * R roads of those envs) so that no
+// lane is a padding lane and a warp's car list is long: G in 1..4 with at most 256 rows, chosen for the fewest padding
+// lanes (ties: the smaller G).  Default 3x3 grid: R = 48 -> G = 2, 96 threads, three warps.  Large grids: G = 1, the CTA
+// padded like the HBM rows (padded_rows).
+static int plan_layout(const te_config *cfg, bool tame, const char *who, te_step_variant_t *out, const StepVariant **sv_out) {
+  if (cfg->m > 1024 || cfg->n > 1024) return fail("%s: a %d x %d grid exceeds one CTA (max 1024 roads)", who, cfg->m, cfg->n);
+  const int R = 4 * cfg->m * cfg->n + 2 * cfg->n + 2 * cfg->m, Rp = padded_rows(R);
+  if (Rp > 1024) return fail("%s: %d roads exceed one CTA (max 1024)", who, Rp);
+  IdmConst c = {};
+  fill_idm(c, cfg->archetype, cfg->rate);
+  const bool validate = (cfg->flags & TE_VALIDATE) != 0, tame_form = runs_tame_form(c, tame);
+  int G = 1, threads = Rp;
+  if (!validate && R < 128 && tame_form) {
+    double best = (double)(Rp - R) / Rp;
+    for (int g = 2; g <= 4 && g * R <= 256; g++) {
+      const int th = (g * R + 31) / 32 * 32;
+      const double waste = (double)(th - g * R) / th;
+      if (waste < best - 1e-9) { best = waste; G = g; threads = th; }
+    }
+  }
+  const StepVariant &sv = step_variant_for(threads, validate, tame_form, G > 1);
+  if (threads > sv.maxt)
+    return fail("%s: %d roads exceed the largest%s kernel variant (te_step_kernel<%d, %d, %s>)", who, threads,
+                validate ? " validate-mode" : "", sv.maxt, sv.minb, validate ? "validate" : sv.tame ? "tame" : "checked");
+  *out = {sv.maxt, sv.minb, sv.validate, sv.tame, sv.grouped, R, Rp, G, threads};
+  if (sv_out) *sv_out = &sv;
+  return 0;
+}
+
 // Threads per CTA, env instances per CTA and the kernel variant of a handle; called by te_create and again when a
 // handle stops being tame (a wild car in loaded records, load_records: the checked, one-env-per-CTA kernels take over).
 static int select_layout(te_handle *h) {
-  const te_config *cfg = &h->cfg;
-  StepParams &p = h->base;
-  // One thread per road.  Small grids put G env instances on one CTA (its rows are the G * R roads of those envs) so
-  // that no lane is a padding lane and a warp's car list is long: G in 1..4 with at most 256 rows, chosen for the
-  // fewest padding lanes (ties: the smaller G).  Default 3x3 grid: R = 48 -> G = 2, 96 threads, three warps.
-  // Large grids: G = 1, the CTA padded like the HBM rows (Rp).
-  if (h->Rp > 1024) { return fail("te_create: %d roads exceed one CTA (max 1024)", h->Rp); }
-  const bool validate = (cfg->flags & TE_VALIDATE) != 0;
-  h->G = 1; h->threads = h->Rp;
-  if (!validate && h->R < 128 && runs_tame_form(h->base.idm, h->tame)) {
-    double best = (double)(h->Rp - h->R) / h->Rp;
-    for (int g = 2; g <= 4 && g * h->R <= 256; g++) {
-      const int th = (g * h->R + 31) / 32 * 32;
-      const double waste = (double)(th - g * h->R) / th;
-      if (waste < best - 1e-9) { best = waste; h->G = g; h->threads = th; }
-    }
-  }
+  const StepVariant *sv = nullptr;
+  if (int rc = plan_layout(&h->cfg, h->tame, "te_create", &h->plan, &sv)) return rc;
+  h->sv = sv; h->G = h->plan.envs_per_cta; h->threads = h->plan.threads;
   h->warps = h->threads / GROUP_ROADS;
-  p.G = h->G;
+  h->base.G = h->G;
   CU(cudaDeviceGetAttribute(&h->smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
-  const StepVariant sv = step_variant_for(h->threads, validate, runs_tame_form(h->base.idm, h->tame), h->G > 1);
-  if (h->threads > sv.maxt) { return fail("te_create: %d roads exceed the largest%s kernel variant (%d)", h->threads, validate ? " validate-mode" : "", sv.maxt); }
-  const int smem_max = smem_bytes(sv.maxt, validate, MAX_K, h->n_entry, h->G);
+  const int smem_max = smem_bytes(sv->maxt, sv->validate, MAX_K, h->n_entry, h->G);
   if (smem_max > h->smem_optin) { return fail("te_create: env needs %d B of shared memory, device allows %d", smem_max, h->smem_optin); }
-  CU(cudaFuncSetAttribute(sv.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
+  CU(cudaFuncSetAttribute(sv->fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
+  return 0;
+}
+
+extern "C" int te_step_variants(te_step_variant_t *out, int32_t cap, int32_t *count) {
+  if (!count || cap < 0 || (cap > 0 && !out)) return fail("te_step_variants: bad argument");
+  for (int i = 0; i < NUM_STEP_VARIANTS && i < cap; i++) {
+    const StepVariant &v = STEP_VARIANTS[i];
+    out[i] = {v.maxt, v.minb, v.validate, v.tame, v.grouped, 0, 0, 0, 0};
+  }
+  *count = NUM_STEP_VARIANTS;
+  return 0;
+}
+
+extern "C" int te_plan_step_variant(const te_config *cfg, int32_t wild, te_step_variant_t *out) {
+  if (!cfg || !out) return fail("te_plan_step_variant: null argument");
+  if (int rc = check_config(cfg, "te_plan_step_variant")) return rc;
+  float v_cap = 0.f;
+  const bool tame = tame_archetype(cfg, &v_cap) && !wild;
+  return plan_layout(cfg, tame, "te_plan_step_variant", out, nullptr);
+}
+
+extern "C" int te_get_step_variant(const te_handle *h, te_step_variant_t *out) {
+  if (!h || !out) return fail("te_get_step_variant: null argument");
+  *out = h->plan;
   return 0;
 }
 
 extern "C" int te_create(const te_config *cfg, te_handle **out) {
   if (!cfg || !out) return fail("te_create: null argument");
-  if (cfg->struct_size != (int32_t)sizeof(te_config)) return fail("te_create: te_config size mismatch (%d vs %zu)", cfg->struct_size, sizeof(te_config));
-  if (cfg->m < 1 || cfg->n < 1 || cfg->num_envs < 1) return fail("te_create: bad dimensions");
-  {
-    // Physically sensible configurations only (bit-parity with the reference is established for these): finite
-    // positive tick length, road length, desired speed, acceleration and braking; and a road longer than twice the
-    // farthest a car can travel in one tick, so that a car handed to the next road cannot leave that road in the
-    // same tick (the reference's sequential road loop could pop it again; the parallel transfer phase does not).
-    const float *a = cfg->archetype;
-    auto pos = [](float f) { return std::isfinite(f) && f > 0.f; };
-    if (!pos(cfg->rate) || !pos(cfg->length)) return fail("te_create: rate and length must be finite and positive");
-    if (!pos(a[5]) || !pos(a[3]) || !pos(a[6]) || !pos(a[4]) || !pos(a[7]))
-      return fail("te_create: archetype v0, a, b, delta and T must be finite and positive");
-    for (int i = 0; i < TE_PARAMS; i++) if (!std::isfinite(a[i])) return fail("te_create: archetype[%d] is not finite", i);
-    if (a[1] < 0.f || a[2] < 0.f || a[8] < 0.f) return fail("te_create: archetype v, l and s0 must be non-negative");
-    const double vmax = std::max((double)a[5] + (double)a[3] * cfg->rate, (double)a[1]);
-    const double max_disp = cfg->rate * vmax + 0.5 * (double)a[3] * cfg->rate * cfg->rate;
-    if ((double)cfg->length <= 2.0 * max_disp)
-      return fail("te_create: road length %.3f is not above twice the maximum displacement per tick (%.3f)", cfg->length, max_disp);
-  }
+  if (int rc = check_config(cfg, "te_create")) return rc;
   int ndev = 0;
   cudaError_t e = cudaGetDeviceCount(&ndev);
   if (e != cudaSuccess || ndev == 0)
@@ -426,14 +492,7 @@ extern "C" int te_create(const te_config *cfg, te_handle **out) {
   CU(upload_math_consts());
   const int m = cfg->m, n = cfg->n;
   h->V = m * n; h->I = h->V; h->r = 4 * h->V; h->R = h->r + 2 * n + 2 * m;
-  h->Rp = (h->R + GROUP_ROADS - 1) / GROUP_ROADS * GROUP_ROADS;
-  {
-    // Whole groups of four warps keep the SM's four schedulers evenly loaded (a 14-warp CTA puts 4, 4, 3, 3 warps on
-    // them; two such CTAs 8, 8, 6, 6): pad to a multiple of 128 threads when that costs at most 20 % more rows.
-    // 10x10 grid: 440 roads -> 512 threads, 16 warps, 64 registers: +1.7 % (measured A/B, 3 runs each).
-    const int rp128 = (h->R + 127) / 128 * 128;
-    if (rp128 * 5 <= h->R * 6) h->Rp = rp128;
-  }
+  h->Rp = padded_rows(h->R);
   // topology (roadgraph.py:35-39, 42-51)
   h->dest.resize(h->R); h->nexts.resize(h->R); h->phases.resize(h->R);
   std::vector<short> nx(h->Rp, -1), up(h->Rp, -1);
@@ -679,7 +738,9 @@ enum class Route { DEVICE, WIRE, FLOATS };
 
 // Host float outputs travel as wire records unless the handle lets the copy engine write them (float_dma); a masked
 // step takes records whenever they fit, so that only the stepped envs are expanded.  Raw ticks and steps of more than
-// WIRE_MAX_K ticks do not fit a record.
+// WIRE_MAX_K ticks do not fit a record.  The kernel writes no staging row of an env it does not step, so a masked step on
+// the float route goes through the handle's page-locked staging and only the stepped rows reach the caller
+// (launch_sliced).
 static Route pick_route(const te_handle *h, const StepReq &q) {
   if (q.memspace != TE_HOST) return Route::DEVICE;
   const bool wire = !q.raw && q.K <= WIRE_MAX_K && (q.wire_only || !h->float_dma || q.env_mask);
@@ -726,6 +787,11 @@ static int step_params(te_handle *h, const StepReq &q, Route route, cudaStream_t
     if (int rc = grow(h->d_done, n, true)) return rc;
     h->float_steps = q.nsteps;
   }
+  if (route == Route::FLOATS && q.env_mask && q.nsteps > h->h_float_steps) {
+    h->h_float_steps = 0;
+    if (int rc = grow(h->h_float, (size_t)q.nsteps * E * (4 * (2 * h->r + 2 * h->I) + 4 * h->I + 1))) return rc;
+    h->h_float_steps = q.nsteps;
+  }
   p.actions = h->d_actions.get(); p.actions_out = greedy ? h->d_actions.get() : nullptr;
   p.env_mask = q.env_mask ? h->d_mask.get() : nullptr;
   p.obs_f = reinterpret_cast<float *>(h->d_obs_i.get()); p.obs_i = h->d_obs_i.get();
@@ -745,7 +811,7 @@ static te_wire_layout_t wire_layout_of(const te_handle *h) {
 // are simulated (envs are independent: any slicing gives the same results).  Fused steps of up to WIRE_MAX_K ticks
 // travel as compact wire records (one copy per slice and actor step, 2.5 x fewer bytes than the float observation)
 // that the handle's helper threads expand into the caller's arrays while the GPU works on the next slices.
-static int launch_sliced(te_handle *h, const StepReq &q, Route route, StepParams &p, StepVariant sv, int smem,
+static int launch_sliced(te_handle *h, const StepReq &q, Route route, StepParams &p, const StepVariant &sv, int smem,
                          cudaStream_t st) {
   const int nsteps = q.nsteps, G = h->G;
   const size_t E = (size_t)h->cfg.num_envs;
@@ -757,6 +823,12 @@ static int launch_sliced(te_handle *h, const StepReq &q, Route route, StepParams
   CU(cudaStreamWaitEvent(h->stream2.get(), h->ev_fork.get(), 0));
   cudaStream_t lanes[2] = {st, h->stream2.get()}, cs_copy = h->stream_copy.get();
   const char *src_obs = (const char *)h->d_obs_i.get();   // int (raw) or float observations
+  // float route: the caller's arrays, or for a masked step the handle's page-locked staging (same [nsteps][E] layout)
+  const bool staged = route == Route::FLOATS && q.env_mask;
+  unsigned char *const stage = h->h_float.get();
+  char *dst_obs = staged ? (char *)stage : (char *)q.obs;
+  float *dst_reward = staged ? (float *)(stage + (size_t)nsteps * E * obs_len * 4) : q.reward;
+  uint8_t *dst_done = staged ? stage + (size_t)nsteps * E * (obs_len + h->I) * 4 : q.done;
   unsigned char *host_wire = q.wire_only ? (unsigned char *)q.obs : h->h_wire.get();
   const unsigned char *dev_wire = h->d_wire.get();
   const size_t wstep = E * (size_t)h->wire_stride;   // records of one actor step
@@ -777,11 +849,11 @@ static int launch_sliced(te_handle *h, const StepReq &q, Route route, StepParams
     } else {
       for (int j = 0; j < nsteps; j++) {      // float arrays written by the copy engine, [nsteps][E][...]
         const size_t eo = (size_t)j * E + e0;
-        CU(cudaMemcpyAsync((char *)q.obs + eo * obs_len * 4, src_obs + eo * obs_len * 4, (size_t)ne * obs_len * 4,
+        CU(cudaMemcpyAsync(dst_obs + eo * obs_len * 4, src_obs + eo * obs_len * 4, (size_t)ne * obs_len * 4,
                            cudaMemcpyDeviceToHost, cs_copy));
-        CU(cudaMemcpyAsync(q.reward + eo * h->I, h->d_reward.get() + eo * h->I, (size_t)ne * h->I * sizeof(float),
+        CU(cudaMemcpyAsync(dst_reward + eo * h->I, h->d_reward.get() + eo * h->I, (size_t)ne * h->I * sizeof(float),
                            cudaMemcpyDeviceToHost, cs_copy));
-        CU(cudaMemcpyAsync(q.done + eo, h->d_done.get() + eo, (size_t)ne, cudaMemcpyDeviceToHost, cs_copy));
+        CU(cudaMemcpyAsync(dst_done + eo, h->d_done.get() + eo, (size_t)ne, cudaMemcpyDeviceToHost, cs_copy));
       }
     }
     nk = k + 1;
@@ -804,6 +876,13 @@ static int launch_sliced(te_handle *h, const StepReq &q, Route route, StepParams
     return 0;
   }
   CU(cudaStreamSynchronize(st));
+  if (staged)
+    for (size_t eo = 0; eo < (size_t)nsteps * E; eo++)
+      if (q.env_mask[eo % E]) {
+        memcpy((char *)q.obs + eo * obs_len * 4, dst_obs + eo * obs_len * 4, obs_len * 4);
+        memcpy(q.reward + eo * h->I, dst_reward + eo * h->I, (size_t)h->I * sizeof(float));
+        q.done[eo] = dst_done[eo];
+      }
   return 0;
 }
 
@@ -825,9 +904,8 @@ static int launch_step(te_handle *h, const StepReq &q) {
     te_reset_kernel<<<(h->cfg.num_envs + RESET_ENVS_PER_CTA - 1) / RESET_ENVS_PER_CTA, 128, 0, st>>>(p, p.env_mask, nullptr, 1);
     CU(cudaGetLastError());
   }
-  const bool validate = (h->cfg.flags & TE_VALIDATE) != 0;
-  const StepVariant sv = step_variant_for(h->threads, validate, runs_tame_form(h->base.idm, h->tame), h->G > 1);
-  const int smem = smem_bytes(sv.maxt, validate, K * nsteps, h->n_entry, h->G);
+  const StepVariant &sv = *h->sv;
+  const int smem = smem_bytes(sv.maxt, sv.validate, K * nsteps, h->n_entry, h->G);
   CU(cudaEventRecord(h->ev0.get(), st));
   if (route != Route::DEVICE) return launch_sliced(h, q, route, p, sv, smem, st);
   p.env0 = 0; p.env_end = h->cfg.num_envs;

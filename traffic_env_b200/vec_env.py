@@ -74,28 +74,49 @@ class WireResult(object):
         return iter((self.obs, self.reward, self.done))
 
 
+def make_config(m=3, n=3, length=250.0, num_envs=1, rate=0.5, ticks_per_step=10, remi=True, learn_switch=False,
+                auto_reset=False, validate=False, arrivals="philox", local_cars_per_sec=0.12, entry="all", seed=0,
+                env_id_base=0, device=0, episode_len=0, gamma=0.8, archetype=None, ordered_transfers=False):
+    """The te_config of VecTrafficEnv(**the same arguments) (ticks_per_step is the Python side's own)."""
+    cfg = _lib.default_config()
+    cfg.m, cfg.n, cfg.length, cfg.rate = int(m), int(n), float(length), float(rate)
+    cfg.num_envs, cfg.env_id_base, cfg.device = int(num_envs), int(env_id_base), int(device)
+    cfg.flags = ((TE_REMI if remi else 0) | (TE_LEARN_SWITCH if learn_switch else 0) |
+                 (TE_AUTO_RESET if auto_reset else 0) | (TE_VALIDATE if validate else 0) |
+                 (TE_ORDERED_TRANSFERS if ordered_transfers else 0))
+    cfg.entry_spec = entry_spec_of(entry)
+    cfg.arrival_mode = {"philox": TE_ARRIVALS_PHILOX, "injected": TE_ARRIVALS_INJECTED,
+                        "none": TE_ARRIVALS_NONE}[arrivals]
+    # FLAGS.cars_per_sec = local_cars_per_sec * m * inv_popcount(spec)  (traffic_env.py:394)
+    cfg.cars_per_tick = float(local_cars_per_sec) * int(m) * inv_popcount(cfg.entry_spec) * float(rate)
+    cfg.seed, cfg.episode_len, cfg.gamma = int(seed), int(episode_len), float(gamma)
+    arch = ARCHETYPE if archetype is None else np.asarray(archetype, dtype=np.float32)
+    for i in range(_lib.TE_PARAMS):
+        cfg.archetype[i] = float(arch[i])
+    return cfg
+
+
+def plan_step_variant(wild=False, **kwargs):
+    """The step-kernel instantiation VecTrafficEnv(**kwargs) runs (te_plan_step_variant, as _lib.variant_dict), or with
+    wild=True the one it runs after a wild car was loaded.  Needs no device."""
+    out = _lib.TeStepVariant()
+    check(_lib.load().te_plan_step_variant(C.byref(make_config(**kwargs)), int(bool(wild)), C.byref(out)))
+    return _lib.variant_dict(out)
+
+
 class VecTrafficEnv(object):
     def __init__(self, m=3, n=3, length=250.0, num_envs=1, rate=0.5, ticks_per_step=10, remi=True,
                  learn_switch=False, auto_reset=False, validate=False, arrivals="philox", local_cars_per_sec=0.12,
                  entry="all", seed=0, env_id_base=0, device=0, episode_len=0, gamma=0.8, archetype=None,
                  ordered_transfers=False):
         L = _lib.load()
-        cfg = _lib.default_config()
-        cfg.m, cfg.n, cfg.length, cfg.rate = int(m), int(n), float(length), float(rate)
-        cfg.num_envs, cfg.env_id_base, cfg.device = int(num_envs), int(env_id_base), int(device)
-        cfg.flags = ((TE_REMI if remi else 0) | (TE_LEARN_SWITCH if learn_switch else 0) |
-                     (TE_AUTO_RESET if auto_reset else 0) | (TE_VALIDATE if validate else 0) |
-                     (TE_ORDERED_TRANSFERS if ordered_transfers else 0))
-        cfg.entry_spec = entry_spec_of(entry)
-        cfg.arrival_mode = {"philox": TE_ARRIVALS_PHILOX, "injected": TE_ARRIVALS_INJECTED,
-                            "none": TE_ARRIVALS_NONE}[arrivals]
+        cfg = make_config(m=m, n=n, length=length, num_envs=num_envs, rate=rate, remi=remi, learn_switch=learn_switch,
+                          auto_reset=auto_reset, validate=validate, arrivals=arrivals,
+                          local_cars_per_sec=local_cars_per_sec, entry=entry, seed=seed, env_id_base=env_id_base,
+                          device=device, episode_len=episode_len, gamma=gamma, archetype=archetype,
+                          ordered_transfers=ordered_transfers)
         # FLAGS.cars_per_sec = local_cars_per_sec * m * inv_popcount(spec)  (traffic_env.py:394)
         self.cars_per_sec = float(local_cars_per_sec) * int(m) * inv_popcount(cfg.entry_spec)
-        cfg.cars_per_tick = self.cars_per_sec * float(rate)
-        cfg.seed, cfg.episode_len, cfg.gamma = int(seed), int(episode_len), float(gamma)
-        arch = ARCHETYPE if archetype is None else np.asarray(archetype, dtype=np.float32)
-        for i in range(_lib.TE_PARAMS):
-            cfg.archetype[i] = float(arch[i])
         self._L = L
         self._h = C.c_void_p()
         check(L.te_create(C.byref(cfg), C.byref(self._h)))
@@ -469,6 +490,12 @@ class VecTrafficEnv(object):
         t = C.c_int32(0)
         check(self._L.te_is_tame(self._h, C.byref(t), None))
         return bool(t.value)
+
+    def step_variant(self):
+        """The step-kernel instantiation the handle runs now (te_get_step_variant, as _lib.variant_dict)."""
+        out = _lib.TeStepVariant()
+        check(self._L.te_get_step_variant(self._h, C.byref(out)))
+        return _lib.variant_dict(out)
 
     def tame_speed_cap(self):
         """Largest car speed te_set_state accepts without leaving the tame mode (0.0: archetype outside the ranges)."""
