@@ -50,6 +50,7 @@ def lib():
             getattr(L, name).argtypes = [vp]
         L.to_steps.restype = f32
         L.to_steps.argtypes = [vp]
+        L.to_set_steps.argtypes = [vp, f32]
         for name in ("to_generated", "to_vehicle_updates", "to_overflows"):
             getattr(L, name).restype = C.c_long
             getattr(L, name).argtypes = [vp]
@@ -151,6 +152,11 @@ class OracleEnv(object):
     @property
     def steps(self):
         return self._L.to_steps(self._h)
+
+    @steps.setter
+    def steps(self, value):
+        """Start the np.float32 clock anywhere (as a reference env's `steps` attribute can be set)."""
+        self._L.to_set_steps(self._h, float(np.float32(value)))
 
     @property
     def generated_cars(self):

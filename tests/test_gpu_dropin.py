@@ -95,6 +95,54 @@ def test_fused_wrappers_match_tick_loop(dropin):
     assert fa.reward_size == 9 and fa.observation_space.shape == [81] and fa.action_space.size == 9
 
 
+def test_fused_wrappers_match_tick_loop_past_clock_limit(dropin, monkeypatch):
+    """Remi(Repeater(10)), fused and on the tick loop, from an episode clock of 2^24 - 40: the float32 clock stops at 2^24
+    on both paths, one float32 add per tick.  Heavy arrivals make fused steps overflow, and such a step reads back the
+    ticks it ran; the count must come from the device, not from the clock, or the injected arrival schedule goes out of
+    step with the device.  A short schedule window makes the host send a new window every few steps."""
+    gym, GridRoad, FLAGS = dropin
+    from gym_traffic.envs import traffic_env as te
+    from traffic_env_b200.wrappers import Remi, Repeater
+    monkeypatch.setattr(te, "_WINDOW", 48)
+    monkeypatch.setattr(FLAGS, "local_cars_per_sec", 0.35)
+    start = np.float32(2 ** 24 - 40)
+
+    def build(fused):
+        np.random.seed(3)
+        base = new_env(gym, GridRoad, seed=11)
+        if not fused:
+            base.rendering = True
+            base.render = lambda *a, **k: None
+        return Remi(Repeater(10)(base)), base
+
+    (fa, fb), (ta, tb) = build(True), build(False)
+    for env, base in ((fa, fb), (ta, tb)):
+        np.random.seed(21)
+        env.reset()          # (Repeater's reset runs a first actor step)
+        base.steps = start
+        st = base._sim.get_state(0, 1)
+        st["steps"][:] = start
+        base._sim.set_state(st)
+    ticks0 = int(tb._sim.stats()["ticks"])
+    assert fb._sim.stats()["ticks"] == ticks0
+    rng = np.random.RandomState(5)
+    fused_overflows = 0
+    for s in range(60):
+        a = rng.randint(2, size=9) if s % 7 else np.zeros(9, np.int32)
+        x1, r1, d1, _ = fa.step(a)
+        x2, r2, d2, _ = ta.step(a)
+        assert x1.tobytes() == np.asarray(x2, np.float32).tobytes(), s
+        assert np.asarray(r1).tobytes() == np.asarray(r2).tobytes() and d1 == d2, s
+        fused_overflows += int(d1)
+        ticks = int(tb._sim.stats()["ticks"]) - ticks0
+        want = np.float32(min(float(start) + ticks, 2.0 ** 24))   # +1 per tick in float32: exact up to 2^24, then stuck
+        assert type(fb.steps) is np.float32 and fb.steps == tb.steps == want, (s, float(fb.steps), float(tb.steps), float(want))
+        assert fb._sim.get_state(0, 1)["steps"][0] == want, s
+        assert fb._sim.stats()["ticks"] == ticks0 + ticks, s
+        assert fb._sim.stats()["cars_generated"] == tb._sim.stats()["cars_generated"], s
+    assert fused_overflows > 3 and float(fb.steps) == 2.0 ** 24
+
+
 def test_agent_loop_contracts(dropin):
     gym, GridRoad, FLAGS = dropin
     from tests.support.wrappers_ref import make_env

@@ -241,21 +241,27 @@ def test_wire_records_equal_float_outputs():
 
 @pytest.mark.parametrize("m,n,L,E,lcps,extra", [
     (3, 3, 250.0, 301, 0.5, {}), (10, 10, 500.0, 6, 0.3, {}), (2, 2, 120.0, 77, 0.9, {}), (4, 4, 150.0, 33, 0.4, {}),
-    (3, 3, 250.0, 65, 0.5, {"learn_switch": True}), (3, 3, 250.0, 40, 0.15, {"validate": True}), (3, 3, 250.0, 50, 0.5, {"remi": False})])
+    (3, 3, 250.0, 65, 0.5, {"learn_switch": True}), (3, 3, 250.0, 40, 0.15, {"validate": True}), (3, 3, 250.0, 50, 0.5, {"remi": False}),
+    (3, 3, 250.0, 40, 0.5, {"clock": 2.0 ** 24 - 15})])
 def test_multi_step_launch_equals_single_steps(m, n, L, E, lcps, extra):
     """te_step_multi (n actor steps per launch, greedy controller evaluated in the kernel or a given action) produces,
     actor step by actor step, exactly what n te_step calls with the same action produce - host and device buffers -
-    including overflow steps (early break) in the middle of a launch and an env count that leaves a partial CTA."""
+    including overflow steps (early break) in the middle of a launch and an env count that leaves a partial CTA.
+    `clock`: the episode clocks start there, and the launches cross 2^24, where the float32 clock stops."""
     import torch
     from traffic_env_b200 import VecTrafficEnv
     kw = dict(m=m, n=n, length=L, num_envs=E, arrivals="philox", seed=11, local_cars_per_sec=lcps, ticks_per_step=10, remi=True)
-    kw.update(extra)
+    kw.update({k: v for k, v in extra.items() if k != "clock"})
     a, b, d = VecTrafficEnv(**kw), VecTrafficEnv(**kw), VecTrafficEnv(**kw)
     I = m * n
     rng = np.random.RandomState(3)
     init = rng.randint(2, size=(E, I))
     for env in (a, b, d):
         env.reset(init_phase=init)
+        if "clock" in extra:
+            st = env.get_state()
+            st["steps"][:] = extra["clock"]
+            env.set_state(st)
     dev = torch.device("cuda", 0)
     NS = 6 if (m, n) == (4, 4) else 3          # 6 x 10 ticks: close to the 64-tick limit of one launch
     d_act = torch.zeros((E, I), dtype=torch.uint8, device=dev)
@@ -289,6 +295,8 @@ def test_multi_step_launch_equals_single_steps(m, n, L, E, lcps, extra):
     sa, sb, sd = a.get_state(), b.get_state(), d.get_state()
     for k in ("leading", "lastcar", "obs", "waiting", "passed_dst", "steps"):
         assert (sa[k] == sb[k]).all() and (sa[k] == sd[k]).all(), k
+    if "clock" in extra:
+        assert (sa["steps"] == np.float32(2 ** 24)).all()
     for e in range(E):
         xa, va = live_walk(sa["leading"][e], sa["lastcar"][e], sa["x"][e], sa["v"][e])
         xb, vb = live_walk(sb["leading"][e], sb["lastcar"][e], sb["x"][e], sb["v"][e])

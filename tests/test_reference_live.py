@@ -66,6 +66,46 @@ def test_oracle_vs_reference_live(case):
         set_flags(ref)
 
 
+def test_oracle_clock_past_2_24_vs_reference_live():
+    """The np.float32 episode clock near 2^24, validate mode: the reference adds 1 per tick to a float32 clock (under
+    NumPy 2 it stays float32), so it stops at 16777216, and cars born after that leave with trip time 0.  The oracle's
+    clock (to_set_steps, then its own tick rule) and its trip times must equal the reference's, tick by tick."""
+    from oracle import ref_harness as rh
+    from oracle.gen_golden import set_flags
+    from oracle.oracle import OracleEnv
+    m, n, length, ticks, seed = 3, 3, 100, 200, 106
+    start = np.float32(2 ** 24 - 20)
+    ref = rh.load()
+    set_flags(ref, local_cars_per_sec=0.2, mode="validate")
+    try:
+        np.random.seed(seed)
+        env = rh.make_env(ref, m, n, length, seed=seed)
+        sched = rh.record_schedule(ref, m, n, ticks, seed=seed)
+        env.reset()
+        env.steps = start
+        o = OracleEnv(m, n, float(length), 0.5, validate=True)
+        o.reset(env.current_phase.copy())
+        o.steps = start
+        rng = np.random.RandomState(seed + 1)
+        for t in range(ticks):
+            if t % 11 == 0:
+                a = rng.randint(2, size=m * n).astype(np.int32)
+            obs, rew, done, _ = env.step(a)
+            od = o.step(a, sched[t])
+            assert type(env.steps) is np.float32 and env.steps.tobytes() == np.float32(o.steps).tobytes(), t
+            xs, vs = rh.live_state(env)
+            oxs, ovs = o.live_state()
+            dr = tick_digest(env.leading, env.lastcar, env.obs, env.waiting, env.passed_dst, rew, done, xs, vs)
+            do = tick_digest(o.leading, o.lastcar, o.obs, o.waiting, o.passed_dst, o.rewards, od, oxs, ovs)
+            assert dr == do, "tick %d: oracle diverges from the live reference" % t
+        assert float(env.steps) == 2.0 ** 24
+        want = np.asarray(env.trip_times, np.float64)
+        assert want.tobytes() == o.trip_times().tobytes()
+        assert (want == 0.0).any() and (want > 0.0).any(), "cars born before and after the clock stopped are meant to leave"
+    finally:
+        set_flags(ref)
+
+
 _LAUNCHER_SCRIPT = r"""
 import importlib, os, sys, types
 sys.path.insert(0, %(root)r)

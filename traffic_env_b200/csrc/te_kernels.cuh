@@ -56,6 +56,21 @@ struct EnvScalars {
   double ep_ret, ep_disc, ep_mult;
 };
 
+// The episode clock after n ticks: the reference adds 1 to its np.float32 clock once per tick (traffic_env.py:247,
+// float32 under NumPy 2's promotion rules), so the clock stops at 2^24 (and at -2^24 from below), and a clock with a
+// fractional part rounds when it reaches 2^23.  One add of n rounds differently in both cases.
+__host__ __device__ __forceinline__ float clock_after(float c, int n) {
+#pragma unroll 1
+  for (int i = 0; i < n; i++) {
+#ifdef __CUDA_ARCH__
+    c = __fadd_rn(c, 1.f);
+#else
+    c = c + 1.f;
+#endif
+  }
+  return c;
+}
+
 struct DeviceStats {
   unsigned long long ticks, actor_steps, vehicle_updates, overflows, cars_generated, episodes, seq_fallback_ticks,
       cars_exited, arrival_saturations;
@@ -617,7 +632,9 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
   const bool is_train = my_road < p.r;
   float *xr = s.xs + my_sr * CAP, *vr = s.vs + my_sr * CAP;
   float *wr = VALIDATE ? s.ws + my_sr * CAP : nullptr;
-  const float steps0 = p.env[env_first + my_g].steps;  // np.float32 tick counter at the start of this launch (small integer: exact)
+  // validate mode: the episode clock of the current tick (birth stamps, trip times), one clock_after step per tick my env
+  // runs.  (Validate kernels run one env per CTA: every lane's env is the CTA's, and every lane runs every tick.)
+  float clk = VALIDATE ? p.env[env_first].steps : 0.f;
   int ld, lc, wait, det, passed = 0;
   float leadx;
   {
@@ -701,7 +718,7 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
       const int na = s.cnt[ei + tt * p.n_entry];
       for (int k = 0; k < na; k++) {
         gen_local++;
-        if (!ring_push(xr, vr, wr, ld, lc, c.x_new, c.v_new, steps0 + (float)tt, c)) dropped++;  // car[wi] = tick, :279
+        if (!ring_push(xr, vr, wr, ld, lc, c.x_new, c.v_new, clk, c)) dropped++;  // car[wi] = tick, :279
       }
     }
     if (is_train && !frozen) {  // update_lights
@@ -813,7 +830,7 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
             if ((long long)(base + k) < p.trip_cap) {
               TripRecord rec;
               rec.env = env_first + my_g;
-              rec.trip = __fsub_rn(steps0 + (float)tt, wr[fs]) / 2.0f;
+              rec.trip = __fsub_rn(clk, wr[fs]) / 2.0f;
               rec.order = (((unsigned long long)(p.env[env_first + my_g].sched_cursor + tt)) << 24) | ((unsigned long long)my_road << 8) | (unsigned)k;
               p.trips[base + k] = rec;
             }
@@ -869,6 +886,7 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
     }
     s.tailx[my_sr] = (lc != ld) ? xr[lc] : INF;
     __syncthreads();
+    if (VALIDATE) clk = clock_after(clk, 1);   // (the tick ran, also when it stops the env below)
     // tick-stamped (a fast warp that has already flagged tick t + 1 cannot be mistaken for tick t)
     if (GROUPED) {
       frozen = frozen || s.env_word(my_g, ENVM_OVF) <= t;
@@ -977,7 +995,7 @@ __global__ void __launch_bounds__(MAXT, MINB) te_step_kernel(const StepParams p)
       esg->ep_ret += mean; esg->ep_disc += mult * mean; esg->ep_mult = mult * (double)p.gamma;
     }
     if (last_step) {
-      esg->steps = esg->steps + (float)ticks_total;
+      esg->steps = clock_after(esg->steps, ticks_total);
       esg->sched_cursor += ticks_total;
       if (p.arrival_mode == ARR_PHILOX) {
         const uint32_t *snapg = snap_base + g * 2 * (KT + 1);

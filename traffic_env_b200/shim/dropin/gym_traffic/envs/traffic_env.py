@@ -51,6 +51,15 @@ def cars_on_roads(leading, lastcar):
     return (lastcar - leading + (CAPACITY - 1) * (leading > lastcar)).astype(np.int32)
 
 
+def clock_after(steps, ticks):
+    """The np.float32 clock after `ticks` ticks of the reference's `self.steps += 1` (traffic_env.py:247): one float32
+    add per tick, so the clock stops at 2^24 - the rule the device's clock follows too."""
+    steps = np.float32(steps)
+    for _ in range(int(ticks)):
+        steps = np.float32(steps + np.float32(1))
+    return steps
+
+
 def _mode():
     try:
         return FLAGS.mode
@@ -175,7 +184,7 @@ class TrafficEnv(gym.Env):
         self._mirror[:] = obs_raw
         self.rewards[:] = rewards
         self._ticks_total += ticks
-        self.steps = np.float32(self.steps + np.float32(ticks))
+        self.steps = clock_after(self.steps, ticks)
 
     def _as_action(self, action):
         """Truthiness per intersection, with numpy broadcasting like the reference's logical_xor(current_phase, action)
@@ -248,7 +257,8 @@ class TrafficEnv(gym.Env):
             st = sim.get_state(0, 1)
             raw = st["obs"][0]
             raw[:r] = 0
-            ticks = int(round(float(st["steps"][0]) - float(self.steps)))
+            # the ticks the launch ran, from the device's tick count (the clock stops at 2^24: its change is no count)
+            ticks = int(sim.stats()["ticks"]) - self._ticks_total
         self._pull(raw, rew[0], ticks)
         return obs[0].copy(), self.rewards, bool(done[0])
 
